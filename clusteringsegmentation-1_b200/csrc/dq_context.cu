@@ -130,6 +130,12 @@ struct dq_context {
     uint32_t *size_out = nullptr;
     int phase = 0;  // quantize_step
     uint32_t flags = 0, flags_all = 0, tie_count = 0, cut_count = 0, k_first = 0, resplits = 0;
+    // row-sharded call (dq_rows): the histogram and the first-seen indexes come from the gathered per-shard lists, not
+    // from pixels, and there is no ordered re-run (that needs the whole image in order)
+    struct Merged {
+      const uint32_t *colours = nullptr, *counts = nullptr, *first = nullptr;  // [world][cap], [world][cap], [world][cap + 1]
+      uint32_t cap = 0, world = 0;
+    } merged;
   } qs;
   cudaEvent_t tie_ev = nullptr;
   // Tie audit of the exact-integer split (dq_tie.cuh): 0 = off, 1 = report in dq_call_stats::tie_flags only,
@@ -599,7 +605,17 @@ void quantize_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t 
   q.records = records, q.mean_out = mean_out, q.size_out = size_out;
   q.phase = 0;
   q.flags = q.flags_all = q.tie_count = q.cut_count = q.k_first = q.resplits = 0;
+  q.merged = dq_context::QuantState::Merged();
   ctx->n_ovr = 0;
+}
+
+// The merged histogram of a row-sharded image in the direct table, and the whole image's first-seen index of every colour
+// in d_map (what the resolver reads); leaves U in d_cb->ucount.
+void run_merge(dq_context *ctx, const dq_context::QuantState::Merged &m) {
+  hist_merge(m.colours, m.counts, m.world * m.cap, ctx->d_table, ctx->d_uniq.ptr, &ctx->d_cb->ucount, ctx->sm_count, ctx->stream,
+             ctx->d_map);
+  hist_merge_first(m.colours, m.counts, m.first, m.cap, m.world, ctx->d_map, ctx->sm_count, ctx->stream);
+  ctx->stats.kernel_launches += 2;
 }
 
 // Second half, as a small state machine so that a host thread that drives several contexts never has to wait inside it:
@@ -661,11 +677,13 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     ctx->d_ovr.ensure(kCutOverrideCap * sizeof(CutOverride) / sizeof(uint32_t));
     DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_ovr.ptr, ctx->h_ovr, ctx->n_ovr * sizeof(CutOverride), cudaMemcpyHostToDevice, ctx->stream));
     reset_control(ctx);
-    run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
+    const bool merged = q.merged.colours != nullptr;
+    if (merged) run_merge(ctx, q.merged);  // (the shards' pixels are not here: merge the gathered lists again)
+    else run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
     uint32_t unused = 0;
     ctx->ovr_active = true;
-    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true, &src, true,
-              false, /*defer=*/true);
+    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true,
+              merged ? nullptr : &src, true, false, /*defer=*/true);
     ctx->ovr_active = false;
     q.resplits++;
     q.phase = 0;
@@ -698,7 +716,7 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     q.phase = 3;
   };
   const bool can_rerun = ctx->tie_policy == 2 && q.table_dirty && ctx->exact_small && K <= kExactMaxColors && K <= kSplit2MaxColors &&
-                         ctx->split_version == 2;
+                         ctx->split_version == 2 && q.merged.colours == nullptr;
   if (q.phase == 0) {
     *k_inout = run_split_finish(ctx, colortable, q.records, q.mean_out, q.size_out);
     q.flags = ctx->stats.tie_flags;
@@ -717,8 +735,10 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
       q.tie_count = ctx->h_cb->ctl[kCtlTieCount];
       q.cut_count = ctx->h_cb->ctl[kCtlCutCount];
       if (q.tie_count + q.cut_count >= 1 && q.tie_count <= kTieListCap && q.cut_count <= kTieListCap && ctx->resolve_mode != 0) {
-        first_seen_launch(exact_sampling(q.d_in, q.rows, q.cols, (uint32_t)q.dec, q.num_bits), ctx->d_map, ctx->stream);
-        ctx->stats.kernel_launches++;
+        if (q.merged.colours == nullptr) {  // (a merged histogram brought its first-seen indexes along: run_merge)
+          first_seen_launch(exact_sampling(q.d_in, q.rows, q.cols, (uint32_t)q.dec, q.num_bits), ctx->d_map, ctx->stream);
+          ctx->stats.kernel_launches++;
+        }
         ctx->ensure_small((size_t)K + 16 + 8 * kTieListCap + 2);
         q.k_first = *k_inout;
         if (!ctx->tie_ev) DQ_CUDA_CHECK(cudaEventCreateWithFlags(&ctx->tie_ev, cudaEventDisableTiming));
@@ -1530,6 +1550,8 @@ struct dq_pipeline {
   bool stop = false;
   std::atomic<uint64_t> launches{0};
   std::atomic<uint64_t> flagged_frames{0};  // frames the tie audit sent through the synchronous path
+  std::atomic<uint64_t> resolved_frames{0};  // ... settled by the resolver / forced cuts (dq_call_stats::tie_resolved, cut_overrides)
+  std::atomic<uint64_t> rerun_frames{0};     // ... computed again on the ordered path (dq_call_stats::ordered_rerun)
   // DIVQUANT_B200_ASYNC=1: the whole chain of a frame is queued without a host wait (palette handling on the device,
   // palette_post).  Off by default: measured at 4K, 12 lanes, it is slower than the host round trip (0.184-0.22 against
   // 0.166 ms/frame): the one-thread std::sort replay costs 93 us per frame on the lane's chain and the lanes' throughput
@@ -1541,6 +1563,12 @@ struct dq_pipeline {
 };
 
 namespace {
+
+// How the tie audit's recovery steps settled the frame the lane's context just finished (before pipeline_complete).
+void pipeline_count_ties(dq_pipeline *p, const dq_context *ctx) {
+  if (ctx->stats.tie_resolved || ctx->stats.cut_overrides) p->resolved_frames++;
+  if (ctx->stats.ordered_rerun) p->rerun_frames++;
+}
 
 void pipeline_complete(dq_pipeline *p, uint64_t ticket, uint64_t launches) {
   p->launches += launches;
@@ -1572,6 +1600,7 @@ void pipeline_run_sync(dq_pipeline *p, dq_pipeline::Lane &lane, const dq_pipelin
     DQ_CUDA_CHECK(cudaMemcpyAsync(job.out, lane.d_out, (size_t)job.n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaEventRecord(lane.end, ctx->stream));
   ctx->wait();
+  pipeline_count_ties(p, ctx);
   pipeline_complete(p, job.ticket, ctx->stats.kernel_launches);
 }
 
@@ -1608,6 +1637,7 @@ void pipeline_dispatcher(dq_pipeline *p, int first_lane, int lane_step) {
           }
         } else {
           if (ctx->stats.tie_flags) p->flagged_frames++;
+          pipeline_count_ties(p, ctx);
           pipeline_complete(p, lane.job.ticket, ctx->stats.kernel_launches);
         }
       } else if (lane.state == kWaitSplit) {
@@ -1817,6 +1847,8 @@ float dq_pipeline_last_elapsed_ms(const dq_pipeline *p) { return p->last_ms; }
 dq_context *dq_pipeline_context(dq_pipeline *p) { return p->lanes[0].ctx; }
 uint64_t dq_pipeline_kernel_launches(const dq_pipeline *p) { return p->launches.load(); }
 uint64_t dq_pipeline_flagged_frames(const dq_pipeline *p) { return p->flagged_frames.load(); }
+uint64_t dq_pipeline_resolved_frames(const dq_pipeline *p) { return p->resolved_frames.load(); }
+uint64_t dq_pipeline_rerun_frames(const dq_pipeline *p) { return p->rerun_frames.load(); }
 int dq_pipeline_lanes(const dq_pipeline *p) { return (int)p->lanes.size(); }
 
 // ---- test hooks ----
@@ -1900,10 +1932,11 @@ uint32_t dq_pixel_histogram(const uint32_t *pixels, uint32_t numPixels, uint32_t
 }  // extern "C"
 
 // ---- pixel-row sharding of one image, exchange inside the library (NCCL) ---------------------------------------------
-// BASELINE config 3.  Every rank histograms its own rows; the per-shard (colour, count) lists are exchanged with ONE
-// grouped ncclAllGather on the context's stream (fixed-capacity slices, unused entries carry count 0, so no sizes have to
-// travel first and nothing waits on the host); every rank merges the lists into its direct table and runs the split
-// replicated -- exact integer sums: identical decisions from identical integers on every GPU -- and remaps its own rows.
+// BASELINE config 3.  Every rank histograms its own rows; the per-shard (colour, count, first-seen index) lists are
+// exchanged with ONE grouped ncclAllGather on the context's stream (fixed-capacity slices, unused entries carry count 0, so
+// no sizes have to travel first and nothing waits on the host); every rank merges the lists into its direct table (and the
+// whole image's first-seen indexes into d_map, for the tie resolver) and runs the split replicated -- exact integer sums:
+// identical decisions from identical integers on every GPU, flagged frames through quantize_step -- and remaps its own rows.
 // NCCL is looked up at run time (dlopen of libnccl.so.2: the copy the process already has, e.g. PyTorch's, or the
 // system's), so the library itself has no link-time dependency on it.
 #include <dlfcn.h>
@@ -1966,6 +1999,7 @@ struct dq_rows {
   uint32_t cap = 0;              // list entries per rank
   uint32_t *d_colours = nullptr;  // [world][cap]
   uint32_t *d_counts = nullptr;   // [world][cap]
+  uint32_t *d_first = nullptr;    // [world][cap + 1]: shard-local first-seen index of every listed colour, then the shard's pixels
   uint32_t *d_overflow = nullptr;
 };
 
@@ -1983,6 +2017,10 @@ dq_rows *dq_rows_create(dq_context *ctx, int world, int rank, const void *unique
     fprintf(stderr, "divquant_b200: dq_rows_create needs 0 <= rank < world and a positive list capacity\n");
     abort();
   }
+  if ((uint64_t)world * ((uint64_t)list_capacity + 1) > 0xFFFFFFFFull) {  // (list offsets and entry counts are 32-bit)
+    fprintf(stderr, "divquant_b200: dq_rows_create: world x (list_capacity + 1) must stay below 2^32\n");
+    abort();
+  }
   dq_rows *r = new dq_rows();
   r->ctx = ctx;
   r->world = world;
@@ -1995,6 +2033,7 @@ dq_rows *dq_rows_create(dq_context *ctx, int world, int rank, const void *unique
   }
   DQ_CUDA_CHECK(cudaMalloc(&r->d_colours, (size_t)world * list_capacity * sizeof(uint32_t)));
   DQ_CUDA_CHECK(cudaMalloc(&r->d_counts, (size_t)world * list_capacity * sizeof(uint32_t)));
+  DQ_CUDA_CHECK(cudaMalloc(&r->d_first, (size_t)world * (list_capacity + 1) * sizeof(uint32_t)));
   DQ_CUDA_CHECK(cudaMalloc(&r->d_overflow, sizeof(uint32_t)));
   DQ_CUDA_CHECK(cudaMemset(r->d_overflow, 0, sizeof(uint32_t)));
   return r;
@@ -2007,6 +2046,7 @@ void dq_rows_destroy(dq_rows *r) {
   if (r->comm) nccl_api()->CommDestroy(r->comm);
   cudaFree(r->d_colours);
   cudaFree(r->d_counts);
+  cudaFree(r->d_first);
   cudaFree(r->d_overflow);
   delete r;
 }
@@ -2025,16 +2065,20 @@ void dq_rows_quant_recurse(dq_rows *r, const uint32_t *d_shard, uint32_t n_shard
   const uint32_t cap = r->cap;
   const size_t entries = (size_t)r->world * cap;
   uint32_t *my_colours = r->d_colours + (size_t)r->rank * cap, *my_counts = r->d_counts + (size_t)r->rank * cap;
-  // 1. this rank's rows -> (colour, count) list in its slice (an empty shard is a list of zero counts)
+  uint32_t *my_first = r->d_first + (size_t)r->rank * (cap + 1);
+  // 1. this rank's rows -> (colour, count, first-seen index) list in its slice (an empty shard is a list of zero counts)
   reset_control(ctx);
   ctx->d_pts0.ensure(std::max<size_t>(n_shard, entries));
   ctx->d_uniq.ensure(std::max<size_t>(n_shard, entries));
   if (n_shard) {
-    run_histogram(ctx, d_shard, n_shard, 1, n_shard, 1, 8);
+    hist_insert(d_shard, n_shard, 1, n_shard, 1, 8, ctx->d_table, ctx->d_uniq.ptr, &ctx->d_cb->ucount, ctx->sm_count, ctx->stream,
+                ctx->d_map);
+    first_seen_launch(exact_sampling(d_shard, 1, n_shard, 1, 8), ctx->d_map, ctx->stream);
     hist_collect(ctx->d_uniq.ptr, &ctx->d_cb->ucount, n_shard, ctx->d_table, ctx->d_pts0.ptr, true, ctx->sm_count, ctx->stream);
-    ctx->stats.kernel_launches++;
+    ctx->stats.kernel_launches += 3;
   }
-  hist_export_padded(ctx->d_pts0.ptr, &ctx->d_cb->ucount, cap, my_colours, my_counts, r->d_overflow, ctx->sm_count, ctx->stream);
+  hist_export_padded(ctx->d_pts0.ptr, &ctx->d_cb->ucount, cap, my_colours, my_counts, r->d_overflow, ctx->sm_count, ctx->stream,
+                     ctx->d_map, my_first, n_shard);
   ctx->stats.kernel_launches++;
   // 2. the one exchange of the data path
   if (r->world > 1) {
@@ -2042,14 +2086,26 @@ void dq_rows_quant_recurse(dq_rows *r, const uint32_t *d_shard, uint32_t n_shard
     nccl_check(nc->GroupStart(), "ncclGroupStart");
     nccl_check(nc->AllGather(my_colours, r->d_colours, cap, ncclUint32, r->comm, ctx->stream), "ncclAllGather(colours)");
     nccl_check(nc->AllGather(my_counts, r->d_counts, cap, ncclUint32, r->comm, ctx->stream), "ncclAllGather(counts)");
+    nccl_check(nc->AllGather(my_first, r->d_first, cap + 1, ncclUint32, r->comm, ctx->stream), "ncclAllGather(first-seen)");
     nccl_check(nc->GroupEnd(), "ncclGroupEnd");
   }
-  // 3. merged histogram of the whole image in this rank's direct table, split replicated, own rows remapped
+  // 3. merged histogram (and first-seen indexes) of the whole image in this rank's direct table, split replicated with the
+  //    tie audit's resolver and forced cuts (quantize_step), own rows remapped
+  dq_context::QuantState &q = ctx->qs;
+  q = dq_context::QuantState();
+  q.merged.colours = r->d_colours, q.merged.counts = r->d_counts, q.merged.first = r->d_first;
+  q.merged.cap = cap, q.merged.world = (uint32_t)r->world;
+  q.n = (uint32_t)total_pixels, q.rows = 1, q.cols = (uint32_t)total_pixels, q.K = K, q.point_cap = (uint32_t)entries;
+  q.norm = sample_norm(1, (uint32_t)total_pixels, 1);  // 1 / N of the WHOLE image (:172)
+  q.table_dirty = true;
+  ctx->n_ovr = 0;
   reset_control(ctx);
-  hist_merge(r->d_colours, r->d_counts, (uint32_t)entries, ctx->d_table, ctx->d_uniq.ptr, &ctx->d_cb->ucount, ctx->sm_count, ctx->stream);
-  ctx->stats.kernel_launches++;
-  const double norm = sample_norm(1, (uint32_t)total_pixels, 1);  // 1 / N of the WHOLE image (:172)
-  uint32_t k = run_split(ctx, (uint32_t)entries, norm, K, 10, 8, outColortablePtr, nullptr, nullptr, nullptr, true, nullptr, true);
+  run_merge(ctx, q.merged);
+  uint32_t k = 0;
+  run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &k, nullptr, nullptr, nullptr, true, nullptr, true, false,
+            /*defer=*/true);
+  k = K;
+  quantize_finish(ctx, &k, outColortablePtr);
   k = dedup_palette(outColortablePtr, k);
   *numClustersPtr = k;
   ctx->stats.actual_colors = k;

@@ -220,15 +220,21 @@ __global__ void __launch_bounds__(256) hist_export_kernel(const uint2 *__restric
 
 // Same into a fixed-capacity slice of the exchange buffers: entries beyond the shard's U get count 0 (the merge skips
 // them), a shard with more than `cap` colours raises *overflow (the caller sized the exchange too small).
+// With `first` (cap + 1 words): first[i] = the shard-local first-seen index of colour i (read from first_table), and
+// first[cap] = the shard's pixel count, from which the merge derives every shard's offset in the whole image.
 __global__ void __launch_bounds__(256) hist_export_padded_kernel(const uint2 *__restrict__ pts, const uint32_t *ucount, uint32_t cap,
-                                                                uint32_t *colours, uint32_t *counts, uint32_t *overflow) {
+                                                                uint32_t *colours, uint32_t *counts, uint32_t *overflow,
+                                                                const uint32_t *__restrict__ first_table, uint32_t *first,
+                                                                uint32_t n_shard) {
   const uint32_t u = *ucount;
   if (u > cap && blockIdx.x == 0 && threadIdx.x == 0) *overflow = u;
+  if (first && blockIdx.x == 0 && threadIdx.x == 0) first[cap] = n_shard;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < cap; i += gridDim.x * blockDim.x) {
     if (i < u) {
       const uint2 p = pts[i];
       colours[i] = p.x;
       counts[i] = p.y;
+      if (first) first[i] = first_table[p.x];
     } else {
       counts[i] = 0u;
     }
@@ -236,9 +242,11 @@ __global__ void __launch_bounds__(256) hist_export_padded_kernel(const uint2 *__
 }
 
 // Merge of gathered per-shard lists into the direct table: counts add up exactly; the entry that bumps a
-// counter from 0 appends the colour to the merged unique list.
+// counter from 0 appends the colour to the merged unique list (and, with seen_init, sets its first-seen entry to
+// 0xFFFFFFFF for hist_merge_first_kernel, as hist_insert does for the first-seen pass over pixels).
 __global__ void __launch_bounds__(256) hist_merge_kernel(const uint32_t *__restrict__ colours, const uint32_t *__restrict__ counts,
-                                                        uint32_t n, uint32_t *table, uint32_t *uniq, uint32_t *ucount) {
+                                                        uint32_t n, uint32_t *table, uint32_t *uniq, uint32_t *ucount,
+                                                        uint32_t *seen_init) {
   const uint32_t stride = gridDim.x * blockDim.x;
   const uint32_t round = (n + 31u) & ~31u;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < round; i += stride) {
@@ -252,8 +260,27 @@ __global__ void __launch_bounds__(256) hist_merge_kernel(const uint32_t *__restr
       uint32_t base = 0;
       if (lane == __ffs(m) - 1) base = atomicAdd(ucount, (uint32_t)__popc(m));
       base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-      if (fresh) uniq[base + __popc(m & ((1u << lane) - 1u))] = c;
+      if (fresh) {
+        uniq[base + __popc(m & ((1u << lane) - 1u))] = c;
+        if (seen_init) seen_init[c] = 0xFFFFFFFFu;
+      }
     }
+  }
+}
+
+// First-seen index of every colour over the whole image from the gathered lists: shard w's rows start at the sum of the
+// pixel counts of shards 0..w-1 (rows are contiguous and in rank order), so the image's index of a colour is the minimum
+// over shards of (offset + shard-local index).  colours / counts: [world][cap], first: [world][cap + 1].
+__global__ void __launch_bounds__(256) hist_merge_first_kernel(const uint32_t *__restrict__ colours, const uint32_t *__restrict__ counts,
+                                                              const uint32_t *__restrict__ first, uint32_t cap, uint32_t world,
+                                                              uint32_t *first_seen) {
+  const uint32_t n = world * cap;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    if (counts[i] == 0u) continue;
+    const uint32_t w = i / cap;
+    uint32_t offset = 0;
+    for (uint32_t v = 0; v < w; ++v) offset += first[v * (cap + 1) + cap];
+    atomicMin(first_seen + (colours[i] & 0x00FFFFFFu), offset + first[w * (cap + 1) + (i - w * cap)]);
   }
 }
 
@@ -325,15 +352,24 @@ void hist_export(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t u_hint, 
 }
 
 void hist_export_padded(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t cap, uint32_t *d_colours, uint32_t *d_counts,
-                        uint32_t *d_overflow, int sm_count, cudaStream_t st) {
-  hist_export_padded_kernel<<<blocks_for(cap, 256, sm_count, 8), 256, 0, st>>>(d_pts, d_ucount, cap, d_colours, d_counts, d_overflow);
+                        uint32_t *d_overflow, int sm_count, cudaStream_t st, const uint32_t *d_first_table, uint32_t *d_first,
+                        uint32_t n_shard) {
+  hist_export_padded_kernel<<<blocks_for(cap, 256, sm_count, 8), 256, 0, st>>>(d_pts, d_ucount, cap, d_colours, d_counts, d_overflow,
+                                                                              d_first_table, d_first, n_shard);
   DQ_CUDA_CHECK(cudaGetLastError());
 }
 
 void hist_merge(const uint32_t *d_colours, const uint32_t *d_counts, uint32_t num_entries, uint32_t *d_table, uint32_t *d_uniq,
-                uint32_t *d_ucount, int sm_count, cudaStream_t st) {
+                uint32_t *d_ucount, int sm_count, cudaStream_t st, uint32_t *d_seen_init) {
   hist_merge_kernel<<<blocks_for(num_entries, 256, sm_count, 8), 256, 0, st>>>(d_colours, d_counts, num_entries, d_table, d_uniq,
-                                                                               d_ucount);
+                                                                               d_ucount, d_seen_init);
+  DQ_CUDA_CHECK(cudaGetLastError());
+}
+
+void hist_merge_first(const uint32_t *d_colours, const uint32_t *d_counts, const uint32_t *d_first, uint32_t cap, uint32_t world,
+                      uint32_t *d_first_seen, int sm_count, cudaStream_t st) {
+  hist_merge_first_kernel<<<blocks_for((uint64_t)world * cap, 256, sm_count, 8), 256, 0, st>>>(d_colours, d_counts, d_first, cap, world,
+                                                                                             d_first_seen);
   DQ_CUDA_CHECK(cudaGetLastError());
 }
 

@@ -26,10 +26,17 @@ void order_sort_emit(const uint2 *d_pts, uint32_t u, uint64_t *d_keys, uint32_t 
                      double *d_weights, int sm_count, cudaStream_t st);
 void hist_export(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_colours, uint32_t *d_counts,
                  int sm_count, cudaStream_t st);
+// d_first (optional, cap + 1 words): the shard-local first-seen index of every exported colour (from d_first_table), then
+// n_shard
 void hist_export_padded(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t cap, uint32_t *d_colours, uint32_t *d_counts,
-                        uint32_t *d_overflow, int sm_count, cudaStream_t st);
+                        uint32_t *d_overflow, int sm_count, cudaStream_t st, const uint32_t *d_first_table = nullptr,
+                        uint32_t *d_first = nullptr, uint32_t n_shard = 0);
 void hist_merge(const uint32_t *d_colours, const uint32_t *d_counts, uint32_t num_entries, uint32_t *d_table, uint32_t *d_uniq,
-                uint32_t *d_ucount, int sm_count, cudaStream_t st);
+                uint32_t *d_ucount, int sm_count, cudaStream_t st, uint32_t *d_seen_init = nullptr);
+// After hist_merge with d_seen_init = d_first_seen: the whole image's first-seen index of every merged colour (exported
+// lists [world][cap], first-seen slices [world][cap + 1] as hist_export_padded writes them)
+void hist_merge_first(const uint32_t *d_colours, const uint32_t *d_counts, const uint32_t *d_first, uint32_t cap, uint32_t world,
+                      uint32_t *d_first_seen, int sm_count, cudaStream_t st);
 
 // ---- dq_map.cu ----
 int map_smem_palette_limit();

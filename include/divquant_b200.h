@@ -230,7 +230,10 @@ void dq_colortable_indexes_device(dq_context *ctx, const uint32_t *d_quantPixels
  *       3. dq_shard_quantize_map(ctx, d_all_colours, d_all_counts, M, N_total, d_shard, n_r, d_out_r, &K, palette)
  *     Step 3 merges the lists in the direct table, runs the split on the merged histogram (replicated:
  *     every rank takes identical decisions from identical integers) and remaps the rank's own rows.
- *     Result: exactly dq_quant_recurse of the whole image.
+ *     Result: dq_quant_recurse of the whole image when dq_call_stats::tie_flags is 0.  This form does NOT resolve
+ *     flagged frames (no first-seen indexes travel in its exchange): a frame whose decision sat inside the reference's
+ *     rounding noise (about 1 % of 1080p / 4K G1 frames) is reported in tie_flags and may differ from the reference by
+ *     one LSB in a palette entry.  dq_rows_* below resolves them.
  * ---------------------------------------------------------------------------------------------- */
 /* Unique colours and counts of a shard into caller-provided DEVICE arrays (capacity n_shard each). */
 uint32_t dq_shard_histogram(dq_context *ctx, const uint32_t *d_shard, uint32_t n_shard, uint32_t *d_colours,
@@ -244,14 +247,21 @@ void dq_shard_quantize_map(dq_context *ctx, const uint32_t *d_all_colours, const
  *   rank 0:      dq_rows_unique_id(id)            -> hand the 128 bytes to every rank (any side channel)
  *   every rank:  rows = dq_rows_create(ctx, world, rank, id, list_capacity)          (collective: ncclCommInitRank)
  *   per image:   dq_rows_quant_recurse(rows, d_shard, n_shard, N_total, d_out_shard, &K, palette)
- * One grouped ncclAllGather of fixed-capacity (colour, count) slices per image on the context's stream (unused entries carry
- * count 0: no sizes travel first, no host synchronisation before the palette); list_capacity >= the largest number of
- * unique colours in any shard (a shard that exceeds it is fatal: message + abort).  world = 1 needs no id and no NCCL.
+ * One grouped ncclAllGather per image on the context's stream of three fixed-capacity slices per rank: colours, counts
+ * and the shard-local first-seen index of every colour (plus the shard's pixel count, from which every rank derives the
+ * offset of each shard's rows in the image: rows are contiguous and in rank order).  Unused entries carry count 0: no
+ * sizes travel first, no host synchronisation before the palette.  list_capacity >= the largest number of unique colours
+ * in any shard (a shard that exceeds it is fatal: message + abort); world x (list_capacity + 1) < 2^32.  world = 1 needs no
+ * id and no NCCL.
+ * Every rank merges the lists into its direct table, and the minimum over shards of (offset + local first-seen index) into
+ * the whole image's first-seen index of every colour; the split runs replicated with the tie audit, and a flagged palette
+ * rounding or cut is settled by the resolver (and a forced-cut re-split, which merges the gathered lists again) exactly as
+ * in the single-GPU call.  Every rank takes identical decisions from identical data, so the palette stays replicated.
  * Result: the palette and this rank's rows of dq_quant_recurse of the whole image, PROVIDED the single-GPU call takes the
  * exact-integer kernels for it (more unique colours than dq_context_set_exact_max_points, default 4096: every BASELINE
- * configuration).  Below that limit the single-GPU call adds in the reference's order, which needs the first-seen index of
- * every colour over the WHOLE image; the sharded call does not exchange those and stays on exact integer sums: it then
- * equals the reference unless dq_call_stats::tie_flags says a decision sat inside the reference's rounding noise. */
+ * configuration) and the frame needs no ordered re-run.  The ordered path (small inputs, and flagged axis / hyperplane /
+ * TSE decisions, none of them among the golden frames) needs the whole image in order, which no rank has: such frames stay
+ * on exact integer sums and are reported in dq_call_stats::tie_flags with ordered_rerun = 0. */
 typedef struct dq_rows dq_rows;
 void dq_rows_unique_id(void *out128);
 dq_rows *dq_rows_create(dq_context *ctx, int world, int rank, const void *unique_id128, uint32_t list_capacity);
@@ -300,6 +310,10 @@ dq_context *dq_pipeline_context(dq_pipeline *pipe);
 uint64_t dq_pipeline_kernel_launches(const dq_pipeline *pipe);
 /* Frames whose tie audit raised a flag and that therefore went through the synchronous path a second time. */
 uint64_t dq_pipeline_flagged_frames(const dq_pipeline *pipe);
+/* Frames (since creation) that the resolver settled (dq_call_stats::tie_resolved or cut_overrides > 0), and frames that were
+ * computed again on the ordered path (dq_call_stats::ordered_rerun = 1). */
+uint64_t dq_pipeline_resolved_frames(const dq_pipeline *pipe);
+uint64_t dq_pipeline_rerun_frames(const dq_pipeline *pipe);
 int dq_pipeline_lanes(const dq_pipeline *pipe);
 /* Lane threads spin while they wait for the GPU (lowest latency; default) or, with enabled = 1, sleep on an event:
  * use it when the pipeline has more lanes than the process has free host cores (several ranks on one host). */

@@ -124,19 +124,21 @@ class Oracle:
         return out if ok else None
 
     # -- quantize -------------------------------------------------------------------------
-    def quant_varpart_resolved(self, pixels, k, num_bits=8, dec_factor=1, max_iters=10):
+    def quant_varpart_resolved(self, pixels, k, num_bits=8, dec_factor=1, max_iters=10, rows=1, cols=None):
         """CPU model of the device's DEFAULT large-input path: exact integer sums + tie audit + the resolver (palette
         roundings and cuts settled by the reference's own mean of the node, csrc/dq_resolve.cu).  Returns (palette,
         info) with info = {"left": decisions still flagged (axis / hyperplane / TSE), "roundings": ..., "cuts_confirmed": ...,
-        "cuts_forced": ...}; with left == 0 the palette must be the reference's."""
+        "cuts_forced": ...}; with left == 0 the palette must be the reference's.  rows / cols: the sampling grid of
+        calc_color_table, as in quant_varpart_fast."""
         px = _u32(pixels)
+        cols = px.size if cols is None else cols
         ct = np.zeros(max(k, 1), np.uint32)
         nk = C.c_uint32(k)
         flags = np.zeros(9, np.uint32)
         fn = self.lib.oracle_quant_varpart_fast_exact_resolved
         fn.restype = C.c_int
         fn.argtypes = [C.c_uint32, _u32p, C.c_uint32, C.c_uint32, _u32p, _u32p, C.c_int, C.c_int, C.c_int, C.c_int, _u32p]
-        fn(px.size, _ptr(px), 1, px.size, C.byref(nk), _ptr(ct), num_bits, dec_factor, max_iters, 0, _ptr(flags))
+        fn(px.size, _ptr(px), rows, cols, C.byref(nk), _ptr(ct), num_bits, dec_factor, max_iters, 0, _ptr(flags))
         return ct[:nk.value].copy(), {"left": int(flags[0]), "roundings": int(flags[6]), "cuts_confirmed": int(flags[7]),
                                       "cuts_forced": int(flags[8]), "left_axis": int(flags[1]), "left_hyperplane": int(flags[3]),
                                       "left_tse": int(flags[4])}

@@ -29,8 +29,8 @@ def test_row_sharded_single_rank(built):
 
 
 def test_row_sharded_few_colours_single_rank(built):
-    # 320x180 G1 has 43 411 colours: below the ordered path's limit the sharded call stays on exact integer sums (it has
-    # no whole-image first-seen order); rows_check fails if that ever differs from the single-GPU call without a tie flag
+    # 320x180 G1 at K=64: the sharded call stays on exact integer sums (it has no ordered path: that needs the whole image
+    # in order); rows_check fails if that ever differs from the single-GPU call
     _run(1, 320, 180, 64)
 
 

@@ -124,7 +124,6 @@ def load_library(path=LIB_PATH):
         "dq_debug_histogram": (C.c_uint32, [vp, _u32p, C.c_uint32, _u32p, _u32p]),
         "dq_debug_split_timeline": (C.c_uint32, [vp, C.c_int, C.POINTER(C.c_uint64), C.c_uint32]),
         "dq_host_dedup_palette": (C.c_uint32, [_u32p, C.c_uint32]),
-        "dq_host_sort_permutation": (None, [_u32p, C.c_int, C.c_int, _u32p]),
         "dq_host_select_cut_overrides": (C.c_uint32, [_u32p, _u32p, _u32p, C.c_uint32, C.c_uint32, _u32p]),
         "dq_host_build_search_tables": (None, [_u32p, C.c_int, _u32p, C.POINTER(C.c_int32)]),
     }
@@ -143,7 +142,7 @@ EXPORTED_C_SYMBOLS = [
     "dq_srm_num_pairs", "dq_srm_sorted_edges", "dq_srm_sorted_edges_device", "dq_context_set_split_ctas", "dq_context_set_exact_small", "dq_context_set_exact_max_points", "dq_context_set_tie_policy", "dq_pixel_histogram", "dq_block_vote", "dq_block_vote_device", "dq_quant_blocks", "dq_colortable_indexes", "dq_colortable_indexes_device", "dq_shard_histogram", "dq_shard_quantize_map", "dq_rows_unique_id", "dq_rows_create", "dq_rows_destroy", "dq_rows_quant_recurse", "dq_pipeline_create", "dq_pipeline_create_lanes", "dq_pipeline_destroy", "dq_pipeline_submit", "dq_pipeline_submit_device", "dq_pipeline_wait", "dq_pipeline_lanes", "dq_pipeline_set_blocking_wait", "dq_pipeline_flush", "dq_pipeline_last_elapsed_ms",
     "dq_pipeline_context", "dq_pipeline_kernel_launches", "dq_pipeline_flagged_frames",
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
-    "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_sort_permutation", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
+    "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
 ]
 
 # The reference's own symbol names (SURVEY.md 8b), exported for relinking the reference's callers.

@@ -27,7 +27,6 @@
 #include "../../include/divquant_b200.h"
 #include "dq_kernels.cuh"
 #include "dq_split.cuh"
-#include "dq_stdsort.cuh"
 
 namespace {
 
@@ -111,7 +110,6 @@ struct dq_context {
   uint32_t exact_max_points = kExactDefaultPoints;  // ... up to this many unique colours (DIVQUANT_B200_EXACT_MAX)
   DevBuf<uint64_t> d_exact;
   DevBuf<uint32_t> d_tie;  // flagged clusters / nodes, resolver status words, a counter (layout: dq_split.cuh, kTieListWords)
-  DevBuf<FrameResult> d_frame;  // frame pipeline: what palette_post hands back (device side)
   // a split that has been launched but whose palette has not been collected yet (run_split / run_split_finish)
   struct PendingSplit {
     SplitArgs a;
@@ -263,7 +261,7 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out, dq_split_re
 uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32_t K, int max_iters, int num_bits,
                    uint32_t *colortable_out, dq_split_record *records_out, double *mean_out, uint32_t *size_out,
                    bool collect_from_hist = false, const ExactSource *exact = nullptr, bool weighted = false,
-                   bool launch_only = false, bool defer = false) {
+                   bool defer = false) {
   if (max_iters < 1 || max_iters > kSplitMaxIters) {
     fprintf(stderr, "divquant_b200: max_iters ( %d ) must be in [1,%d] (the reference hard-wires local k-means on)\n",
             max_iters, kSplitMaxIters);
@@ -355,7 +353,7 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
     x.collect_table = collect_from_hist ? ctx->d_table : nullptr;
     if (getenv("DQ_PROFILE_NARROW")) DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_progress.ptr, 0, 1024 * sizeof(uint32_t), ctx->stream));
     const bool mail = ctx->use_mailbox && !ctx->blocking_wait && !ctx->trace_split && records_out == nullptr &&
-                      mean_out == nullptr && size_out == nullptr && !launch_only;
+                      mean_out == nullptr && size_out == nullptr;
     if (mail) {
       void *dev = nullptr;
       DQ_CUDA_CHECK(cudaHostGetDevicePointer(&dev, const_cast<uint32_t *>(ctx->mailbox), 0));
@@ -389,7 +387,6 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   }
   ctx->mark(3);
   ctx->stats.kernel_launches++;
-  if (launch_only) return 0;  // frame pipeline: the palette stays on the device (palette_post), nothing to wait for
   ctx->pend.a = a;
   ctx->pend.use_v2 = use_v2;
   ctx->pend.K = K;
@@ -598,7 +595,7 @@ void quantize_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t 
   const ExactSource src = {d_in, rows, cols, (uint32_t)dec, num_bits};
   uint32_t unused = 0;
   run_split(ctx, point_cap, norm, K, max_iters, num_bits, &unused, records, mean_out, size_out, table_dirty,
-            table_dirty ? &src : nullptr, table_dirty, false, /*defer=*/true);
+            table_dirty ? &src : nullptr, table_dirty, /*defer=*/true);
   dq_context::QuantState &q = ctx->qs;
   q.n = n, q.rows = rows, q.cols = cols, q.K = K, q.point_cap = point_cap, q.d_in = d_in;
   q.num_bits = num_bits, q.dec = dec, q.max_iters = max_iters, q.norm = norm, q.table_dirty = table_dirty;
@@ -665,8 +662,7 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     reset_control(ctx);
     run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
     uint32_t unused = 0;
-    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true, &src, true,
-              false, /*defer=*/true);
+    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true, &src, true, /*defer=*/true);
     ctx->exact_max_points = keep;
     q.phase = 2;
   };
@@ -683,7 +679,7 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     uint32_t unused = 0;
     ctx->ovr_active = true;
     run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true,
-              merged ? nullptr : &src, true, false, /*defer=*/true);
+              merged ? nullptr : &src, true, /*defer=*/true);
     ctx->ovr_active = false;
     q.resplits++;
     q.phase = 0;
@@ -876,12 +872,12 @@ void recurse_remap_tail(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint3
 }
 
 void quant_recurse_device_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout,
-                               uint32_t *colortable, int all_unique, double *ms_quant, double *ms_map, bool final_sync = true) {
+                               uint32_t *colortable, int all_unique, double *ms_quant, double *ms_map) {
   auto t0 = std::chrono::steady_clock::now();
   recurse_begin(ctx, n, d_in, *k_inout, all_unique);
   auto t1 = t0;
   recurse_remap(ctx, n, d_in, d_out, k_inout, colortable, &t1);  // waits for the palette, then queues the remap
-  if (final_sync || ctx->profiling) ctx->wait();
+  ctx->wait();
   if (ctx->profiling) {
     auto span = [&](int a, int b) {
       float ms = 0.f;
@@ -899,57 +895,6 @@ void quant_recurse_device_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in
   auto t2 = std::chrono::steady_clock::now();
   if (ms_quant) *ms_quant = std::chrono::duration<double, std::milli>(t1 - t0).count();
   if (ms_map) *ms_map = std::chrono::duration<double, std::milli>(t2 - t1).count();
-}
-
-// Frame pipeline: the whole of one quant_recurse queued on the context's stream without a single host wait -- histogram,
-// split, palette handling on the device (duplicates, the reference's std::sort order, lut_init: palette_post), remap
-// through the unique-colour table, and one small copy of the FrameResult to pinned host memory.  The host looks at the
-// frame only once it is complete (frame_async_collect).
-bool frame_async_supported(const dq_context *ctx, uint32_t K, int all_unique) {
-  return !all_unique && ctx->split_version == 2 && K <= kSplit2MaxColors && K <= (uint32_t)kFrameMaxColors && K >= 1;
-}
-
-void frame_async_enqueue(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t K, FrameResult *h_frame) {
-  check_quant_args(n, K, 8);
-  reset_control(ctx);
-  ctx->d_pts0.ensure(n);
-  run_histogram(ctx, d_in, n, 1, n, 1, 8);
-  const ExactSource src = {d_in, 1, n, 1, 8};
-  uint32_t unused = 0;
-  run_split(ctx, n, sample_norm(1, n, 1), K, 10, 8, &unused, nullptr, nullptr, nullptr, true, &src, true, /*launch_only=*/true);
-  ctx->d_sorted.ensure((size_t)K + kLutEntries);
-  ctx->d_frame.ensure(1);
-  palette_post(ctx->d_palette.ptr, ctx->d_cb->result, ctx->d_cb->ctl, &ctx->d_cb->ucount, (int)K, ctx->d_sorted.ptr, ctx->d_frame.ptr,
-               ctx->stream);
-  map_unique_dev(ctx->d_uniq.ptr, &ctx->d_cb->ucount, n, ctx->d_map, ctx->d_sorted.ptr, (int)K, ctx->d_frame.ptr, ctx->sm_count,
-                 ctx->stream);
-  map_gather(d_in, n, d_out, ctx->d_map, ctx->sm_count, ctx->stream);
-  DQ_CUDA_CHECK(cudaMemcpyAsync(h_frame, ctx->d_frame.ptr, sizeof(FrameResult), cudaMemcpyDeviceToHost, ctx->stream));
-  ctx->stats.kernel_launches += 3;
-}
-
-// The frame is complete (its stream position has been waited for).  Returns true when the palette in h_frame is final;
-// false when the tie audit flagged the frame (the caller runs it again through the synchronous path, which resolves it).
-bool frame_async_collect(dq_context *ctx, const FrameResult *h_frame, uint32_t K, uint32_t *k_out, uint32_t *colortable) {
-  if (h_frame->ctl[kCtlError] != 0) {
-    fprintf(stderr, "divquant_b200: split controller failed (code %u, frame pipeline; internal error)\n", h_frame->ctl[kCtlError]);
-    abort();
-  }
-  const uint32_t flags = (ctx->tie_policy != 0) ? h_frame->ctl[kCtlTie] : 0u;
-  if (flags != 0u && ctx->tie_policy == 2) return false;
-  const uint32_t k = h_frame->num_colors;
-  if (h_frame->result[1]) fprintf(stderr, "# empty clusters: %d\n", (int)h_frame->result[1]);  // (:1067-1070)
-  memcpy(colortable, h_frame->palette, (size_t)k * sizeof(uint32_t));
-  *k_out = k;
-  ctx->stats.num_points = h_frame->num_points;
-  ctx->stats.requested_colors = K;
-  ctx->stats.actual_colors = k;
-  ctx->stats.empty_clusters = h_frame->result[1];
-  ctx->stats.split_rounds = h_frame->ctl[kCtlRounds];
-  ctx->stats.splits_computed = h_frame->ctl[kCtlSplits];
-  ctx->stats.tie_flags = flags;
-  ctx->stats.remap_path = 2;
-  return true;
 }
 
 std::mutex g_default_mutex;
@@ -996,21 +941,6 @@ uint32_t dq_host_select_cut_overrides(const uint32_t *begin, const uint32_t *siz
   const uint32_t added = select_cut_overrides(rec, status, n, out, &n_out, kCutOverrideCap);
   for (uint32_t k = 0; k < added; ++k) picked_out[k] = (uint32_t)out[first + k].mean_here;  // the entry's index
   return added;
-}
-
-void dq_host_sort_permutation(const uint32_t *keys, int n, int use_replay, uint32_t *perm_out) {
-  if (n <= 0) return;
-  if (use_replay) {  // csrc/dq_stdsort.cuh, the code the device runs
-    std::vector<uint32_t> v((size_t)n);
-    for (int i = 0; i < n; ++i) v[i] = (keys[i] << 16) | (uint32_t)i;
-    stdsort::sort(v.data(), n);
-    for (int i = 0; i < n; ++i) perm_out[i] = v[i] & 0xFFFFu;
-  } else {  // std::sort on the reference's element type and comparator
-    std::vector<PaletteEntry> v((size_t)n);
-    for (int i = 0; i < n; ++i) v[i].red = i, v[i].green = v[i].blue = 0, v[i].weight = (int)keys[i];
-    std::sort(v.begin(), v.end(), palette_less);
-    for (int i = 0; i < n; ++i) perm_out[i] = (uint32_t)v[i].red;
-  }
 }
 
 dq_context *dq_context_create(int device) {
@@ -1103,7 +1033,6 @@ void dq_context_destroy(dq_context *ctx) {
   ctx->d_ovr.release();
   ctx->d_flat.release();
   ctx->d_sortvals.release();
-  ctx->d_frame.release();
   cudaFree(ctx->d_table);
   cudaFree(ctx->d_map);
   cudaFree(ctx->d_cb);
@@ -1514,9 +1443,9 @@ void dq_shard_quantize_map(dq_context *ctx, const uint32_t *d_all_colours, const
 // ---- frame pipeline: lanes ------------------------------------------------------------------------------------
 // One frame's critical path is a chain of ~100 dependent passes inside the persistent split kernel, which keeps
 // most of the GPU idle.  Frames are independent, so the pipeline runs `lanes` of them side by side: every lane
-// owns a context (stream, tables, scratch), a pair of frame buffers and a host thread that walks one frame at a
-// time through H2D -> kernels -> D2H.  Split kernels of different lanes occupy disjoint groups of SMs
-// (dq_context_set_split_ctas); histogram / remap kernels and the copy engines fill in around them.
+// owns a context (stream, tables, scratch) and a pair of frame buffers, and one host thread (pipeline_dispatcher)
+// walks each lane's frames, one at a time, through H2D -> kernels -> D2H.  Split kernels of different lanes occupy
+// disjoint groups of SMs (dq_context_set_split_ctas); histogram / remap kernels and the copy engines fill in around them.
 struct dq_pipeline {
   struct Job {
     uint64_t ticket = 0;
@@ -1531,12 +1460,9 @@ struct dq_pipeline {
     uint32_t *d_in = nullptr, *d_out = nullptr;
     cudaEvent_t begin = nullptr, end = nullptr;
     bool have_begin = false;
-    FrameResult *h_frame[2] = {nullptr, nullptr};  // pinned: result of the frame queued on the lane's stream (asynchronous chain)
-    cudaEvent_t done[2] = {nullptr, nullptr};
+    cudaEvent_t done = nullptr;
     // dispatcher state
     int state = 0;
-    bool async_chain = false;
-    uint64_t launches = 0;
     Job job;
   };
   int device = 0;
@@ -1549,16 +1475,11 @@ struct dq_pipeline {
   uint64_t submitted = 0, low_water = 0;  // every ticket < low_water has completed
   bool stop = false;
   std::atomic<uint64_t> launches{0};
-  std::atomic<uint64_t> flagged_frames{0};  // frames the tie audit sent through the synchronous path
+  std::atomic<uint64_t> flagged_frames{0};  // frames whose tie audit raised a flag
   std::atomic<uint64_t> resolved_frames{0};  // ... settled by the resolver / forced cuts (dq_call_stats::tie_resolved, cut_overrides)
   std::atomic<uint64_t> rerun_frames{0};     // ... computed again on the ordered path (dq_call_stats::ordered_rerun)
-  // DIVQUANT_B200_ASYNC=1: the whole chain of a frame is queued without a host wait (palette handling on the device,
-  // palette_post).  Off by default: measured at 4K, 12 lanes, it is slower than the host round trip (0.184-0.22 against
-  // 0.166 ms/frame): the one-thread std::sort replay costs 93 us per frame on the lane's chain and the lanes' throughput
-  // is bounded by the histogram / remap kernels sharing the SMs the split kernels leave free, not by the host.
-  int async_frames = 0;
   int poll_sleep = 0;    // the dispatcher sleeps 20 us between polling rounds instead of spinning (dq_pipeline_set_blocking_wait)
-  std::vector<std::thread> dispatchers;
+  std::thread dispatcher;
   float last_ms = 0.f;
 };
 
@@ -1583,63 +1504,30 @@ void pipeline_complete(dq_pipeline *p, uint64_t ticket, uint64_t launches) {
   p->cv_done.notify_all();
 }
 
-// One frame through the blocking path, start to end (frames the tie audit flagged in the asynchronous chain).
-void pipeline_run_sync(dq_pipeline *p, dq_pipeline::Lane &lane, const dq_pipeline::Job &job) {
-  dq_context *ctx = lane.ctx;
-  const uint32_t *d_in = job.in;
-  uint32_t *d_out = job.out;
-  if (!job.device_ptrs) {
-    d_in = lane.d_in;
-    d_out = lane.d_out;
-    DQ_CUDA_CHECK(cudaMemcpyAsync(lane.d_in, job.in, (size_t)job.n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  }
-  memset(&ctx->stats, 0, sizeof(ctx->stats));
-  ctx->stats.num_pixels = job.n;
-  quant_recurse_device_impl(ctx, job.n, d_in, d_out, job.k_ptr, job.colortable, job.all_unique, nullptr, nullptr, false);
-  if (!job.device_ptrs)
-    DQ_CUDA_CHECK(cudaMemcpyAsync(job.out, lane.d_out, (size_t)job.n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  DQ_CUDA_CHECK(cudaEventRecord(lane.end, ctx->stream));
-  ctx->wait();
-  pipeline_count_ties(p, ctx);
-  pipeline_complete(p, job.ticket, ctx->stats.kernel_launches);
-}
-
-// The dispatcher: ONE host thread walks the frames of all its lanes through the GPU.  A lane is a small state machine
+// The dispatcher: ONE host thread walks the frames of all lanes through the GPU.  A lane is a small state machine
 //   idle -> [H2D] histogram + split queued -> (palette arrives in the lane's mailbox) host palette handling, remap [+ D2H]
 //        queued -> (the lane's event fires) frame complete -> idle
 // and the thread only ever polls: mailboxes are host memory, events are cudaEventQuery.  Nothing sleeps on the GPU and
-// nothing spins per lane, so the pipeline needs one busy host core per dispatcher however many lanes it feeds (round 1
+// nothing spins per lane, so the pipeline needs one busy host core however many lanes it feeds (round 1
 // had a spinning thread per lane, and lost a quarter of its throughput where ranks had fewer cores than lanes).
-void pipeline_dispatcher(dq_pipeline *p, int first_lane, int lane_step) {
-  require_device(p->lanes[first_lane].ctx);
+void pipeline_dispatcher(dq_pipeline *p) {
+  require_device(p->lanes[0].ctx);
   enum { kIdle = 0, kWaitSplit = 1, kWaitDone = 2 };
   for (;;) {
     bool progress = false;
     int busy = 0;
-    for (size_t li = (size_t)first_lane; li < p->lanes.size(); li += (size_t)lane_step) {
-      dq_pipeline::Lane &lane = p->lanes[li];
+    for (dq_pipeline::Lane &lane : p->lanes) {
       dq_context *ctx = lane.ctx;
       if (lane.state == kWaitDone) {
-        if (cudaEventQuery(lane.done[0]) == cudaErrorNotReady) {
+        if (cudaEventQuery(lane.done) == cudaErrorNotReady) {
           ++busy;
           continue;
         }
         progress = true;
         lane.state = kIdle;
-        if (lane.async_chain) {
-          uint32_t k = 0;
-          if (frame_async_collect(ctx, lane.h_frame[0], *lane.job.k_ptr, &k, lane.job.colortable)) {
-            *lane.job.k_ptr = k;
-            pipeline_complete(p, lane.job.ticket, lane.launches);
-          } else {
-            p->flagged_frames++;
-            pipeline_run_sync(p, lane, lane.job);
-          }
-        } else {
-          if (ctx->stats.tie_flags) p->flagged_frames++;
-          pipeline_count_ties(p, ctx);
-          pipeline_complete(p, lane.job.ticket, ctx->stats.kernel_launches);
-        }
+        if (ctx->stats.tie_flags) p->flagged_frames++;
+        pipeline_count_ties(p, ctx);
+        pipeline_complete(p, lane.job.ticket, ctx->stats.kernel_launches);
       } else if (lane.state == kWaitSplit) {
         ++busy;
         if (!quantize_pending_ready(ctx)) continue;
@@ -1652,14 +1540,13 @@ void pipeline_dispatcher(dq_pipeline *p, int first_lane, int lane_step) {
         recurse_remap_tail(ctx, job.n, d_in, d_out, job.k_ptr, job.colortable);
         if (!job.device_ptrs)
           DQ_CUDA_CHECK(cudaMemcpyAsync(job.out, lane.d_out, (size_t)job.n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        DQ_CUDA_CHECK(cudaEventRecord(lane.done[0], ctx->stream));
+        DQ_CUDA_CHECK(cudaEventRecord(lane.done, ctx->stream));
         DQ_CUDA_CHECK(cudaEventRecord(lane.end, ctx->stream));
         lane.state = kWaitDone;
       }
     }
     // new frames for the idle lanes
-    for (size_t li = (size_t)first_lane; li < p->lanes.size(); li += (size_t)lane_step) {
-      dq_pipeline::Lane &lane = p->lanes[li];
+    for (dq_pipeline::Lane &lane : p->lanes) {
       if (lane.state != kIdle) continue;
       {
         std::lock_guard<std::mutex> lock(p->mu);
@@ -1675,28 +1562,13 @@ void pipeline_dispatcher(dq_pipeline *p, int first_lane, int lane_step) {
         DQ_CUDA_CHECK(cudaEventRecord(lane.begin, ctx->stream));
         lane.have_begin = true;
       }
-      const uint32_t *d_in = job.in;
-      uint32_t *d_out = job.out;
-      if (!job.device_ptrs) {
-        d_in = lane.d_in;
-        d_out = lane.d_out;
+      const uint32_t *d_in = job.device_ptrs ? job.in : lane.d_in;
+      if (!job.device_ptrs)
         DQ_CUDA_CHECK(cudaMemcpyAsync(lane.d_in, job.in, (size_t)job.n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-      }
       memset(&ctx->stats, 0, sizeof(ctx->stats));
       ctx->stats.num_pixels = job.n;
-      lane.async_chain = p->async_frames && frame_async_supported(ctx, *job.k_ptr, job.all_unique);
-      if (lane.async_chain) {
-        frame_async_enqueue(ctx, job.n, d_in, d_out, *job.k_ptr, lane.h_frame[0]);
-        if (!job.device_ptrs)
-          DQ_CUDA_CHECK(cudaMemcpyAsync(job.out, lane.d_out, (size_t)job.n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        DQ_CUDA_CHECK(cudaEventRecord(lane.done[0], ctx->stream));
-        DQ_CUDA_CHECK(cudaEventRecord(lane.end, ctx->stream));
-        lane.launches = ctx->stats.kernel_launches;
-        lane.state = kWaitDone;
-      } else {
-        recurse_begin(ctx, job.n, d_in, *job.k_ptr, job.all_unique);
-        lane.state = kWaitSplit;
-      }
+      recurse_begin(ctx, job.n, d_in, *job.k_ptr, job.all_unique);
+      lane.state = kWaitSplit;
     }
     if (progress) continue;
     if (busy == 0) {
@@ -1758,15 +1630,9 @@ dq_pipeline *dq_pipeline_create_lanes(int device, uint32_t max_pixels, int lanes
     }
     DQ_CUDA_CHECK(cudaEventCreate(&lane.begin));
     DQ_CUDA_CHECK(cudaEventCreate(&lane.end));
-    for (int s = 0; s < 2; ++s) {
-      DQ_CUDA_CHECK(cudaMallocHost(&lane.h_frame[s], sizeof(FrameResult)));
-      DQ_CUDA_CHECK(cudaEventCreateWithFlags(&lane.done[s], cudaEventBlockingSync | cudaEventDisableTiming));
-    }
+    DQ_CUDA_CHECK(cudaEventCreateWithFlags(&lane.done, cudaEventBlockingSync | cudaEventDisableTiming));
   }
-  if (const char *e = getenv("DIVQUANT_B200_ASYNC")) p->async_frames = (e[0] != '0');
-  int n_disp = 1;  // host threads that drive the lanes (each polls its share of them)
-  if (const char *e = getenv("DIVQUANT_B200_DISPATCHERS")) n_disp = std::min(std::max(atoi(e), 1), lanes);
-  for (int i = 0; i < n_disp; ++i) p->dispatchers.emplace_back(pipeline_dispatcher, p, i, n_disp);
+  p->dispatcher = std::thread(pipeline_dispatcher, p);
   return p;
 }
 
@@ -1789,17 +1655,14 @@ void dq_pipeline_destroy(dq_pipeline *p) {
     p->stop = true;
   }
   p->cv_work.notify_all();
-  for (auto &t : p->dispatchers) t.join();
+  p->dispatcher.join();
   for (auto &lane : p->lanes) {
     require_device(lane.ctx);
     cudaFree(lane.d_in);
     cudaFree(lane.d_out);
     cudaEventDestroy(lane.begin);
     cudaEventDestroy(lane.end);
-    for (int s = 0; s < 2; ++s) {
-      cudaFreeHost(lane.h_frame[s]);
-      cudaEventDestroy(lane.done[s]);
-    }
+    cudaEventDestroy(lane.done);
     dq_context_destroy(lane.ctx);
   }
   delete p;
@@ -2102,8 +1965,7 @@ void dq_rows_quant_recurse(dq_rows *r, const uint32_t *d_shard, uint32_t n_shard
   reset_control(ctx);
   run_merge(ctx, q.merged);
   uint32_t k = 0;
-  run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &k, nullptr, nullptr, nullptr, true, nullptr, true, false,
-            /*defer=*/true);
+  run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &k, nullptr, nullptr, nullptr, true, nullptr, true, /*defer=*/true);
   k = K;
   quantize_finish(ctx, &k, outColortablePtr);
   k = dedup_palette(outColortablePtr, k);

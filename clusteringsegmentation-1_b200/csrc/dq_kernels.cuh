@@ -52,24 +52,6 @@ struct MapTablesParam {
 };
 void map_unique_params(const MapTablesParam &tables, const uint32_t *d_uniq, const uint32_t *d_ucount, uint32_t u_hint,
                        uint32_t *d_table, int num_colors, int sm_count, cudaStream_t st);
-// ---- palette handling on the device (frame pipeline): quant_util.cpp:93-118 + DivQuantMapColors.cpp:267-383 ----
-// What a frame of the pipeline hands back to the host in one copy.
-constexpr int kFrameMaxColors = 512;
-struct FrameResult {
-  uint32_t num_colors;      // palette entries after the duplicates are dropped
-  uint32_t num_points;      // U
-  uint32_t result[4];       // SplitArgs::result
-  uint32_t ctl[16];         // SplitArgs::ctl (kCtlWords <= 16)
-  uint32_t palette[kFrameMaxColors];  // first occurrence of every word, order kept (quant_util.cpp:93-118)
-};
-// One CTA: drops duplicate palette words, orders the rest by r+g+b exactly as the reference's std::sort does
-// (dq_stdsort.cuh), builds lut_init.  d_sorted: [max_colors palette words | 766 lut entries] as upload_search_tables lays
-// them out; d_frame receives the FrameResult.
-void palette_post(const uint32_t *d_palette, const uint32_t *d_result, const uint32_t *d_ctl, const uint32_t *d_ucount,
-                  int max_colors, uint32_t *d_sorted, FrameResult *d_frame, cudaStream_t st);
-// map_unique with the number of colours read from the device (FrameResult::num_colors).
-void map_unique_dev(const uint32_t *d_uniq, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_table, const uint32_t *d_sorted,
-                    int max_colors, const FrameResult *d_frame, int sm_count, cudaStream_t st);
 void block_vote(const uint32_t *d_quant, uint32_t width, uint32_t height, uint32_t dim, uint32_t *d_blocks, int sm_count,
                 cudaStream_t st);
 void map_labels(const uint32_t *d_in, uint32_t n, uint32_t *d_out, const uint2 *d_pairs, int num_pairs, int greyscale,

@@ -19,7 +19,6 @@
 #include <atomic>
 
 #include "dq_kernels.cuh"
-#include "dq_stdsort.cuh"
 
 namespace dq {
 namespace {
@@ -317,85 +316,6 @@ __global__ void __launch_bounds__(kMapThreads) map_unique_fast_kernel(const uint
   map_unique_fast_body(uniq, ucount, table, sorted, num_colors, lut_init);
 }
 
-// Same, the number of colours comes from the device (the palette never went to the host): shared memory is sized for
-// max_colors at launch, the tables sit at [max_colors words | lut].
-__global__ void __launch_bounds__(kMapThreads) map_unique_fast_dev_kernel(const uint32_t *__restrict__ uniq, const uint32_t *ucount,
-                                                                         uint32_t *table, const uint32_t *sorted, int max_colors,
-                                                                         const FrameResult *frame) {
-  const int num_colors = (int)frame->num_colors;
-  if (num_colors <= 0 || num_colors > max_colors) return;  // (an error exit of the split kernel: the host reports it)
-  map_unique_fast_body(uniq, ucount, table, sorted, num_colors, reinterpret_cast<const int *>(sorted + max_colors));
-}
-
-// ---- palette handling on the device -------------------------------------------------------------------------
-constexpr int kPostThreads = 256;
-__global__ void __launch_bounds__(kPostThreads) palette_post_kernel(const uint32_t *palette, const uint32_t *result,
-                                                                   const uint32_t *ctl, const uint32_t *ucount, int max_colors,
-                                                                   uint32_t *sorted, FrameResult *frame) {
-  __shared__ uint32_t s_pal[kFrameMaxColors], s_keep[kFrameMaxColors], s_word[kFrameMaxColors];
-  __shared__ int s_warp[kPostThreads / 32];
-  __shared__ int s_n;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  int n0 = (int)result[0];
-  if (n0 > max_colors || n0 > kFrameMaxColors) n0 = 0;  // never on a healthy run; the host sees ctl / result itself
-  for (int i = tid; i < n0; i += kPostThreads) s_pal[i] = palette[i];
-  if (tid == 0) s_n = 0;
-  __syncthreads();
-  // first occurrence of each word survives, order kept (quant_util.cpp:93-118)
-  for (int base = 0; base < n0; base += kPostThreads) {
-    const int i = base + tid;
-    bool keep = false;
-    if (i < n0) {
-      keep = true;
-      const uint32_t w = s_pal[i];
-      for (int j = 0; j < i; ++j) keep = keep && (s_pal[j] != w);
-    }
-    const unsigned ballot = __ballot_sync(0xffffffffu, keep);
-    if (lane == 0) s_warp[warp] = __popc(ballot);
-    __syncthreads();
-    int before = s_n;
-    for (int q = 0; q < warp; ++q) before += s_warp[q];
-    if (keep) s_keep[before + __popc(ballot & ((1u << lane) - 1u))] = s_pal[i];
-    __syncthreads();
-    if (tid == 0) {
-      int tot = 0;
-      for (int q = 0; q < kPostThreads / 32; ++q) tot += s_warp[q];
-      s_n += tot;
-    }
-    __syncthreads();
-  }
-  const int n = s_n;
-  // sort by r+g+b: the reference's std::sort, step for step (one thread; a few thousand element moves)
-  for (int i = tid; i < n; i += kPostThreads) {
-    const uint32_t p = s_keep[i];
-    s_word[i] = ((((p >> 16) & 0xFF) + ((p >> 8) & 0xFF) + (p & 0xFF)) << 16) | (uint32_t)i;
-  }
-  __syncthreads();
-  if (tid == 0) stdsort::sort(s_word, n);
-  __syncthreads();
-  int *lut = reinterpret_cast<int *>(sorted + max_colors);
-  for (int i = tid; i < n; i += kPostThreads) sorted[i] = s_keep[s_word[i] & 0xFFFFu];
-  // lut_init (DivQuantMapColors.cpp:331-383): entry ic owns the sums from the rounded midpoint to its lower neighbour up
-  // to the rounded midpoint to its upper neighbour; (int)(0.5 (a + b) + 0.5) == (a + b + 1) >> 1 for these integers
-  if (n == 1) {
-    for (int k = tid; k < (int)kLutEntries; k += kPostThreads) lut[k] = 0;
-  } else if (n >= 2) {
-    for (int ic = tid; ic < n; ic += kPostThreads) {
-      const int w = (int)(s_word[ic] >> 16);
-      const int low = (ic == 0) ? 0 : (((int)(s_word[ic - 1] >> 16) + w + 1) >> 1);
-      const int high = (ic == n - 1) ? (int)kLutEntries : ((w + (int)(s_word[ic + 1] >> 16) + 1) >> 1);
-      for (int k = low; k < high; ++k) lut[k] = ic;
-    }
-  }
-  for (int i = tid; i < n; i += kPostThreads) frame->palette[i] = s_keep[i];
-  if (tid < 4) frame->result[tid] = result[tid];
-  if (tid < 16) frame->ctl[tid] = (tid < 12) ? ctl[tid] : 0u;
-  if (tid == 0) {
-    frame->num_colors = (uint32_t)n;
-    frame->num_points = *ucount;
-  }
-}
-
 // Tables inside the parameter block (constant bank): K <= 256.
 __global__ void __launch_bounds__(kMapThreads) map_unique_fast_param_kernel(const __grid_constant__ MapTablesParam tables,
                                                                            const uint32_t *__restrict__ uniq,
@@ -616,22 +536,6 @@ void map_unique_params(const MapTablesParam &tables, const uint32_t *d_uniq, con
   int per_sm = (int)std::min<size_t>(8, std::max<size_t>(1, (200 * 1024) / smem));
   map_unique_fast_param_kernel<<<blocks_for(u_hint / kUniqPix + 1, kMapThreads, sm_count, per_sm), kMapThreads, smem, st>>>(
       tables, d_uniq, d_ucount, d_table, num_colors);
-  DQ_CUDA_CHECK(cudaGetLastError());
-}
-
-void palette_post(const uint32_t *d_palette, const uint32_t *d_result, const uint32_t *d_ctl, const uint32_t *d_ucount,
-                  int max_colors, uint32_t *d_sorted, FrameResult *d_frame, cudaStream_t st) {
-  palette_post_kernel<<<1, kPostThreads, 0, st>>>(d_palette, d_result, d_ctl, d_ucount, max_colors, d_sorted, d_frame);
-  DQ_CUDA_CHECK(cudaGetLastError());
-}
-
-void map_unique_dev(const uint32_t *d_uniq, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_table, const uint32_t *d_sorted,
-                    int max_colors, const FrameResult *d_frame, int sm_count, cudaStream_t st) {
-  const size_t smem = fast_smem_bytes(max_colors);
-  DQ_RAISE_SMEM(map_unique_fast_dev_kernel, smem);
-  int per_sm = (int)std::min<size_t>(8, std::max<size_t>(1, (200 * 1024) / smem));
-  map_unique_fast_dev_kernel<<<blocks_for(u_hint / kUniqPix + 1, kMapThreads, sm_count, per_sm), kMapThreads, smem, st>>>(
-      d_uniq, d_ucount, d_table, d_sorted, max_colors, d_frame);
   DQ_CUDA_CHECK(cudaGetLastError());
 }
 

@@ -273,9 +273,9 @@ void dq_rows_quant_recurse(dq_rows *rows, const uint32_t *d_shard, uint32_t n_sh
  * 2b. Frame pipeline: quant_recurse over a stream of frames (BASELINE.json config 4, "batch of frames", and both
  *     legs of bench.py).  Frames are independent units and one frame's critical path (the chain of dependent
  *     passes of the split) leaves most of the GPU idle, so the pipeline runs `lanes` frames side by side: every
- *     lane owns a context, a pair of frame buffers and a host thread that walks one frame at a time through
- *     H2D -> kernels -> D2H.  The split kernels of different lanes occupy disjoint groups of SMs, histogram / remap
- *     kernels and both copy engines fill in around them.  Results are exactly those of dq_quant_recurse frame by
+ *     lane owns a context and a pair of frame buffers, and one host thread walks each lane's frames, one at a time,
+ *     through H2D -> kernels -> D2H.  The split kernels of different lanes occupy disjoint groups of SMs,
+ *     histogram / remap kernels and both copy engines fill in around them.  Results are exactly those of dq_quant_recurse frame by
  *     frame (they do not depend on the lane or on split_ctas).
  *     Host buffers should be pinned (cudaHostAlloc / torch pin_memory) for the copies to be asynchronous;
  *     pageable buffers work but serialise.  All pointers of a frame (pixels, numClustersPtr, colortable) must stay
@@ -308,15 +308,15 @@ float dq_pipeline_last_elapsed_ms(const dq_pipeline *pipe);
 dq_context *dq_pipeline_context(dq_pipeline *pipe);
 /* Kernels launched since creation (sum over frames and lanes). */
 uint64_t dq_pipeline_kernel_launches(const dq_pipeline *pipe);
-/* Frames whose tie audit raised a flag and that therefore went through the synchronous path a second time. */
+/* Frames (since creation) whose tie audit raised a flag (dq_call_stats::tie_flags != 0). */
 uint64_t dq_pipeline_flagged_frames(const dq_pipeline *pipe);
 /* Frames (since creation) that the resolver settled (dq_call_stats::tie_resolved or cut_overrides > 0), and frames that were
  * computed again on the ordered path (dq_call_stats::ordered_rerun = 1). */
 uint64_t dq_pipeline_resolved_frames(const dq_pipeline *pipe);
 uint64_t dq_pipeline_rerun_frames(const dq_pipeline *pipe);
 int dq_pipeline_lanes(const dq_pipeline *pipe);
-/* Lane threads spin while they wait for the GPU (lowest latency; default) or, with enabled = 1, sleep on an event:
- * use it when the pipeline has more lanes than the process has free host cores (several ranks on one host). */
+/* The pipeline's one host thread polls its lanes while they wait for the GPU.  It spins (lowest latency; default) or,
+ * with enabled = 1, sleeps 20 us between polling rounds: use it when host cores are scarce (several ranks on one host). */
 void dq_pipeline_set_blocking_wait(dq_pipeline *pipe, int enabled);
 
 /* ------------------------------------------------------------------------------------------------
@@ -357,11 +357,6 @@ uint32_t dq_debug_split_timeline(dq_context *ctx, int enable, uint64_t *pairs_ou
  *   dq_host_build_search_tables sorted palette (the reference's std::sort by r+g+b) and lut_init[766]
  *                               (DivQuantMapColors.cpp:267-383). */
 uint32_t dq_host_dedup_palette(uint32_t *colortable, uint32_t num_colors);
-/* Permutation that sorting n <= 65536 entries by keys[i] (< 65536) produces: perm_out[j] = original index of the entry
- * that ends at position j.  use_replay = 0: std::sort on the reference's Pixel_Int / comparator (what the host shim
- * calls); 1: the step-for-step replay of libstdc++'s introsort that the device runs (csrc/dq_stdsort.cuh).  The two
- * must agree for every input, equal keys included -- tests/test_stdsort.py. */
-void dq_host_sort_permutation(const uint32_t *keys, int n, int use_replay, uint32_t *perm_out);
 void dq_host_build_search_tables(const uint32_t *colortable, int num_colors, uint32_t *sorted_out, int32_t *lut_init_out);
 /* Host logic of the re-split with forced cuts (dq_call_stats::cut_overrides): of n <= 16 flagged cut entries, each a range
  * [begin, begin + size) of point positions with the resolver's status (3 = the reference cuts this node elsewhere), which

@@ -586,14 +586,12 @@ def test_ordered_path_above_the_default_limit(dq, oracle, golden):
         dq.lib.dq_context_set_exact_max_points(ctx, EXACT_DEFAULT_LIMIT)
 
 
-def test_frame_pipeline_device_side_palette_chain(dq, pkg, oracle, monkeypatch):
-    """DIVQUANT_B200_ASYNC=1: the whole chain of a frame is queued without a host wait -- duplicates dropped, the palette
-    ordered by the step-for-step replay of libstdc++'s std::sort (csrc/dq_stdsort.cuh) and lut_init built on the device
-    (palette_post), remap through the unique-colour table.  Must equal the blocking call frame by frame, including
-    palettes with duplicate words and many equal r+g+b sums (greys)."""
+def test_frame_pipeline_duplicate_and_equal_sum_palettes(dq, pkg, oracle):
+    """The frame pipeline's host palette handling (duplicates dropped, std::sort by r+g+b, lut_init) must equal the
+    blocking call frame by frame on the palettes no other pipeline test gives it: duplicate words, many equal r+g+b sums
+    (greys), K > U, and K = 300 / 512 (map_unique with uploaded tables)."""
     import ctypes as C
     import torch
-    monkeypatch.setenv("DIVQUANT_B200_ASYNC", "1")
     rng = np.random.default_rng(3)
     frames = [oracle.generate(1, 320, 200, 300 + i) for i in range(6)]
     frames.append((rng.integers(0, 256, 5000).astype(np.uint32) * 0x010101))          # greys: every sum distinct by 3

@@ -101,15 +101,14 @@ def _run_pipeline(dq, pkg, oracle, frames, images, seq, k, lanes, split_ctas, de
         pipe.close()
 
 
-ENV_MODES = {"default": {}, "async": {"DIVQUANT_B200_ASYNC": "1"}, "resolve_large": {"DIVQUANT_B200_RESOLVE": "2"}}
+ENV_MODES = {"default": {}, "resolve_large": {"DIVQUANT_B200_RESOLVE": "2"}}
 
 
 @pytest.mark.parametrize("mode", list(ENV_MODES))
 def test_pipeline_flagged_c4_frames(dq, pkg, oracle, frames, images, monkeypatch, mode):
     """Lanes poll quantize_step one phase at a time (resolver and re-split of one lane run while others start frames);
-    split kernels run on a share of the SMs.  ASYNC=1: a flagged frame is found after its whole chain ran and goes again
-    through the blocking path.  RESOLVE=2: every flagged rounding goes through the resolver's large form.  Environment
-    variables are read when the pipeline and its contexts are created."""
+    split kernels run on a share of the SMs.  RESOLVE=2: every flagged rounding goes through the resolver's large form.
+    Environment variables are read when the pipeline and its contexts are created."""
     for name, value in ENV_MODES[mode].items():
         monkeypatch.setenv(name, value)
     seq = _c4_sequence()

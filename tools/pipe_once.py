@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""A few frames through the frame pipeline (for ncu launch lists of the asynchronous chain).
+"""A few frames through the frame pipeline (for ncu launch lists of its kernels).
 usage: python tools/pipe_once.py [width height K frames lanes]"""
 import ctypes as C
 import importlib

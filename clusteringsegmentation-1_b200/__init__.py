@@ -49,6 +49,15 @@ class CallStats(C.Structure):
         return d
 
 
+class BatchStats(C.Structure):
+    """dq_batch_stats: which path the items of the last batch call took."""
+    _fields_ = [("items", C.c_uint32), ("batched_items", C.c_uint32), ("single_call_items", C.c_uint32),
+                ("empty_clusters", C.c_uint32), ("kernel_launches", C.c_uint32), ("host_palette_ms", C.c_float)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 def build(verbose=False):
     """Compile libdivquant_b200.so in-tree (nvcc, sm_100a only)."""
     subprocess.run(["make", "-C", _HERE, "-j4"], check=True, stdout=None if verbose else subprocess.DEVNULL)
@@ -85,6 +94,9 @@ def load_library(path=LIB_PATH):
         "dq_quant_varpart_device": (None, [vp, C.c_uint32, vp, C.c_uint32, C.c_uint32, _u32p, _u32p, C.c_int,
                                            C.c_int, C.c_int, C.c_int]),
         "dq_quant_recurse_ctx": (None, [vp, C.c_uint32, _u32p, _u32p, _u32p, _u32p, C.c_int]),
+        "dq_quant_recurse_batch_device": (None, [vp, C.c_uint32, _u32p, C.c_uint32, vp, vp, _u32p, _u32p, C.c_int]),
+        "dq_quant_recurse_batch_ctx": (None, [vp, C.c_uint32, _u32p, C.c_uint32, _u32p, _u32p, _u32p, _u32p, C.c_int]),
+        "dq_context_last_batch_stats": (None, [vp, C.POINTER(BatchStats)]),
         "dq_context_set_split_ctas": (None, [vp, C.c_int]),
         "dq_context_set_exact_small": (None, [vp, C.c_int]),
         "dq_context_set_exact_max_points": (None, [vp, C.c_uint32]),
@@ -142,6 +154,7 @@ EXPORTED_C_SYMBOLS = [
     "dq_srm_num_pairs", "dq_srm_sorted_edges", "dq_srm_sorted_edges_device", "dq_context_set_split_ctas", "dq_context_set_exact_small", "dq_context_set_exact_max_points", "dq_context_set_tie_policy", "dq_pixel_histogram", "dq_block_vote", "dq_block_vote_device", "dq_quant_blocks", "dq_colortable_indexes", "dq_colortable_indexes_device", "dq_shard_histogram", "dq_shard_quantize_map", "dq_rows_unique_id", "dq_rows_create", "dq_rows_destroy", "dq_rows_quant_recurse", "dq_pipeline_create", "dq_pipeline_create_lanes", "dq_pipeline_destroy", "dq_pipeline_submit", "dq_pipeline_submit_device", "dq_pipeline_wait", "dq_pipeline_lanes", "dq_pipeline_set_blocking_wait", "dq_pipeline_flush", "dq_pipeline_last_elapsed_ms",
     "dq_pipeline_context", "dq_pipeline_kernel_launches", "dq_pipeline_flagged_frames",
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
+    "dq_quant_recurse_batch_device", "dq_quant_recurse_batch_ctx", "dq_context_last_batch_stats",
     "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
 ]
 
@@ -186,6 +199,51 @@ class DivQuant:
         self.lib.dq_quant_varpart_fast(px.size, _p(px), _p(tmp), rows, cols, C.byref(nk), _p(ct), num_bits, dec_factor,
                                        max_iters, all_unique)
         return ct[:nk.value].copy(), int(k) - nk.value
+
+    def quant_recurse_batch(self, items, ks, all_unique=0, ctx=None):
+        """quant_recurse of every pixel set in `items` (uint32 arrays) with the K in `ks`, in one call
+        (dq_quant_recurse_batch_ctx).  Returns a list of (out, palette), one per item, each equal to
+        quant_recurse(items[i], ks[i], all_unique) on the same context."""
+        arrs = [_u32(a) for a in items]
+        ks = [int(k) for k in ks]
+        if len(arrs) != len(ks):
+            raise ValueError("one K per item")
+        if not arrs:
+            return []
+        offsets = np.zeros(len(arrs) + 1, np.uint32)
+        np.cumsum([a.size for a in arrs], out=offsets[1:])
+        flat = np.concatenate(arrs) if offsets[-1] else np.zeros(1, np.uint32)
+        out = np.zeros_like(flat)
+        nk = np.asarray(ks, np.uint32)
+        pal_off = np.concatenate([[0], np.cumsum(ks)]).astype(np.int64)
+        ct = np.zeros(max(int(pal_off[-1]), 1), np.uint32)
+        self.lib.dq_quant_recurse_batch_ctx(ctx or self.lib.dq_default_context(), len(arrs), _p(offsets), flat.size, _p(flat), _p(out),
+                                            _p(nk), _p(ct), all_unique)
+        return [(out[offsets[i]:offsets[i + 1]].copy(), ct[pal_off[i]:pal_off[i] + nk[i]].copy()) for i in range(len(arrs))]
+
+    def quant_recurse_batch_device(self, flat, offsets, ks, all_unique=0, ctx=None, out=None):
+        """Device form (dq_quant_recurse_batch_device): `flat` is a CUDA tensor of 32-bit pixels holding the items end to
+        end, item i = flat[offsets[i]:offsets[i+1]].  Returns (out tensor, palettes, actual K): palettes is the uint32
+        array of sum(ks) words in which item i's palette starts at sum(ks[:i]) and holds actual_k[i] entries."""
+        import torch
+        offs = _u32(offsets)
+        nk = _u32(ks).copy()
+        if offs.size != nk.size + 1:
+            raise ValueError("offsets need one entry more than ks")
+        if flat.dtype not in (torch.int32, torch.uint32) or not flat.is_cuda or not flat.is_contiguous():
+            raise ValueError("flat must be a contiguous CUDA tensor of 32-bit pixels")
+        out = torch.empty_like(flat) if out is None else out
+        ct = np.zeros(max(int(nk.astype(np.int64).sum()), 1), np.uint32)
+        if nk.size:
+            torch.cuda.current_stream(flat.device).synchronize()  # the library works on its context's stream
+            self.lib.dq_quant_recurse_batch_device(ctx or self.lib.dq_default_context(), nk.size, _p(offs), flat.numel(),
+                                                   flat.data_ptr(), out.data_ptr(), _p(nk), _p(ct), all_unique)
+        return out, ct, nk
+
+    def last_batch_stats(self, ctx=None):
+        st = BatchStats()
+        self.lib.dq_context_last_batch_stats(ctx or self.lib.dq_default_context(), C.byref(st))
+        return st.as_dict()
 
     def map_colors_mps(self, pixels, colortable):
         px = _u32(pixels)

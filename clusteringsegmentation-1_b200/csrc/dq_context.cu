@@ -70,6 +70,25 @@ struct PaletteEntry {
 inline bool palette_less(const PaletteEntry &a, const PaletteEntry &b) { return a.weight < b.weight; }
 
 constexpr int kLutEntries = 3 * 255 + 1;
+static_assert(kLutEntries == kBatchLutEntries, "lut_init of the batch remap");
+
+// Pinned host staging that grows like DevBuf.
+struct PinnedBuf {
+  uint32_t *ptr = nullptr;
+  size_t cap = 0;
+  void ensure(size_t n) {
+    if (n <= cap) return;
+    if (ptr) DQ_CUDA_CHECK(cudaFreeHost(ptr));
+    const size_t want = n + n / 8 + 64;
+    DQ_CUDA_CHECK(cudaMallocHost(&ptr, want * sizeof(uint32_t)));
+    cap = want;
+  }
+  void release() {
+    if (ptr) cudaFreeHost(ptr);
+    ptr = nullptr;
+    cap = 0;
+  }
+};
 
 }  // namespace
 
@@ -161,6 +180,13 @@ struct dq_context {
   // host mailbox of the split kernel (mapped pinned memory, SplitArgs::mailbox)
   volatile uint32_t *mailbox = nullptr;
   uint32_t mailbox_seq = 0;
+  // quant_recurse over a batch of items (dq_batch.cu; quant_recurse_batch below)
+  DevBuf<uint32_t> b_work;    // [items | per-item results | palettes | histogram slices: colours, counts, first seen]
+  DevBuf<uint32_t> b_tables;  // [remap tiles | per-item (offset, size) | sorted palettes | lut_init as uint16]
+  DevBuf<uint32_t> b_cluster_size;
+  DevBuf<double> b_cluster_mean;
+  PinnedBuf b_up, b_down, b_tab;
+  dq_batch_stats batch_stats = {};
   int use_mailbox = 1;  // DIVQUANT_B200_MAILBOX=0: always wait for the stream and copy
   void wait() {
     if (!blocking_wait) {
@@ -897,6 +923,142 @@ void quant_recurse_device_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in
   if (ms_map) *ms_map = std::chrono::duration<double, std::milli>(t2 - t1).count();
 }
 
+// ---- quant_recurse over a batch of items (kernels: dq_batch.cu) -------------------------------------------------------
+// Fatal like every other bad argument: offsets that decrease or end beyond the input, an item with no pixels or K = 0.
+void check_batch_args(uint32_t num_items, const uint32_t *offsets, uint32_t num_pixels, const uint32_t *ks) {
+  for (uint32_t i = 0; i < num_items; ++i) {
+    if (offsets[i + 1] < offsets[i]) {
+      fprintf(stderr, "divquant_b200: batch offsets decrease at item %u (%u -> %u)\n", i, offsets[i], offsets[i + 1]);
+      abort();
+    }
+  }
+  if (offsets[num_items] > num_pixels) {
+    fprintf(stderr, "divquant_b200: batch offsets end at %u, beyond the %u input pixels\n", offsets[num_items], num_pixels);
+    abort();
+  }
+  for (uint32_t i = 0; i < num_items; ++i) check_quant_args(offsets[i + 1] - offsets[i], ks[i], 8);
+}
+
+// Every item gets what quant_recurse_device_impl gives it alone on this context.  An item is batched when the single call
+// would split it on the ordered path in shared memory: weighted (all_unique = 0), K <= kSplit2MaxColors and at most
+// min(exact_max_points, kBatchMaxPoints) distinct colours with the ordered path on.  The histogram kernel finds U; any
+// other item goes through quant_recurse_device_impl, in item order between the batched items' palette handling, so that
+// the "# empty clusters" lines come out as a loop of single calls prints them.
+void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, const uint32_t *d_in, uint32_t *d_out,
+                              uint32_t *ks, uint32_t *colortables, int all_unique) {
+  dq_batch_stats &bs = ctx->batch_stats;
+  bs = dq_batch_stats();
+  bs.items = num_items;
+  uint32_t launches = 0;
+  const uint32_t base = offsets[0], total = offsets[num_items] - base;
+  const uint32_t limit = ctx->exact_small ? std::min<uint32_t>(ctx->exact_max_points, kBatchMaxPoints) : 0u;
+  std::vector<uint32_t> cand_of(num_items, UINT32_MAX), cand_pal;
+  size_t sum_k = 0;
+  for (uint32_t i = 0; i < num_items; ++i) {
+    if (all_unique || limit == 0u || ks[i] > kSplit2MaxColors) continue;
+    cand_of[i] = (uint32_t)cand_pal.size();
+    cand_pal.push_back((uint32_t)sum_k);
+    sum_k += ks[i];
+  }
+  const uint32_t nc = (uint32_t)cand_pal.size();
+  const size_t w_items = (size_t)4 * nc, w_res = (size_t)kBatchResultWords * nc;
+  if (nc > 0) {
+    static_assert(sizeof(BatchItem) == 4 * sizeof(uint32_t), "four words per item");
+    ctx->b_work.ensure(w_items + w_res + sum_k + (size_t)3 * total);
+    ctx->b_cluster_size.ensure(sum_k);
+    ctx->b_cluster_mean.ensure(3 * sum_k);
+    ctx->b_up.ensure(w_items);
+    BatchItem *h_items = reinterpret_cast<BatchItem *>(ctx->b_up.ptr);
+    for (uint32_t i = 0; i < num_items; ++i) {
+      const uint32_t j = cand_of[i];
+      if (j != UINT32_MAX) h_items[j] = {offsets[i] - base, offsets[i + 1] - offsets[i], ks[i], cand_pal[j]};
+    }
+    uint32_t *const d_items = ctx->b_work.ptr, *const d_res = d_items + w_items, *const d_pal = d_res + w_res;
+    uint32_t *const d_colours = d_pal + sum_k, *const d_counts = d_colours + total, *const d_first = d_counts + total;
+    const BatchItem *d_items_b = reinterpret_cast<const BatchItem *>(d_items);
+    DQ_CUDA_CHECK(cudaMemcpyAsync(d_items, h_items, w_items * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    batch_hist_launch(d_in + base, d_items_b, nc, d_colours, d_counts, d_first, d_res, ctx->stream);
+    batch_split_launch(d_items_b, nc, limit, d_colours, d_counts, d_first, d_res, d_pal, ctx->b_cluster_size.ptr, ctx->b_cluster_mean.ptr,
+                       ctx->stream);
+    launches += 2;
+    // results and palettes of all items come back in one copy
+    ctx->b_down.ensure(w_res + sum_k);
+    DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->b_down.ptr, d_res, (w_res + sum_k) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    ctx->wait();
+  }
+  std::vector<BatchTile> tiles;
+  std::vector<uint2> tabs;
+  std::vector<uint32_t> sorted;
+  std::vector<uint16_t> luts;
+  tabs.reserve(nc);
+  luts.reserve((size_t)nc * kLutEntries);
+  double host_ms = 0.0;
+  size_t pal_off = 0;
+  for (uint32_t i = 0; i < num_items; ++i) {
+    const uint32_t n = offsets[i + 1] - offsets[i];
+    uint32_t *const ct = colortables + pal_off;
+    pal_off += ks[i];
+    const uint32_t j = cand_of[i];
+    const uint32_t *r = (j != UINT32_MAX) ? ctx->b_down.ptr + (size_t)kBatchResultWords * j : nullptr;
+    if (r != nullptr && r[0] <= limit) {
+      const auto t0 = std::chrono::steady_clock::now();
+      const uint32_t *ctl = r + 4;
+      if (ctl[kCtlError] != 0) {
+        fprintf(stderr, "divquant_b200: split of batch item %u failed (code %u; internal error)\n", i, ctl[kCtlError]);
+        abort();
+      }
+      const uint32_t actual = r[1], empty = r[2];
+      memcpy(ct, ctx->b_down.ptr + w_res + cand_pal[j], actual * sizeof(uint32_t));
+      if (empty) fprintf(stderr, "# empty clusters: %d\n", (int)empty);  // (:1067-1070)
+      const uint32_t k = dedup_palette(ct, actual);
+      ks[i] = k;
+      const uint32_t t = (uint32_t)tabs.size();
+      tabs.push_back(make_uint2((uint32_t)sorted.size(), k));
+      sorted.resize(sorted.size() + k);
+      int lut[kLutEntries];
+      build_search_tables(ct, (int)k, sorted.data() + tabs.back().x, lut);
+      for (int e = 0; e < kLutEntries; ++e) luts.push_back((uint16_t)lut[e]);
+      const uint32_t b0 = offsets[i] - base;
+      for (uint32_t b = 0; b < n; b += (uint32_t)kBatchTilePixels)
+        tiles.push_back({b0 + b, b0 + std::min<uint32_t>(n, b + (uint32_t)kBatchTilePixels), t, 0u});
+      bs.batched_items++;
+      bs.empty_clusters += empty;
+      host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    } else {
+      memset(&ctx->stats, 0, sizeof(ctx->stats));
+      ctx->stats.num_pixels = n;
+      quant_recurse_device_impl(ctx, n, d_in + offsets[i], d_out + offsets[i], &ks[i], ct, all_unique, nullptr, nullptr);
+      launches += ctx->stats.kernel_launches;
+      bs.empty_clusters += ctx->stats.empty_clusters;
+      bs.single_call_items++;
+    }
+  }
+  if (!tiles.empty()) {
+    // tiles, (offset, size) per item, sorted palettes and lut_init go up in one copy
+    static_assert(sizeof(BatchTile) == 4 * sizeof(uint32_t), "four words per tile");
+    const size_t w_tiles = 4 * tiles.size(), w_tabs = 2 * tabs.size(), w_luts = (luts.size() + 1) / 2;
+    const size_t words = w_tiles + w_tabs + sorted.size() + w_luts;
+    ctx->b_tab.ensure(words);
+    uint32_t *h = ctx->b_tab.ptr;
+    memcpy(h, tiles.data(), w_tiles * sizeof(uint32_t));
+    memcpy(h + w_tiles, tabs.data(), w_tabs * sizeof(uint32_t));
+    memcpy(h + w_tiles + w_tabs, sorted.data(), sorted.size() * sizeof(uint32_t));
+    memcpy(h + w_tiles + w_tabs + sorted.size(), luts.data(), luts.size() * sizeof(uint16_t));
+    ctx->b_tables.ensure(words);
+    uint32_t *d = ctx->b_tables.ptr;
+    DQ_CUDA_CHECK(cudaMemcpyAsync(d, h, words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    batch_remap_launch(d_in + base, d_out + base, reinterpret_cast<const BatchTile *>(d), (uint32_t)tiles.size(), d + w_tiles + w_tabs,
+                       reinterpret_cast<const uint2 *>(d + w_tiles), reinterpret_cast<const uint16_t *>(d + w_tiles + w_tabs + sorted.size()),
+                       ctx->stream);
+    launches++;
+    ctx->wait();
+  }
+  memset(&ctx->stats, 0, sizeof(ctx->stats));  // (dq_call_stats describes one frame: only the launches are kept)
+  ctx->stats.kernel_launches = launches;
+  bs.kernel_launches = launches;
+  bs.host_palette_ms = (float)host_ms;
+}
+
 std::mutex g_default_mutex;
 dq_context *g_default = nullptr;
 // The reference's functions are re-entrant; the entry points that run on the one lazily created default context are
@@ -1033,6 +1195,13 @@ void dq_context_destroy(dq_context *ctx) {
   ctx->d_ovr.release();
   ctx->d_flat.release();
   ctx->d_sortvals.release();
+  ctx->b_work.release();
+  ctx->b_tables.release();
+  ctx->b_cluster_size.release();
+  ctx->b_cluster_mean.release();
+  ctx->b_up.release();
+  ctx->b_down.release();
+  ctx->b_tab.release();
   cudaFree(ctx->d_table);
   cudaFree(ctx->d_map);
   cudaFree(ctx->d_cb);
@@ -1132,7 +1301,35 @@ void dq_map_colors_device(dq_context *ctx, const uint32_t *d_in, uint32_t numPix
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
 }
 
+void dq_quant_recurse_batch_device(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *d_in,
+                                   uint32_t *d_out, uint32_t *numClusters, uint32_t *colortables, int allPixelsUnique) {
+  if (num_items == 0) return;
+  require_device(ctx);
+  check_batch_args(num_items, offsets, numPixels, numClusters);
+  quant_recurse_batch_impl(ctx, num_items, offsets, d_in, d_out, numClusters, colortables, allPixelsUnique);
+}
+
+void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out) { *out = ctx->batch_stats; }
+
 // ---- host-pointer entry points ----
+
+void dq_quant_recurse_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *inPixels,
+                                uint32_t *outPixels, uint32_t *numClusters, uint32_t *colortables, int allPixelsUnique) {
+  if (num_items == 0) return;
+  require_device(ctx);
+  check_batch_args(num_items, offsets, numPixels, numClusters);
+  // only the pixels the items cover travel, from offsets[0] on
+  const uint32_t base = offsets[0], total = offsets[num_items] - base;
+  std::vector<uint32_t> local(offsets, offsets + num_items + 1);
+  for (uint32_t &o : local) o -= base;
+  ctx->d_in.ensure(total);
+  ctx->d_out.ensure(total);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels + base, (size_t)total * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  quant_recurse_batch_impl(ctx, num_items, local.data(), ctx->d_in.ptr, ctx->d_out.ptr, numClusters, colortables, allPixelsUnique);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels + base, ctx->d_out.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+}
+
 
 void dq_quant_recurse_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixelsPtr, uint32_t *outPixelsPtr,
                           uint32_t *numClustersPtr, uint32_t *outColortablePtr, int allPixelsUnique) {

@@ -58,6 +58,33 @@ void map_labels(const uint32_t *d_in, uint32_t n, uint32_t *d_out, const uint2 *
                 uint32_t *d_error, int sm_count, cudaStream_t st);
 void map_gather(const uint32_t *d_in, uint32_t n, uint32_t *d_out, const uint32_t *d_table, int sm_count, cudaStream_t st);
 
+// ---- dq_batch.cu: quant_recurse over many small items (one CTA per item) ----
+constexpr uint32_t kBatchMaxPoints = 4096;       // distinct colours a batched item may have (its points stay in shared memory)
+constexpr uint32_t kBatchOverflow = 0xFFFFFFFFu;  // result word 0 of an item with more colours than that
+constexpr uint32_t kBatchResultWords = 16;        // per item: [0] U | [1] palette entries [2] empty clusters | [4, 16) ctl words
+constexpr int kBatchTilePixels = 1024;            // pixels per CTA of the remap
+constexpr int kBatchLutEntries = 3 * 255 + 1;
+struct BatchItem {
+  uint32_t begin, n;  // pixels [begin, begin + n) of the flat input; the item's histogram slices start at begin as well
+  uint32_t k, pal;    // requested K; offset of its palette in the palette buffer
+};
+struct BatchTile {
+  uint32_t begin, end;  // pixels of the flat input
+  uint32_t table;       // batched item whose tables map them
+  uint32_t pad;
+};
+// One launch each, one CTA per item.  d_colours / d_counts / d_first: as many words as the flat input.
+void batch_hist_launch(const uint32_t *d_in, const BatchItem *d_items, uint32_t num_items, uint32_t *d_colours, uint32_t *d_counts,
+                       uint32_t *d_first, uint32_t *d_res, cudaStream_t st);
+// Items whose U (result word 0) exceeds max_points (at most kBatchMaxPoints) are left alone.  d_cluster_size / d_cluster_mean:
+// 1 / 3 entries per palette word.
+void batch_split_launch(const BatchItem *d_items, uint32_t num_items, uint32_t max_points, const uint32_t *d_colours, uint32_t *d_counts,
+                        const uint32_t *d_first, uint32_t *d_res, uint32_t *d_palette, uint32_t *d_cluster_size, double *d_cluster_mean,
+                        cudaStream_t st);
+// d_tables[i] = (offset in d_sorted, palette size) of batched item i, d_luts[i * kBatchLutEntries ...] its lut_init.
+void batch_remap_launch(const uint32_t *d_in, uint32_t *d_out, const BatchTile *d_tiles, uint32_t num_tiles, const uint32_t *d_sorted,
+                        const uint2 *d_tables, const uint16_t *d_luts, cudaStream_t st);
+
 // ---- dq_srm.cu ----
 uint32_t srm_num_pairs(uint32_t width, uint32_t height);
 size_t srm_scratch_words(uint32_t width, uint32_t height);

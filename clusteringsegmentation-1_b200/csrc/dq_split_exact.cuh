@@ -521,13 +521,34 @@ __device__ __forceinline__ void split_passes(Shared &S, const Points &P, int cur
   }
 }
 
+// Where the prologue finds the U points, through three arrays (colours, counts, first) whose meaning the source gives.
+// FromTable: the histogram of a call -- colours = the unique colours in arrival order, counts = the direct count table
+// (zeroed on the way), first = the first-seen table indexed by colour; the points are also left in A.pts[0].
+struct FromTable {
+  static __device__ __forceinline__ uint32_t colour(const uint32_t *uniq, int i) { return uniq[i]; }
+  static __device__ __forceinline__ uint32_t first(const uint32_t *first_seen, int, uint32_t c) { return ld_cg_u32(first_seen + c); }
+  static __device__ __forceinline__ uint32_t take_count(uint32_t *table, int, uint32_t c) {
+    const uint32_t count = table[c];
+    table[c] = 0u;  // the count table is all-zero again when the call ends
+    return count;
+  }
+  static __device__ __forceinline__ void keep(const SplitArgs &A, int i, uint32_t c, uint32_t count) { A.pts[0][i] = make_uint2(c, count); }
+};
+// FromSlices: one item of a batch (dq_batch.cu) -- point i is (colours[i], counts[i]), first seen at pixel first[i].
+struct FromSlices {
+  static __device__ __forceinline__ uint32_t colour(const uint32_t *colours, int i) { return colours[i]; }
+  static __device__ __forceinline__ uint32_t first(const uint32_t *first, int i, uint32_t) { return first[i]; }
+  static __device__ __forceinline__ uint32_t take_count(uint32_t *counts, int i, uint32_t) { return counts[i]; }
+  static __device__ __forceinline__ void keep(const SplitArgs &, int, uint32_t, uint32_t) {}
+};
+
 // The whole divisive phase of one input by one CTA of THREADS threads.  smem: sizeof(Shared) bytes; scratch:
 // kScratchBytes of global memory (used when U > kSmemPoints).
-// uniq / table: the histogram (unique colours in arrival order, counts; the counts are zeroed on the way);
-// first_seen[c]: smallest sample index of colour c; g_*: per-cluster scratch in global memory, used when K > 1024.
-template <int THREADS>
-__device__ __noinline__ void split_exact_body(const SplitArgs &A, int U, unsigned char *smem, unsigned char *scratch, const uint32_t *uniq,
-                                 uint32_t *table, const uint32_t *first_seen, double *g_weight, double *g_tse, double *g_mean,
+// colours / counts / first: the points, read through Src (FromTable: the histogram and the first-seen table of the call);
+// g_*: per-cluster scratch in global memory, used when K > kSmemColors.
+template <int THREADS, typename Src = FromTable>
+__device__ __noinline__ void split_exact_body(const SplitArgs &A, int U, unsigned char *smem, unsigned char *scratch, const uint32_t *colours,
+                                 uint32_t *counts, const uint32_t *first, double *g_weight, double *g_tse, double *g_mean,
                                  double *g_var, int32_t *g_size) {
   Shared &S = *reinterpret_cast<Shared *>(smem);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -559,10 +580,10 @@ __device__ __noinline__ void split_exact_body(const SplitArgs &A, int U, unsigne
   for (int i = tid; i < sort_n; i += THREADS) {
     unsigned long long key = ~0ull;
     if (i < U) {
-      const uint32_t c = uniq[i];
+      const uint32_t c = Src::colour(colours, i);
       const long R = (c >> 16) & 0xFF, G = (c >> 8) & 0xFF, B = c & 0xFF;
       const unsigned long long bucket = (unsigned long long)(((R * 33023 + G * 30013 + B * 27011) & 0x7fffffff) % 20023);
-      key = (bucket << (31 + kIndexBits)) | ((unsigned long long)(0x7FFFFFFFu - ld_cg_u32(first_seen + c)) << kIndexBits) |
+      key = (bucket << (31 + kIndexBits)) | ((unsigned long long)(0x7FFFFFFFu - Src::first(first, i, c)) << kIndexBits) |
             (unsigned long long)i;
     }
     P.keys[i] = key;
@@ -585,14 +606,14 @@ __device__ __noinline__ void split_exact_body(const SplitArgs &A, int U, unsigne
     }
   }
   for (int i = tid; i < U; i += THREADS) {
-    const uint32_t c = uniq[(int)(P.keys[i] & ((1ull << kIndexBits) - 1ull))];
-    const uint32_t count = table[c];
-    table[c] = 0u;  // the count table is all-zero again when the call ends
+    const int idx = (int)(P.keys[i] & ((1ull << kIndexBits) - 1ull));
+    const uint32_t c = Src::colour(colours, idx);
+    const uint32_t count = Src::take_count(counts, idx, c);
     P.colour[i] = c;
     P.w[i] = fmul(A.norm, (double)(int)count);  // weights[i] = weight * count (:185)
     P.member[i] = 0;
     P.cur[i] = (uint32_t)i;
-    A.pts[0][i] = make_uint2(c, count);
+    Src::keep(A, i, c, count);
   }
   for (int i = tid; i < K; i += THREADS) {  // `new T[n]()` of the reference (:296-324)
     weight[i] = 0.0;

@@ -320,6 +320,36 @@ int dq_pipeline_lanes(const dq_pipeline *pipe);
 void dq_pipeline_set_blocking_wait(dq_pipeline *pipe, int enabled);
 
 /* ------------------------------------------------------------------------------------------------
+ * 2c. Many small inputs in one call: quant_recurse over num_items independent pixel sets (regions of a segmentation,
+ *     tiles of an image, thumbnails) packed end to end.  Item i is pixels [offsets[i], offsets[i+1]) of the input.
+ *     Each item's result equals dq_quant_recurse_device on this context for that item alone, bit for bit: its palette
+ *     (colortables), its actual K (numClusters) and its remapped pixels, and the same "# empty clusters: n" line on stderr.
+ *     An item that the single call would split on the ordered path in shared memory (allPixelsUnique = 0, K <= 512 and at
+ *     most min(dq_context_set_exact_max_points, 4096) distinct colours with the ordered path on) is computed by batch
+ *     kernels, one CTA per item, in launches whose number does not depend on the number of items; every other item goes
+ *     through the single call inside the same call, in item order.
+ *   offsets:     HOST array of num_items + 1 non-decreasing words, offsets[num_items] <= numPixels.
+ *   numClusters: HOST, num_items words: in = requested K of item i, out = actual.
+ *   colortables: HOST, sum of the requested K words; item i's palette starts at the sum of the requested K of items < i.
+ * Decreasing offsets, offsets beyond numPixels, an item with no pixels or K = 0 are fatal (message + abort).
+ * num_items = 0 does nothing.  Neither form prints timing lines.  Synchronous on return.  Afterwards dq_call_stats is
+ * zeroed apart from kernel_launches (all the call launched); dq_context_last_batch_stats tells which path the items took.
+ * ---------------------------------------------------------------------------------------------- */
+void dq_quant_recurse_batch_device(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *d_in,
+                                   uint32_t *d_out, uint32_t *numClusters, uint32_t *colortables, int allPixelsUnique);
+void dq_quant_recurse_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *inPixels,
+                                uint32_t *outPixels, uint32_t *numClusters, uint32_t *colortables, int allPixelsUnique);
+typedef struct {
+  uint32_t items;              /* num_items of the last batch call                                    */
+  uint32_t batched_items;      /* items computed by the batch kernels                                  */
+  uint32_t single_call_items;  /* items that went through the single call                              */
+  uint32_t empty_clusters;     /* sum over all items                                                   */
+  uint32_t kernel_launches;    /* kernels launched by the whole call, single calls included            */
+  float host_palette_ms;       /* wall clock of the host's palette handling of the batched items      */
+} dq_batch_stats;
+void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out);
+
+/* ------------------------------------------------------------------------------------------------
  * 3. Test hooks (used by tests/ to compare intermediate results with the oracle).
  * ---------------------------------------------------------------------------------------------- */
 

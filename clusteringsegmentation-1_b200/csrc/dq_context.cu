@@ -1815,10 +1815,12 @@ dq_pipeline *dq_pipeline_create_lanes(int device, uint32_t max_pixels, int lanes
   for (auto &lane : p->lanes) {
     lane.ctx = dq_context_create(device);
     p->device = lane.ctx->device;
-    // Default SM partition: the split kernels of all lanes together hold 11/16 of the SMs; the rest stays free for the
+    // Default SM partition: the split kernels of all lanes together hold 3/4 of the SMs; the rest stays free for the
     // histogram / remap kernels, which cannot share an SM with a split CTA (it owns the register file).  Measured at
-    // 4K, 12 lanes: 6 CTAs each 0.182 ms/frame, 7: 0.169, 8: 0.160, 9: 0.170, 10: 0.186 (tools/lanes_check.py).
-    if (split_ctas <= 0) split_ctas = std::max(split2_max_ctas(lane.ctx->sm_count, 256) * 11 / 16 / lanes, lanes > 1 ? 4 : 1);
+    // 4K, 12 lanes, with the chunked histogram (tools/lanes_check.py, B200): 8 CTAs each 0.158 ms/frame, 9: 0.153,
+    // 10: 0.154, 11: 0.156; 1080p K = 64: 8: 0.100, 9: 0.095, 10: 0.094, 11: 0.093.  Before the chunked histogram the
+    // best was 8 CTAs (11/16): more split SMs left it too few free SMs to keep enough L2 atomics in flight.
+    if (split_ctas <= 0) split_ctas = std::max(split2_max_ctas(lane.ctx->sm_count, 256) * 3 / 4 / lanes, lanes > 1 ? 4 : 1);
     if (lanes == 1) split_ctas = 0;  // a single lane is a single call: all SMs
     dq_context_set_split_ctas(lane.ctx, split_ctas);
     if (max_pixels) {

@@ -8,37 +8,18 @@
 // that occur are ever touched, so for natural images the working set lives in L2).  The table is
 // all-zero between calls: whoever dirties it clears exactly the entries it touched.
 //   hist_insert   : count += 1 per sampled pixel; the thread that sees 0 appends the colour to the
-//                   unique list (one warp-aggregated cursor bump per warp).
+//                   unique list (one warp-aggregated cursor bump per warp).  Contiguous inputs of a 32 768-pixel
+//                   chunk per SM or more are counted per chunk in shared memory first (dq_hist_chunk.cuh).
 //   hist_collect  : (colour, count) points for the divisive phase.
 //   table_clear   : zero the touched entries.
+#include <mutex>
+#include <set>
+
+#include "dq_hist_chunk.cuh"
 #include "dq_kernels.cuh"
 
 namespace dq {
 namespace {
-
-__device__ __forceinline__ uint32_t cut_colour(uint32_t pixel, uint32_t word_mask, uint32_t shift) {
-  // whole-word variant of cut_bits (DivQuantUni.cpp:60-74); mask also drops the alpha byte
-  return (pixel & word_mask) >> shift;
-}
-
-// seen_init (may be null): second direct table; a colour's entry is set to 0xFFFFFFFF by its first toucher, which is
-// what the first-seen pass of the small-input path starts from (dq_split_exact.cu).
-__device__ __forceinline__ void insert_colour(uint32_t c, bool active, uint32_t *table, uint32_t *uniq,
-                                              uint32_t *ucount, uint32_t *seen_init) {
-  bool fresh = false;
-  if (active) fresh = (atomicAdd(table + c, 1u) == 0u);
-  const unsigned m = __ballot_sync(0xffffffffu, fresh);
-  if (m) {
-    const int lane = threadIdx.x & 31;
-    uint32_t base = 0;
-    if (lane == __ffs(m) - 1) base = atomicAdd(ucount, (uint32_t)__popc(m));
-    base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-    if (fresh) {
-      uniq[base + __popc(m & ((1u << lane) - 1u))] = c;
-      if (seen_init) seen_init[c] = 0xFFFFFFFFu;
-    }
-  }
-}
 
 // Contiguous sampling (dec_factor == 1, numRows == 1: every live caller, quant_util.cpp:60).
 __global__ void __launch_bounds__(256) hist_insert_kernel(const uint32_t *__restrict__ in, uint32_t n,
@@ -284,6 +265,17 @@ __global__ void __launch_bounds__(256) hist_merge_first_kernel(const uint32_t *_
   }
 }
 
+// hist_insert_chunked_kernel's table is above the default 48 KB of dynamic shared memory: the limit is raised once per device.
+void hist_chunk_allow_smem() {
+  static std::mutex mu;
+  static std::set<int> raised;
+  int dev = 0;
+  DQ_CUDA_CHECK(cudaGetDevice(&dev));
+  std::lock_guard<std::mutex> lock(mu);
+  if (raised.insert(dev).second)
+    DQ_CUDA_CHECK(cudaFuncSetAttribute(hist_insert_chunked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_chunk::kSmemBytes));
+}
+
 inline int blocks_for(uint64_t items, int threads, int sm_count, int per_sm) {
   uint64_t want = (items + threads - 1) / threads;
   uint64_t cap = (uint64_t)sm_count * per_sm;
@@ -301,8 +293,16 @@ void hist_insert(const uint32_t *d_in, uint32_t n, uint32_t num_rows, uint32_t n
   const bool aligned = (reinterpret_cast<uintptr_t>(d_in) & 15u) == 0;  // uint4 loads
   if (dec == 1 && num_rows == 1 && aligned) {
     const uint32_t count = num_cols < n ? num_cols : n;
-    hist_insert_kernel<<<blocks_for((count >> 2) + 32, 256, sm_count, 8), 256, 0, st>>>(d_in, count, word_mask, shift,
-                                                                                        d_table, d_uniq, d_ucount, d_seen_init);
+    if (count / hist_chunk::kChunk >= (uint32_t)sm_count) {
+      // a chunk per SM or more (4K frames): one L2 atomic per distinct colour of a chunk instead of one per pixel
+      hist_chunk_allow_smem();
+      hist_insert_chunked_kernel<<<blocks_for(count, (int)hist_chunk::kChunk, sm_count, 8), hist_chunk::kThreads,
+                                   hist_chunk::kSmemBytes, st>>>(d_in, count, hist_chunk::kChunk >> 2, word_mask, shift,
+                                                                 d_table, d_uniq, d_ucount, d_seen_init);
+    } else {
+      hist_insert_kernel<<<blocks_for((count >> 2) + 32, 256, sm_count, 8), 256, 0, st>>>(d_in, count, word_mask, shift,
+                                                                                          d_table, d_uniq, d_ucount, d_seen_init);
+    }
   } else {
     const uint32_t nr = (num_rows + dec - 1) / dec, nc = (num_cols + dec - 1) / dec;
     const uint32_t samples = nr * nc;

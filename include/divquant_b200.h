@@ -284,7 +284,7 @@ void dq_rows_quant_recurse(dq_rows *rows, const uint32_t *d_shard, uint32_t n_sh
  * ---------------------------------------------------------------------------------------------- */
 typedef struct dq_pipeline dq_pipeline;
 /* lanes = frames in flight (1..16); max_pixels = largest HOST frame that will be submitted (0 if only device frames
- * are used); split_ctas = CTAs of each lane's split kernel, 0 = (11/16 of the SMs) / lanes, which leaves the histogram /
+ * are used); split_ctas = CTAs of each lane's split kernel, 0 = (3/4 of the SMs) / lanes, which leaves the histogram /
  * remap kernels of the other lanes SMs of their own. */
 dq_pipeline *dq_pipeline_create_lanes(int device, uint32_t max_pixels, int lanes, int split_ctas);
 /* Same with lanes = depth (2..8) and the default SM partition. */

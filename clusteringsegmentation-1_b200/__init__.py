@@ -97,6 +97,8 @@ def load_library(path=LIB_PATH):
         "dq_quant_recurse_batch_device": (None, [vp, C.c_uint32, _u32p, C.c_uint32, vp, vp, _u32p, _u32p, C.c_int]),
         "dq_quant_recurse_batch_ctx": (None, [vp, C.c_uint32, _u32p, C.c_uint32, _u32p, _u32p, _u32p, _u32p, C.c_int]),
         "dq_context_last_batch_stats": (None, [vp, C.POINTER(BatchStats)]),
+        "dq_map_colors_batch_device": (None, [vp, C.c_uint32, _u32p, C.c_uint32, vp, vp, C.POINTER(C.c_int), _u32p, vp]),
+        "dq_map_colors_batch_ctx": (None, [vp, C.c_uint32, _u32p, C.c_uint32, _u32p, _u32p, C.POINTER(C.c_int), _u32p, _u32p]),
         "dq_context_set_split_ctas": (None, [vp, C.c_int]),
         "dq_context_set_exact_small": (None, [vp, C.c_int]),
         "dq_context_set_exact_max_points": (None, [vp, C.c_uint32]),
@@ -138,6 +140,7 @@ def load_library(path=LIB_PATH):
         "dq_host_dedup_palette": (C.c_uint32, [_u32p, C.c_uint32]),
         "dq_host_select_cut_overrides": (C.c_uint32, [_u32p, _u32p, _u32p, C.c_uint32, C.c_uint32, _u32p]),
         "dq_host_build_search_tables": (None, [_u32p, C.c_int, _u32p, C.POINTER(C.c_int32)]),
+        "dq_host_build_label_table": (None, [_u32p, C.c_int, _u32p]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(lib, name)
@@ -155,7 +158,9 @@ EXPORTED_C_SYMBOLS = [
     "dq_pipeline_context", "dq_pipeline_kernel_launches", "dq_pipeline_flagged_frames",
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
     "dq_quant_recurse_batch_device", "dq_quant_recurse_batch_ctx", "dq_context_last_batch_stats",
+    "dq_map_colors_batch_device", "dq_map_colors_batch_ctx",
     "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
+    "dq_host_build_label_table",
 ]
 
 # The reference's own symbol names (SURVEY.md 8b), exported for relinking the reference's callers.
@@ -239,6 +244,51 @@ class DivQuant:
             self.lib.dq_quant_recurse_batch_device(ctx or self.lib.dq_default_context(), nk.size, _p(offs), flat.numel(),
                                                    flat.data_ptr(), out.data_ptr(), _p(nk), _p(ct), all_unique)
         return out, ct, nk
+
+    def map_colors_batch(self, items, palettes, labels=False, ctx=None):
+        """map_colors_mps of every pixel set in `items` to its own palette in `palettes`, in one call
+        (dq_map_colors_batch_ctx).  Returns a list of outputs, each equal to map_colors_mps(items[i], palettes[i]) on the
+        same context; with labels=True a list of (out, labels) pairs, labels = colortable_indexes(out, palettes[i])."""
+        arrs = [_u32(a) for a in items]
+        pals = [_u32(p) for p in palettes]
+        if len(arrs) != len(pals):
+            raise ValueError("one palette per item")
+        if not arrs:
+            return []
+        offsets = np.zeros(len(arrs) + 1, np.uint32)
+        np.cumsum([a.size for a in arrs], out=offsets[1:])
+        flat = np.concatenate(arrs) if offsets[-1] else np.zeros(1, np.uint32)
+        out = np.zeros_like(flat)
+        lab = np.zeros_like(flat) if labels else None
+        sizes = np.asarray([p.size for p in pals], np.int32)
+        ct = np.concatenate(pals) if sizes.sum() else np.zeros(1, np.uint32)
+        self.lib.dq_map_colors_batch_ctx(ctx or self.lib.dq_default_context(), len(arrs), _p(offsets), flat.size, _p(flat), _p(out),
+                                         sizes.ctypes.data_as(C.POINTER(C.c_int)), _p(ct), _p(lab) if labels else None)
+        outs = [out[offsets[i]:offsets[i + 1]].copy() for i in range(len(arrs))]
+        if not labels:
+            return outs
+        return [(o, lab[offsets[i]:offsets[i + 1]].copy()) for i, o in enumerate(outs)]
+
+    def map_colors_batch_device(self, flat, offsets, palettes, labels=False, ctx=None, out=None):
+        """Device form (dq_map_colors_batch_device): `flat` is a CUDA tensor of 32-bit pixels holding the items end to
+        end, item i = flat[offsets[i]:offsets[i+1]], mapped to palettes[i].  Returns (out tensor, labels tensor or None)."""
+        import torch
+        offs = _u32(offsets)
+        pals = [_u32(p) for p in palettes]
+        if offs.size != len(pals) + 1:
+            raise ValueError("offsets need one entry more than palettes")
+        if flat.dtype not in (torch.int32, torch.uint32) or not flat.is_cuda or not flat.is_contiguous():
+            raise ValueError("flat must be a contiguous CUDA tensor of 32-bit pixels")
+        out = torch.empty_like(flat) if out is None else out
+        lab = torch.empty_like(flat) if labels else None
+        sizes = np.asarray([p.size for p in pals], np.int32)
+        ct = np.concatenate(pals) if sizes.sum() else np.zeros(1, np.uint32)
+        if pals:
+            torch.cuda.current_stream(flat.device).synchronize()  # the library works on its context's stream
+            self.lib.dq_map_colors_batch_device(ctx or self.lib.dq_default_context(), len(pals), _p(offs), flat.numel(),
+                                                flat.data_ptr(), out.data_ptr(), sizes.ctypes.data_as(C.POINTER(C.c_int)), _p(ct),
+                                                lab.data_ptr() if labels else None)
+        return out, lab
 
     def last_batch_stats(self, ctx=None):
         st = BatchStats()
@@ -324,6 +374,14 @@ class DivQuant:
         lut = np.zeros(766, np.int32)
         self.lib.dq_host_build_search_tables(_p(ct), ct.size, _p(srt), lut.ctypes.data_as(C.POINTER(C.c_int32)))
         return srt, lut
+
+    def host_build_label_table(self, colortable):
+        """For each entry of host_build_search_tables' sorted palette, the index of the last entry of `colortable` with
+        that 24-bit colour."""
+        ct = _u32(colortable).copy()
+        lab = np.zeros_like(ct)
+        self.lib.dq_host_build_label_table(_p(ct), ct.size, _p(lab))
+        return lab
 
     # -- diagnostics ---------------------------------------------------------------------------
     def last_stats(self, ctx=None):

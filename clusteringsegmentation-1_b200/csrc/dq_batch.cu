@@ -116,17 +116,25 @@ __global__ void __launch_bounds__(kBatchThreads, 1) batch_split_kernel(const Bat
 constexpr int kRemapPix = kBatchTilePixels / kBatchThreads;  // pixels per thread and tile
 static_assert(kBatchTilePixels % kBatchThreads == 0, "whole tiles");
 
+// kLabels: also labels[p] = the caller's palette index of the entry pixel p maps to, from the item's label table
+// (label_tables + the item's sorted-palette offset, one entry per sorted position).  The parameters after luts are only
+// read by that instantiation.
+template <bool kLabels>
 __global__ void __launch_bounds__(kBatchThreads) batch_remap_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out,
                                                                      const BatchTile *tiles, const uint32_t *sorted, const uint2 *tables,
-                                                                     const uint16_t *luts) {
+                                                                     const uint16_t *luts, const uint16_t *label_tables,
+                                                                     uint32_t *__restrict__ labels) {
   __shared__ __align__(16) int4 s_ent[kIntColors];
   __shared__ int s_lut[kBatchLutEntries];
+  __shared__ uint16_t s_lab[kLabels ? kIntColors : 1];
   const BatchTile t = tiles[blockIdx.x];
   const uint2 tab = tables[t.table];  // (offset of the item's sorted palette, its size)
   const int k = (int)tab.y;
   stage_palette_int(sorted + tab.x, k, s_ent);
   const uint16_t *lut = luts + (size_t)t.table * kBatchLutEntries;
   for (int i = threadIdx.x; i < kBatchLutEntries; i += kBatchThreads) s_lut[i] = (int)lut[i];
+  if constexpr (kLabels)
+    for (int i = threadIdx.x; i < k; i += kBatchThreads) s_lab[i] = label_tables[tab.x + i];
   __syncthreads();
   uint32_t c[kRemapPix];
   int lo[kRemapPix], hi[kRemapPix];
@@ -139,7 +147,11 @@ __global__ void __launch_bounds__(kBatchThreads) batch_remap_kernel(const uint32
 #pragma unroll
   for (int q = 0; q < kRemapPix; ++q) {
     const uint32_t p = t.begin + threadIdx.x + (uint32_t)q * kBatchThreads;
-    if (p < t.end) out[p] = resolve_int(s_ent, c[q], s_lut[((c[q] >> 16) & 0xFF) + ((c[q] >> 8) & 0xFF) + (c[q] & 0xFF)], lo[q], hi[q]);
+    if (p < t.end) {
+      const int win = resolve_int_index(s_ent, c[q], s_lut[((c[q] >> 16) & 0xFF) + ((c[q] >> 8) & 0xFF) + (c[q] & 0xFF)], lo[q], hi[q]);
+      out[p] = (uint32_t)s_ent[win].w;
+      if constexpr (kLabels) labels[p] = s_lab[win];
+    }
   }
 }
 
@@ -163,8 +175,13 @@ void batch_split_launch(const BatchItem *d_items, uint32_t num_items, uint32_t m
 }
 
 void batch_remap_launch(const uint32_t *d_in, uint32_t *d_out, const BatchTile *d_tiles, uint32_t num_tiles, const uint32_t *d_sorted,
-                        const uint2 *d_tables, const uint16_t *d_luts, cudaStream_t st) {
-  batch_remap_kernel<<<num_tiles, kBatchThreads, 0, st>>>(d_in, d_out, d_tiles, d_sorted, d_tables, d_luts);
+                        const uint2 *d_tables, const uint16_t *d_luts, const uint16_t *d_label_tables, uint32_t *d_labels,
+                        cudaStream_t st) {
+  if (d_labels != nullptr)
+    batch_remap_kernel<true><<<num_tiles, kBatchThreads, 0, st>>>(d_in, d_out, d_tiles, d_sorted, d_tables, d_luts, d_label_tables,
+                                                                  d_labels);
+  else
+    batch_remap_kernel<false><<<num_tiles, kBatchThreads, 0, st>>>(d_in, d_out, d_tiles, d_sorted, d_tables, d_luts, nullptr, nullptr);
   DQ_CUDA_CHECK(cudaGetLastError());
 }
 

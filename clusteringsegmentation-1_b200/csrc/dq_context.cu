@@ -26,6 +26,7 @@
 
 #include "../../include/divquant_b200.h"
 #include "dq_kernels.cuh"
+#include "dq_map_int.cuh"
 #include "dq_split.cuh"
 
 namespace {
@@ -182,7 +183,8 @@ struct dq_context {
   uint32_t mailbox_seq = 0;
   // quant_recurse over a batch of items (dq_batch.cu; quant_recurse_batch below)
   DevBuf<uint32_t> b_work;    // [items | per-item results | palettes | histogram slices: colours, counts, first seen]
-  DevBuf<uint32_t> b_tables;  // [remap tiles | per-item (offset, size) | sorted palettes | lut_init as uint16]
+  DevBuf<uint32_t> b_tables;  // [remap tiles | per-item (offset, size) | sorted palettes | lut_init, label tables as uint16]
+  DevBuf<uint32_t> b_labels;  // label image of dq_map_colors_batch_ctx
   DevBuf<uint32_t> b_cluster_size;
   DevBuf<double> b_cluster_mean;
   PinnedBuf b_up, b_down, b_tab;
@@ -259,6 +261,19 @@ void build_search_tables(const uint32_t *colortable, int n, uint32_t *sorted_out
     low = (int)(0.5 * (v[ic - 1].weight + v[ic].weight) + 0.5);
     high = (int)(0.5 * (v[ic].weight + v[ic + 1].weight) + 0.5);
     for (int k = low; k < high; ++k) lut_out[k] = ic;
+  }
+}
+
+// For every entry of the sorted palette of build_search_tables, the caller's index of the LAST palette entry with that
+// 24-bit colour: the label mapQuantPixelsToColortableIndexes gives a pixel mapped to it (it fills an unordered_map in
+// palette order, OpenCVUtil.cpp:795-799).
+void build_label_table(const uint32_t *colortable, int n, const uint32_t *sorted, uint32_t *labels_out) {
+  std::vector<uint64_t> keyed((size_t)n);  // (colour, index): ascending colour, then ascending index
+  for (int i = 0; i < n; ++i) keyed[i] = ((uint64_t)(colortable[i] & 0x00FFFFFFu) << 32) | (uint32_t)i;
+  std::sort(keyed.begin(), keyed.end());
+  for (int s = 0; s < n; ++s) {
+    const uint64_t past = ((uint64_t)sorted[s] + 1) << 32;  // every sorted entry is in the palette: the one before is its last
+    labels_out[s] = (uint32_t)*(std::lower_bound(keyed.begin(), keyed.end(), past) - 1);
   }
 }
 
@@ -924,8 +939,8 @@ void quant_recurse_device_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in
 }
 
 // ---- quant_recurse over a batch of items (kernels: dq_batch.cu) -------------------------------------------------------
-// Fatal like every other bad argument: offsets that decrease or end beyond the input, an item with no pixels or K = 0.
-void check_batch_args(uint32_t num_items, const uint32_t *offsets, uint32_t num_pixels, const uint32_t *ks) {
+// Fatal like every other bad argument: offsets that decrease or end beyond the input.
+void check_batch_offsets(uint32_t num_items, const uint32_t *offsets, uint32_t num_pixels) {
   for (uint32_t i = 0; i < num_items; ++i) {
     if (offsets[i + 1] < offsets[i]) {
       fprintf(stderr, "divquant_b200: batch offsets decrease at item %u (%u -> %u)\n", i, offsets[i], offsets[i + 1]);
@@ -936,8 +951,65 @@ void check_batch_args(uint32_t num_items, const uint32_t *offsets, uint32_t num_
     fprintf(stderr, "divquant_b200: batch offsets end at %u, beyond the %u input pixels\n", offsets[num_items], num_pixels);
     abort();
   }
+}
+
+// ... and for quant_recurse, an item with no pixels or K = 0.
+void check_batch_args(uint32_t num_items, const uint32_t *offsets, uint32_t num_pixels, const uint32_t *ks) {
+  check_batch_offsets(num_items, offsets, num_pixels);
   for (uint32_t i = 0; i < num_items; ++i) check_quant_args(offsets[i + 1] - offsets[i], ks[i], 8);
 }
+
+// The batch remap (batch_remap_kernel) of the items added to it: per item its sorted palette, lut_init and, for a label
+// image, its label table, plus its pixels cut into kBatchTilePixels tiles.  run() sends all of it up in one copy and
+// launches one kernel.
+struct BatchRemap {
+  std::vector<BatchTile> tiles;
+  std::vector<uint2> tabs;  // (offset in sorted, palette size) per item
+  std::vector<uint32_t> sorted;
+  std::vector<uint16_t> luts, labels;  // labels: one per sorted entry, at the same offsets as sorted
+
+  // pixels [begin, begin + n) of the launch's input mapped to colortable[0, k), k <= kIntColors
+  void add(const uint32_t *colortable, uint32_t k, uint32_t begin, uint32_t n, bool with_labels) {
+    const uint32_t t = (uint32_t)tabs.size(), off = (uint32_t)sorted.size();
+    tabs.push_back(make_uint2(off, k));
+    sorted.resize(off + k);
+    int lut[kLutEntries];
+    build_search_tables(colortable, (int)k, sorted.data() + off, lut);
+    for (int e = 0; e < kLutEntries; ++e) luts.push_back((uint16_t)lut[e]);
+    if (with_labels) {
+      uint32_t lab[kIntColors];
+      build_label_table(colortable, (int)k, sorted.data() + off, lab);
+      labels.insert(labels.end(), lab, lab + k);
+    }
+    for (uint32_t b = 0; b < n; b += (uint32_t)kBatchTilePixels)
+      tiles.push_back({begin + b, begin + std::min<uint32_t>(n, b + (uint32_t)kBatchTilePixels), t, 0u});
+  }
+
+  // d_labels: nullptr, or (when every item was added with labels) the label image.  Returns the kernels launched.
+  uint32_t run(dq_context *ctx, const uint32_t *d_in, uint32_t *d_out, uint32_t *d_labels) {
+    if (tiles.empty()) return 0;
+    // tiles, (offset, size) per item, sorted palettes, lut_init and label tables go up in one copy
+    static_assert(sizeof(BatchTile) == 4 * sizeof(uint32_t), "four words per tile");
+    const size_t w_tiles = 4 * tiles.size(), w_tabs = 2 * tabs.size(), w_u16 = (luts.size() + labels.size() + 1) / 2;
+    const size_t words = w_tiles + w_tabs + sorted.size() + w_u16;
+    ctx->b_tab.ensure(words);
+    uint32_t *h = ctx->b_tab.ptr;
+    memcpy(h, tiles.data(), w_tiles * sizeof(uint32_t));
+    memcpy(h + w_tiles, tabs.data(), w_tabs * sizeof(uint32_t));
+    memcpy(h + w_tiles + w_tabs, sorted.data(), sorted.size() * sizeof(uint32_t));
+    uint16_t *h16 = reinterpret_cast<uint16_t *>(h + w_tiles + w_tabs + sorted.size());
+    memcpy(h16, luts.data(), luts.size() * sizeof(uint16_t));
+    memcpy(h16 + luts.size(), labels.data(), labels.size() * sizeof(uint16_t));
+    ctx->b_tables.ensure(words);
+    uint32_t *d = ctx->b_tables.ptr;
+    DQ_CUDA_CHECK(cudaMemcpyAsync(d, h, words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    const uint16_t *d16 = reinterpret_cast<const uint16_t *>(d + w_tiles + w_tabs + sorted.size());
+    batch_remap_launch(d_in, d_out, reinterpret_cast<const BatchTile *>(d), (uint32_t)tiles.size(), d + w_tiles + w_tabs,
+                       reinterpret_cast<const uint2 *>(d + w_tiles), d16, d16 + luts.size(), d_labels, ctx->stream);
+    ctx->wait();
+    return 1;
+  }
+};
 
 // Every item gets what quant_recurse_device_impl gives it alone on this context.  An item is batched when the single call
 // would split it on the ordered path in shared memory: weighted (all_unique = 0), K <= kSplit2MaxColors and at most
@@ -986,12 +1058,9 @@ void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_
     DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->b_down.ptr, d_res, (w_res + sum_k) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
     ctx->wait();
   }
-  std::vector<BatchTile> tiles;
-  std::vector<uint2> tabs;
-  std::vector<uint32_t> sorted;
-  std::vector<uint16_t> luts;
-  tabs.reserve(nc);
-  luts.reserve((size_t)nc * kLutEntries);
+  BatchRemap remap;
+  remap.tabs.reserve(nc);
+  remap.luts.reserve((size_t)nc * kLutEntries);
   double host_ms = 0.0;
   size_t pal_off = 0;
   for (uint32_t i = 0; i < num_items; ++i) {
@@ -1012,15 +1081,7 @@ void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_
       if (empty) fprintf(stderr, "# empty clusters: %d\n", (int)empty);  // (:1067-1070)
       const uint32_t k = dedup_palette(ct, actual);
       ks[i] = k;
-      const uint32_t t = (uint32_t)tabs.size();
-      tabs.push_back(make_uint2((uint32_t)sorted.size(), k));
-      sorted.resize(sorted.size() + k);
-      int lut[kLutEntries];
-      build_search_tables(ct, (int)k, sorted.data() + tabs.back().x, lut);
-      for (int e = 0; e < kLutEntries; ++e) luts.push_back((uint16_t)lut[e]);
-      const uint32_t b0 = offsets[i] - base;
-      for (uint32_t b = 0; b < n; b += (uint32_t)kBatchTilePixels)
-        tiles.push_back({b0 + b, b0 + std::min<uint32_t>(n, b + (uint32_t)kBatchTilePixels), t, 0u});
+      remap.add(ct, k, offsets[i] - base, n, false);
       bs.batched_items++;
       bs.empty_clusters += empty;
       host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1033,27 +1094,67 @@ void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_
       bs.single_call_items++;
     }
   }
-  if (!tiles.empty()) {
-    // tiles, (offset, size) per item, sorted palettes and lut_init go up in one copy
-    static_assert(sizeof(BatchTile) == 4 * sizeof(uint32_t), "four words per tile");
-    const size_t w_tiles = 4 * tiles.size(), w_tabs = 2 * tabs.size(), w_luts = (luts.size() + 1) / 2;
-    const size_t words = w_tiles + w_tabs + sorted.size() + w_luts;
-    ctx->b_tab.ensure(words);
-    uint32_t *h = ctx->b_tab.ptr;
-    memcpy(h, tiles.data(), w_tiles * sizeof(uint32_t));
-    memcpy(h + w_tiles, tabs.data(), w_tabs * sizeof(uint32_t));
-    memcpy(h + w_tiles + w_tabs, sorted.data(), sorted.size() * sizeof(uint32_t));
-    memcpy(h + w_tiles + w_tabs + sorted.size(), luts.data(), luts.size() * sizeof(uint16_t));
-    ctx->b_tables.ensure(words);
-    uint32_t *d = ctx->b_tables.ptr;
-    DQ_CUDA_CHECK(cudaMemcpyAsync(d, h, words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    batch_remap_launch(d_in + base, d_out + base, reinterpret_cast<const BatchTile *>(d), (uint32_t)tiles.size(), d + w_tiles + w_tabs,
-                       reinterpret_cast<const uint2 *>(d + w_tiles), reinterpret_cast<const uint16_t *>(d + w_tiles + w_tabs + sorted.size()),
-                       ctx->stream);
-    launches++;
-    ctx->wait();
-  }
+  launches += remap.run(ctx, d_in + base, d_out + base, nullptr);
   memset(&ctx->stats, 0, sizeof(ctx->stats));  // (dq_call_stats describes one frame: only the launches are kept)
+  ctx->stats.kernel_launches = launches;
+  bs.kernel_launches = launches;
+  bs.host_palette_ms = (float)host_ms;
+}
+
+// Fatal before any device work: bad offsets, an empty palette, and with labels a palette above dq_colortable_indexes'
+// limit.
+void check_map_batch_args(uint32_t num_items, const uint32_t *offsets, uint32_t num_pixels, const int *sizes, bool labels) {
+  check_batch_offsets(num_items, offsets, num_pixels);
+  for (uint32_t i = 0; i < num_items; ++i) {
+    if (sizes[i] <= 0) {
+      fprintf(stderr, "divquant_b200: batch item %u has a colortable of %d entries; map_colors_mps needs a non-empty one\n", i,
+              sizes[i]);
+      abort();  // assert(num_colors > 0) (:266)
+    }
+    if (labels && sizes[i] > 24000) {
+      fprintf(stderr, "divquant_b200: batch item %u has a colortable of %d entries; label images support 1..24000\n", i, sizes[i]);
+      abort();
+    }
+  }
+}
+
+// Every item gets what dq_map_colors_device (prefer_table = 1) gives it alone on this context, and with d_labels its
+// dq_colortable_indexes (asGreyscale = 0).  Items whose palette fits the integer arg-min (<= kIntColors entries) go
+// through one batch remap launch; the others run the single call in item order.  Items with no pixels write nothing.
+void map_colors_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, const uint32_t *d_in, uint32_t *d_out,
+                           const int *sizes, const uint32_t *colortables, uint32_t *d_labels) {
+  dq_batch_stats &bs = ctx->batch_stats;
+  bs = dq_batch_stats();
+  bs.items = num_items;
+  uint32_t launches = 0;
+  const uint32_t base = offsets[0];
+  BatchRemap remap;
+  double host_ms = 0.0;
+  size_t pal_off = 0;
+  for (uint32_t i = 0; i < num_items; ++i) {
+    const uint32_t n = offsets[i + 1] - offsets[i];
+    const int k = sizes[i];
+    const uint32_t *const ct = colortables + pal_off;
+    pal_off += (size_t)k;
+    if (k <= kIntColors) {
+      bs.batched_items++;
+      if (n == 0) continue;
+      const auto t0 = std::chrono::steady_clock::now();
+      remap.add(ct, (uint32_t)k, offsets[i] - base, n, d_labels != nullptr);
+      host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    } else {
+      bs.single_call_items++;
+      if (n == 0) continue;
+      dq_map_colors_device(ctx, d_in + offsets[i], n, d_out + offsets[i], ct, k, 1);
+      launches += ctx->stats.kernel_launches;
+      if (d_labels != nullptr) {
+        dq_colortable_indexes_device(ctx, d_out + offsets[i], n, ct, k, d_labels + offsets[i], 0);
+        launches++;  // map_labels
+      }
+    }
+  }
+  launches += remap.run(ctx, d_in + base, d_out + base, d_labels != nullptr ? d_labels + base : nullptr);
+  memset(&ctx->stats, 0, sizeof(ctx->stats));  // (as after a quant_recurse batch: only the launches are kept)
   ctx->stats.kernel_launches = launches;
   bs.kernel_launches = launches;
   bs.host_palette_ms = (float)host_ms;
@@ -1091,6 +1192,13 @@ uint32_t dq_host_dedup_palette(uint32_t *colortable, uint32_t num_colors) { retu
 
 void dq_host_build_search_tables(const uint32_t *colortable, int num_colors, uint32_t *sorted_out, int32_t *lut_init_out) {
   build_search_tables(colortable, num_colors, sorted_out, lut_init_out);
+}
+
+void dq_host_build_label_table(const uint32_t *colortable, int num_colors, uint32_t *labels_out) {
+  std::vector<uint32_t> sorted((size_t)num_colors);
+  int lut[kLutEntries];
+  build_search_tables(colortable, num_colors, sorted.data(), lut);
+  build_label_table(colortable, num_colors, sorted.data(), labels_out);
 }
 
 uint32_t dq_host_select_cut_overrides(const uint32_t *begin, const uint32_t *size, const uint32_t *status, uint32_t n,
@@ -1197,6 +1305,7 @@ void dq_context_destroy(dq_context *ctx) {
   ctx->d_sortvals.release();
   ctx->b_work.release();
   ctx->b_tables.release();
+  ctx->b_labels.release();
   ctx->b_cluster_size.release();
   ctx->b_cluster_mean.release();
   ctx->b_up.release();
@@ -1309,6 +1418,14 @@ void dq_quant_recurse_batch_device(dq_context *ctx, uint32_t num_items, const ui
   quant_recurse_batch_impl(ctx, num_items, offsets, d_in, d_out, numClusters, colortables, allPixelsUnique);
 }
 
+void dq_map_colors_batch_device(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *d_in,
+                                uint32_t *d_out, const int *colormapSizes, const uint32_t *colortables, uint32_t *d_labels) {
+  if (num_items == 0) return;
+  require_device(ctx);
+  check_map_batch_args(num_items, offsets, numPixels, colormapSizes, d_labels != nullptr);
+  map_colors_batch_impl(ctx, num_items, offsets, d_in, d_out, colormapSizes, colortables, d_labels);
+}
+
 void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out) { *out = ctx->batch_stats; }
 
 // ---- host-pointer entry points ----
@@ -1327,6 +1444,27 @@ void dq_quant_recurse_batch_ctx(dq_context *ctx, uint32_t num_items, const uint3
   DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels + base, (size_t)total * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   quant_recurse_batch_impl(ctx, num_items, local.data(), ctx->d_in.ptr, ctx->d_out.ptr, numClusters, colortables, allPixelsUnique);
   DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels + base, ctx->d_out.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+}
+
+void dq_map_colors_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *inPixels,
+                             uint32_t *outPixels, const int *colormapSizes, const uint32_t *colortables, uint32_t *labels) {
+  if (num_items == 0) return;
+  require_device(ctx);
+  check_map_batch_args(num_items, offsets, numPixels, colormapSizes, labels != nullptr);
+  // only the pixels the items cover travel, from offsets[0] on
+  const uint32_t base = offsets[0], total = offsets[num_items] - base;
+  std::vector<uint32_t> local(offsets, offsets + num_items + 1);
+  for (uint32_t &o : local) o -= base;
+  ctx->d_in.ensure(total);
+  ctx->d_out.ensure(total);
+  if (labels != nullptr) ctx->b_labels.ensure(total);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels + base, (size_t)total * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  map_colors_batch_impl(ctx, num_items, local.data(), ctx->d_in.ptr, ctx->d_out.ptr, colormapSizes, colortables,
+                        labels != nullptr ? ctx->b_labels.ptr : nullptr);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels + base, ctx->d_out.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (labels != nullptr)
+    DQ_CUDA_CHECK(cudaMemcpyAsync(labels + base, ctx->b_labels.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
 }
 

@@ -82,8 +82,10 @@ void batch_split_launch(const BatchItem *d_items, uint32_t num_items, uint32_t m
                         const uint32_t *d_first, uint32_t *d_res, uint32_t *d_palette, uint32_t *d_cluster_size, double *d_cluster_mean,
                         cudaStream_t st);
 // d_tables[i] = (offset in d_sorted, palette size) of batched item i, d_luts[i * kBatchLutEntries ...] its lut_init.
+// d_labels != nullptr: also d_labels[p] = d_label_tables[offset + w] for the sorted entry w that pixel p maps to.
 void batch_remap_launch(const uint32_t *d_in, uint32_t *d_out, const BatchTile *d_tiles, uint32_t num_tiles, const uint32_t *d_sorted,
-                        const uint2 *d_tables, const uint16_t *d_luts, cudaStream_t st);
+                        const uint2 *d_tables, const uint16_t *d_luts, const uint16_t *d_label_tables, uint32_t *d_labels,
+                        cudaStream_t st);
 
 // ---- dq_srm.cu ----
 uint32_t srm_num_pairs(uint32_t width, uint32_t height);

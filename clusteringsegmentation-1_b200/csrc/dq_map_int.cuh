@@ -49,8 +49,8 @@ __device__ __forceinline__ void nearest_int(const int4 *s_ent, int num_colors, c
   }
 }
 
-// The palette word for one colour from its two keys; s = the reference's start index for it.
-__device__ __forceinline__ uint32_t resolve_int(const int4 *s_ent, uint32_t c, int s, int lo, int hi) {
+// The sorted-palette index of the entry one colour maps to, from its two keys; s = the reference's start index for it.
+__device__ __forceinline__ int resolve_int_index(const int4 *s_ent, uint32_t c, int s, int lo, int hi) {
   const int ka = 511 - (lo & 511), kb = hi & 511;
   int win = ka;
   if (ka != kb) {
@@ -69,7 +69,12 @@ __device__ __forceinline__ uint32_t resolve_int(const int4 *s_ent, uint32_t c, i
       }
     }
   }
-  return (uint32_t)s_ent[win].w;
+  return win;
+}
+
+// The palette word for one colour from its two keys.
+__device__ __forceinline__ uint32_t resolve_int(const int4 *s_ent, uint32_t c, int s, int lo, int hi) {
+  return (uint32_t)s_ent[resolve_int_index(s_ent, c, s, lo, hi)].w;
 }
 
 }  // namespace dq

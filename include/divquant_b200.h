@@ -349,6 +349,32 @@ typedef struct {
 } dq_batch_stats;
 void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out);
 
+/* map_colors_mps over num_items independent pixel sets, each mapped to its OWN palette (the per-region remaps of
+ * ClusteringSegmentation.cpp:2434, :3816), optionally with the label image mapQuantPixelsToColortableIndexes makes of the
+ * result (OpenCVUtil.cpp:787-849).  Item i is pixels [offsets[i], offsets[i+1]) of the input; its palette is
+ * colortables[P_i, P_i + colormapSizes[i]), P_i = the sum of colormapSizes of the items before i (the packing of the
+ * quant_recurse batch).  Palettes may hold duplicates, alpha bits, equal r+g+b sums and colours absent from the item.
+ *   out:    for every item, bit for bit what dq_map_colors_device (prefer_table = 1) on this context returns for it alone:
+ *           alpha ignored on input, zero on output.
+ *   labels: NULL = none; else labels[p] = dq_colortable_indexes(out of that item, its palette, asGreyscale = 0)[p]: the
+ *           0-based index within the item's palette of the LAST entry whose 24-bit colour equals out[p].
+ *   offsets, colormapSizes, colortables: HOST arrays (num_items + 1, num_items and sum of colormapSizes words).
+ * An item whose palette has at most 512 entries is mapped by one batch remap launch over 1024-pixel tiles of all such
+ * items (an all-batched call is one kernel launch, with or without labels); every other item runs dq_map_colors_device
+ * (and, for labels, dq_colortable_indexes_device) in item order inside the same call.
+ * Decreasing offsets, offsets beyond numPixels, colormapSizes[i] <= 0 and, with labels, colormapSizes[i] > 24000 are
+ * fatal (message + abort) before any device work.  An item with no pixels writes nothing; num_items = 0 does nothing.
+ * d_out and d_labels must not overlap d_in or each other.  The _ctx form copies only pixels offsets[0] .. offsets[num_items]
+ * and copies labels back only when asked for.  Synchronous on return, no timing lines.  Afterwards dq_call_stats is zeroed
+ * apart from kernel_launches; dq_context_last_batch_stats gives items, batched_items (palettes <= 512 entries),
+ * single_call_items, empty_clusters = 0, kernel_launches and host_palette_ms (building the search and label tables). */
+void dq_map_colors_batch_device(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels,
+                                const uint32_t *d_in, uint32_t *d_out, const int *colormapSizes,
+                                const uint32_t *colortables, uint32_t *d_labels);
+void dq_map_colors_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels,
+                             const uint32_t *inPixels, uint32_t *outPixels, const int *colormapSizes,
+                             const uint32_t *colortables, uint32_t *labels);
+
 /* ------------------------------------------------------------------------------------------------
  * 3. Test hooks (used by tests/ to compare intermediate results with the oracle).
  * ---------------------------------------------------------------------------------------------- */
@@ -385,9 +411,12 @@ uint32_t dq_debug_split_timeline(dq_context *ctx, int enable, uint64_t *pairs_ou
  * kernels, exposed so that CPU-only tests can check it against the oracle.
  *   dq_host_dedup_palette       first occurrence wins, order kept (quant_util.cpp:93-118); returns the new size.
  *   dq_host_build_search_tables sorted palette (the reference's std::sort by r+g+b) and lut_init[766]
- *                               (DivQuantMapColors.cpp:267-383). */
+ *                               (DivQuantMapColors.cpp:267-383).
+ *   dq_host_build_label_table   for each position s of that sorted palette, the caller's index of the last entry with
+ *                               that 24-bit colour: the per-item table the batch remap reads for labels. */
 uint32_t dq_host_dedup_palette(uint32_t *colortable, uint32_t num_colors);
 void dq_host_build_search_tables(const uint32_t *colortable, int num_colors, uint32_t *sorted_out, int32_t *lut_init_out);
+void dq_host_build_label_table(const uint32_t *colortable, int num_colors, uint32_t *labels_out);
 /* Host logic of the re-split with forced cuts (dq_call_stats::cut_overrides): of n <= 16 flagged cut entries, each a range
  * [begin, begin + size) of point positions with the resolver's status (3 = the reference cuts this node elsewhere), which
  * ones are forced in the next run -- the status-3 entries whose range does not lie inside another status-3 entry's, while

@@ -575,14 +575,15 @@ void remap_bruteforce(dq_context *ctx, const uint32_t *d_in, uint32_t n, uint32_
 
 // Table path: requires the unique list of exactly these pixels in d_uniq / d_cb->ucount.
 void remap_through_table(dq_context *ctx, const uint32_t *d_in, uint32_t n, uint32_t *d_out, int k, uint32_t u_hint) {
+  if (k > map_smem_palette_limit()) ctx->d_pal_scratch.ensure(k);
   ctx->mark(4);
-  map_unique(ctx->d_uniq.ptr, &ctx->d_cb->ucount, u_hint, ctx->d_map, ctx->d_sorted.ptr, k, ctx->d_lut, ctx->sm_count,
-             ctx->stream);
+  map_unique(ctx->d_uniq.ptr, &ctx->d_cb->ucount, u_hint, ctx->d_map, ctx->d_sorted.ptr, k, ctx->d_lut, ctx->d_pal_scratch.ptr,
+             ctx->sm_count, ctx->stream);
   ctx->mark(5);
   map_gather(d_in, n, d_out, ctx->d_map, ctx->sm_count, ctx->stream);
   ctx->mark(6);
   ctx->mark(7);
-  ctx->stats.kernel_launches += 2;
+  ctx->stats.kernel_launches += (k > map_smem_palette_limit()) ? 3 : 2;
   ctx->stats.remap_path = 2;
 }
 

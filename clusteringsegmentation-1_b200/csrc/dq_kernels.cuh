@@ -42,8 +42,9 @@ void hist_merge_first(const uint32_t *d_colours, const uint32_t *d_counts, const
 int map_smem_palette_limit();
 void map_pixels(const uint32_t *d_in, uint32_t n, uint32_t *d_out, const uint32_t *d_sorted, int num_colors,
                 const int *d_lut, int4 *d_pal_scratch, int sm_count, cudaStream_t st);
+// d_pal_scratch: num_colors int4 entries, used above map_smem_palette_limit() (as by map_pixels)
 void map_unique(const uint32_t *d_uniq, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_table,
-                const uint32_t *d_sorted, int num_colors, const int *d_lut, int sm_count, cudaStream_t st);
+                const uint32_t *d_sorted, int num_colors, const int *d_lut, int4 *d_pal_scratch, int sm_count, cudaStream_t st);
 // Sorted palette and start-index table small enough (K <= 256) to travel inside the kernel's parameter block: no
 // upload, no extra dependency between the host's table building and the launch.
 struct MapTablesParam {

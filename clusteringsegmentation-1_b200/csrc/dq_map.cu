@@ -281,6 +281,17 @@ __global__ void __launch_bounds__(kMapThreads) map_pixels_big_kernel(const uint3
     out[i] = nearest_entry(in[i], pal, num_colors, lut_init);
 }
 
+// One evaluation per unique colour, palette read from global memory (palettes too large for shared memory).
+__global__ void __launch_bounds__(kMapThreads) map_unique_big_kernel(const uint32_t *__restrict__ uniq, const uint32_t *ucount,
+                                                                    uint32_t *table, const int4 *pal, int num_colors,
+                                                                    const int *lut_init) {
+  const uint32_t u = *ucount;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < u; i += gridDim.x * blockDim.x) {
+    const uint32_t c = uniq[i] & 0xFFFFFFu;
+    table[c] = 0x80000000u | nearest_entry(c, pal, num_colors, lut_init);
+  }
+}
+
 __global__ void __launch_bounds__(kMapThreads) expand_palette_kernel(const uint32_t *sorted, int num_colors, int4 *pal) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < num_colors; k += gridDim.x * blockDim.x) {
     const uint32_t c = sorted[k] & 0x00FFFFFFu;
@@ -456,7 +467,15 @@ void map_pixels(const uint32_t *d_in, uint32_t n, uint32_t *d_out, const uint32_
 }
 
 void map_unique(const uint32_t *d_uniq, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_table,
-                const uint32_t *d_sorted, int num_colors, const int *d_lut, int sm_count, cudaStream_t st) {
+                const uint32_t *d_sorted, int num_colors, const int *d_lut, int4 *d_pal_scratch, int sm_count, cudaStream_t st) {
+  if (num_colors > map_smem_palette_limit()) {
+    expand_palette_kernel<<<blocks_for(num_colors, kMapThreads, sm_count, 1), kMapThreads, 0, st>>>(d_sorted, num_colors,
+                                                                                                   d_pal_scratch);
+    map_unique_big_kernel<<<blocks_for(u_hint, kMapThreads, sm_count, 8), kMapThreads, 0, st>>>(d_uniq, d_ucount, d_table,
+                                                                                               d_pal_scratch, num_colors, d_lut);
+    DQ_CUDA_CHECK(cudaGetLastError());
+    return;
+  }
   const size_t smem = fast_smem_bytes(num_colors);
   DQ_RAISE_SMEM(map_unique_fast_kernel, smem);
   int per_sm = (int)std::min<size_t>(8, std::max<size_t>(1, (200 * 1024) / smem));

@@ -112,8 +112,6 @@ def load_library(path=LIB_PATH):
         "dq_quant_blocks": (None, [_u32p, C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_int, _u32p, _u32p]),
         "dq_colortable_indexes": (None, [_u32p, C.c_uint32, _u32p, C.c_int, _u32p, C.c_int]),
         "dq_colortable_indexes_device": (None, [vp, vp, C.c_uint32, _u32p, C.c_int, vp, C.c_int]),
-        "dq_shard_histogram": (C.c_uint32, [vp, vp, C.c_uint32, vp, vp]),
-        "dq_shard_quantize_map": (None, [vp, vp, vp, C.c_uint32, C.c_uint64, vp, C.c_uint32, vp, _u32p, _u32p]),
         "dq_rows_unique_id": (None, [vp]),
         "dq_rows_create": (vp, [vp, C.c_int, C.c_int, vp, C.c_uint32]),
         "dq_rows_destroy": (None, [vp]),
@@ -154,7 +152,7 @@ EXPORTED_C_SYMBOLS = [
     "dq_get_double_scale", "dq_validate_num_bits", "dq_set_display_timings", "dq_context_create", "dq_context_destroy",
     "dq_default_context", "dq_context_stream", "dq_context_synchronize", "dq_context_last_stats", "dq_context_set_profiling",
     "dq_quant_recurse_device", "dq_map_colors_device", "dq_quant_varpart_device", "dq_quant_recurse_ctx",
-    "dq_srm_num_pairs", "dq_srm_sorted_edges", "dq_srm_sorted_edges_device", "dq_context_set_split_ctas", "dq_context_set_exact_small", "dq_context_set_exact_max_points", "dq_context_set_tie_policy", "dq_pixel_histogram", "dq_block_vote", "dq_block_vote_device", "dq_quant_blocks", "dq_colortable_indexes", "dq_colortable_indexes_device", "dq_shard_histogram", "dq_shard_quantize_map", "dq_rows_unique_id", "dq_rows_create", "dq_rows_destroy", "dq_rows_quant_recurse", "dq_pipeline_create", "dq_pipeline_create_lanes", "dq_pipeline_destroy", "dq_pipeline_submit", "dq_pipeline_submit_device", "dq_pipeline_wait", "dq_pipeline_lanes", "dq_pipeline_set_blocking_wait", "dq_pipeline_flush", "dq_pipeline_last_elapsed_ms",
+    "dq_srm_num_pairs", "dq_srm_sorted_edges", "dq_srm_sorted_edges_device", "dq_context_set_split_ctas", "dq_context_set_exact_small", "dq_context_set_exact_max_points", "dq_context_set_tie_policy", "dq_pixel_histogram", "dq_block_vote", "dq_block_vote_device", "dq_quant_blocks", "dq_colortable_indexes", "dq_colortable_indexes_device", "dq_rows_unique_id", "dq_rows_create", "dq_rows_destroy", "dq_rows_quant_recurse", "dq_pipeline_create", "dq_pipeline_create_lanes", "dq_pipeline_destroy", "dq_pipeline_submit", "dq_pipeline_submit_device", "dq_pipeline_wait", "dq_pipeline_lanes", "dq_pipeline_set_blocking_wait", "dq_pipeline_flush", "dq_pipeline_last_elapsed_ms",
     "dq_pipeline_context", "dq_pipeline_kernel_launches", "dq_pipeline_flagged_frames",
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
     "dq_quant_recurse_batch_device", "dq_quant_recurse_batch_ctx", "dq_context_last_batch_stats",
@@ -464,48 +462,6 @@ def merge_histograms(colour_lists, count_lists):
     merged = np.zeros(uniq.size, np.uint64)
     np.add.at(merged, inv, counts)
     return uniq, merged
-
-
-def row_sharded_quant_recurse(lib, ctx, shard, total_pixels, k, dist=None, workspace=None):
-    """quant_recurse of ONE image whose pixel rows are spread over the ranks of `dist` (torch.distributed, NCCL).
-
-    shard: this rank's rows as a CUDA int32/uint32-viewed torch tensor (flat).  Returns (out_shard, palette).
-    One exchange on the data path: an all-gather of the per-shard (colour, count) lists (sizes first)."""
-    import torch
-
-    n = shard.numel()
-    dev = shard.device
-    ws = workspace if workspace is not None else {}
-    if ws.get("n") != n:  # reusable scratch (pass the same dict again to avoid per-call allocations)
-        ws["n"] = n
-        ws["colours"] = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
-        ws["counts"] = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
-        ws["out"] = torch.empty_like(shard)
-    colours, counts = ws["colours"], ws["counts"]
-    u = lib.dq_shard_histogram(ctx, shard.data_ptr(), n, colours.data_ptr(), counts.data_ptr())
-    if dist is not None and dist.get_world_size() > 1:
-        world = dist.get_world_size()
-        sizes = torch.zeros(world, dtype=torch.int64, device=dev)
-        dist.all_gather_into_tensor(sizes, torch.tensor([u], dtype=torch.int64, device=dev))
-        sizes_h = sizes.cpu().tolist()
-        cap = max(max(sizes_h), 1)
-        packed = torch.zeros(2, cap, dtype=torch.int32, device=dev)  # padding has count 0 and is skipped by the merge
-        packed[0, :u] = colours[:u]
-        packed[1, :u] = counts[:u]
-        gathered = torch.empty(world, 2, cap, dtype=torch.int32, device=dev)
-        dist.all_gather_into_tensor(gathered.view(-1), packed.view(-1))
-        all_colours = gathered[:, 0, :].contiguous().view(-1)
-        all_counts = gathered[:, 1, :].contiguous().view(-1)
-        entries = world * cap
-    else:
-        all_colours, all_counts, entries = colours, counts, u
-    torch.cuda.current_stream(dev).synchronize()
-    out = ws["out"]
-    ct = np.zeros(max(int(k), 1), np.uint32)
-    nk = C.c_uint32(k)
-    lib.dq_shard_quantize_map(ctx, all_colours.data_ptr(), all_counts.data_ptr(), entries, total_pixels, shard.data_ptr(), n,
-                              out.data_ptr(), C.byref(nk), _p(ct))
-    return out, ct[:nk.value].copy()
 
 
 class RowShards:

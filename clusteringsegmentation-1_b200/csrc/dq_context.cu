@@ -107,9 +107,6 @@ struct dq_context {
   DevBuf<uint2> d_flat;         // large tie resolver: the points by position
   DevBuf<uint32_t> d_sortvals;  // ... and the payload of its sort
   DevBuf<uint32_t> d_ovr;       // cuts taken from the resolver (SplitArgs::cut_overrides) of the call in flight
-  CutOverride h_ovr[kCutOverrideCap];
-  uint32_t n_ovr = 0;
-  bool ovr_active = false;
   DevBuf<uint64_t> d_keys;
   // sized by K
   DevBuf<SplitNode> d_nodes;
@@ -134,20 +131,24 @@ struct dq_context {
   struct PendingSplit {
     SplitArgs a;
     bool use_v2 = false, unaudited = false;
-    uint32_t K = 0;
   } pend;
-  // a quantize call between its two halves (quantize_begin / quantize_finish)
+  // A quantize call between its two halves (quantize_begin / quantize_finish): the one description of its split, from
+  // which every run of the split kernel takes its inputs and outputs (run_split).
   struct QuantState {
     uint32_t n = 0, rows = 0, cols = 0, K = 0, point_cap = 0;
     const uint32_t *d_in = nullptr;
     int num_bits = 8, dec = 1, max_iters = 10;
     double norm = 0.0;
+    // the points are a histogram (of the sampled pixels of d_in, or of the merged lists): weighted, collected by the split
+    // kernel's first pass, and a unique list of them stays in d_uniq for a table remap.  Otherwise they are in d_pts0.
     bool table_dirty = false;
     dq_split_record *records = nullptr;
     double *mean_out = nullptr;
     uint32_t *size_out = nullptr;
     int phase = 0;  // quantize_step
     uint32_t flags = 0, flags_all = 0, tie_count = 0, cut_count = 0, k_first = 0, resplits = 0;
+    CutOverride h_ovr[kCutOverrideCap];  // forced cuts of the next run (SplitRun::kForcedCuts)
+    uint32_t n_ovr = 0;
     // row-sharded call (dq_rows): the histogram and the first-seen indexes come from the gathered per-shard lists, not
     // from pixels, and there is no ordered re-run (that needs the whole image in order)
     struct Merged {
@@ -163,6 +164,7 @@ struct dq_context {
   long long spin_cycles = 0;  // DIVQUANT_B200_SPIN_MS: bound of the split kernel's waits on other CTAs (0 = built-in 0.2 s)
   int split_version = 2;  // 1 = generic kernel, 2 = latency-optimised kernel (falls back to 1 when it cannot run)
   int trace_split = 0;
+  int profile_narrow = 0;  // DQ_PROFILE_NARROW set: the cycle counters of a -DDQ_PROFILE_NARROW build to stderr after every split
   int *d_lut = nullptr;
   // pinned staging for the palette-sized transfers
   uint32_t *h_small = nullptr;
@@ -283,26 +285,20 @@ void reset_control(dq_context *ctx) {
   DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_cb, 0, sizeof(ControlBlock), ctx->stream));
 }
 
-// The sampled pixels behind a histogram: what split_exact_kernel needs to put a small input's unique colours
-// into calc_color_table's emission order.
-struct ExactSource {
-  const uint32_t *d_in;
-  uint32_t rows, cols, dec;
-  int bits;
-};
+// Which run of a quantize call's split: the first, the ordered re-run of a flagged frame (every input the ordered path
+// can hold goes there), or the re-run with the resolver's forced cuts (QuantState::h_ovr).
+enum class SplitRun { kFirst, kOrdered, kForcedCuts };
 
-int plan_ctas_hint(const dq_context *ctx, uint32_t K) { return split2_plan(ctx->split_ctas, ctx->sm_count, K, true).grid; }
-
-uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out, dq_split_record *records_out, double *mean_out,
-                          uint32_t *size_out);
-
-// Runs the divisive phase on ctx->d_pts0[0..U).  U is read on the device from d_cb->ucount.
-// Leaves palette/result/ctl in ctx->h_cb / ctx->h_small after a stream synchronisation.
-// Returns the number of palette entries.
-uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32_t K, int max_iters, int num_bits,
-                   uint32_t *colortable_out, dq_split_record *records_out, double *mean_out, uint32_t *size_out,
-                   bool collect_from_hist = false, const ExactSource *exact = nullptr, bool weighted = false,
-                   bool defer = false) {
+// Queues the divisive phase that ctx->qs describes, on its points: the histogram in the direct table and d_uniq
+// (q.table_dirty), or ctx->d_pts0[0..U).  U is read on the device from d_cb->ucount.  Nothing is waited for: the caller
+// polls split_ready() and collects the palette with run_split_finish().
+void run_split(dq_context *ctx, SplitRun run) {
+  const dq_context::QuantState &q = ctx->qs;
+  const uint32_t K = q.K, point_capacity = q.point_cap;
+  const int max_iters = q.max_iters;
+  // a histogram is collected by the split kernel and weighted; one of the pixels in q.d_in also gives the ordered path
+  // its input (a merged one has no pixels here)
+  const bool hist = q.table_dirty, pixels = hist && q.merged.colours == nullptr;
   if (max_iters < 1 || max_iters > kSplitMaxIters) {
     fprintf(stderr, "divquant_b200: max_iters ( %d ) must be in [1,%d] (the reference hard-wires local k-means on)\n",
             max_iters, kSplitMaxIters);
@@ -318,7 +314,7 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   ctx->d_palette.ensure(K);
   ctx->d_cluster_size.ensure(K);
   ctx->d_cluster_mean.ensure((size_t)3 * K);
-  if (records_out) ctx->d_records.ensure(K);
+  if (q.records) ctx->d_records.ensure(K);
 
   SplitArgs a;
   memset(&a, 0, sizeof(a));
@@ -328,8 +324,8 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   a.num_points_dev = &ctx->d_cb->ucount;
   a.num_colors = K;
   a.max_iters = max_iters;
-  a.shift = 8 - num_bits;
-  a.norm = norm;
+  a.shift = 8 - q.num_bits;
+  a.norm = q.norm;
   a.nodes = ctx->d_nodes.ptr;
   a.node_cap = node_cap;
   a.jobs = ctx->d_jobs.ptr;
@@ -343,7 +339,7 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   a.result = ctx->d_cb->result;
   a.cluster_mean = ctx->d_cluster_mean.ptr;
   a.cluster_size = ctx->d_cluster_size.ptr;
-  a.records = records_out ? ctx->d_records.ptr : nullptr;
+  a.records = q.records ? ctx->d_records.ptr : nullptr;
   if (ctx->trace_split) {
     ctx->d_timeline.ensure(8192);
     DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_timeline.ptr, 0, sizeof(unsigned long long), ctx->stream));
@@ -354,28 +350,29 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   const bool use_v2 = ctx->split_version == 2 && K <= kSplit2MaxColors;
   // weighted points on exact-integer sums: audit the decisions against the reference's rounding noise (dq_tie.cuh)
   a.spin_cycles = ctx->spin_cycles;
-  a.tie_audit = (weighted && use_v2 && ctx->tie_policy != 0) ? 1u : 0u;
+  a.tie_audit = (hist && use_v2 && ctx->tie_policy != 0) ? 1u : 0u;
   if (a.tie_audit) {
     ctx->d_tie.ensure(kTieListWords);
     a.tie_list = ctx->d_tie.ptr;
-    if (ctx->ovr_active && ctx->n_ovr) {  // (only the re-split of quantize_step: other callers never inherit a frame's cuts)
+    if (run == SplitRun::kForcedCuts) {
       a.cut_overrides = reinterpret_cast<const CutOverride *>(ctx->d_ovr.ptr);
-      a.num_cut_overrides = ctx->n_ovr;
+      a.num_cut_overrides = q.n_ovr;
     }
   }
   ctx->mark(2);
-  const bool exact_path = exact != nullptr && collect_from_hist && K <= kExactMaxColors && ctx->exact_small && ctx->exact_max_points > 0;
+  const uint32_t max_points = run == SplitRun::kOrdered ? kExactMaxPoints : ctx->exact_max_points;
+  const bool exact_path = pixels && K <= kExactMaxColors && ctx->exact_small && max_points > 0;
   ExactSampling sampling;
   memset(&sampling, 0, sizeof(sampling));
   if (exact_path) {
     // small inputs: the reference's own summation order (dq_split_exact.cuh); large ones take one branch
     ctx->d_ctl_f64.ensure((size_t)8 * K + node_cap + 16);
     a.g_cluster_tse = ctx->d_ctl_f64.ptr;
-    a.exact_small_max = std::min<uint32_t>(ctx->exact_max_points, kExactMaxPoints);
+    a.exact_small_max = std::min<uint32_t>(max_points, kExactMaxPoints);
     // the generic kernel (K > kSplit2MaxColors) carries no tie audit: everything the ordered path can hold goes there
-    if (weighted && !use_v2 && ctx->tie_policy != 0) a.exact_small_max = kExactMaxPoints;
+    if (!use_v2 && ctx->tie_policy != 0) a.exact_small_max = kExactMaxPoints;
     ctx->d_exact.ensure((split_exact_scratch_bytes() + ((size_t)8 * K + 16 + 64) * sizeof(uint32_t)) / 8 + 2);
-    sampling = exact_sampling(exact->d_in, exact->rows, exact->cols, exact->dec, exact->bits);
+    sampling = exact_sampling(q.d_in, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
   }
   if (use_v2) {
     Split2Extra x;
@@ -390,11 +387,11 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
     x.cursors = ctx->d_cursors.ptr;
     ctx->d_progress.ensure(1024);
     x.progress = ctx->d_progress.ptr;
-    x.collect_uniq = collect_from_hist ? ctx->d_uniq.ptr : nullptr;
-    x.collect_table = collect_from_hist ? ctx->d_table : nullptr;
-    if (getenv("DQ_PROFILE_NARROW")) DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_progress.ptr, 0, 1024 * sizeof(uint32_t), ctx->stream));
-    const bool mail = ctx->use_mailbox && !ctx->blocking_wait && !ctx->trace_split && records_out == nullptr &&
-                      mean_out == nullptr && size_out == nullptr;
+    x.collect_uniq = hist ? ctx->d_uniq.ptr : nullptr;
+    x.collect_table = hist ? ctx->d_table : nullptr;
+    if (ctx->profile_narrow) DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_progress.ptr, 0, 1024 * sizeof(uint32_t), ctx->stream));
+    const bool mail = ctx->use_mailbox && !ctx->blocking_wait && !ctx->trace_split && q.records == nullptr &&
+                      q.mean_out == nullptr && q.size_out == nullptr;
     if (mail) {
       void *dev = nullptr;
       DQ_CUDA_CHECK(cudaHostGetDevicePointer(&dev, const_cast<uint32_t *>(ctx->mailbox), 0));
@@ -402,25 +399,23 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
       a.mailbox_seq = ++ctx->mailbox_seq;
       if (a.mailbox_seq == 0) a.mailbox_seq = ++ctx->mailbox_seq;  // 0 is the idle value
     }
-    const bool fuse = exact_path && split2_plan(0, ctx->sm_count, K, true).smem_bytes >= split_exact_smem_bytes();
-    if (fuse) {
-      x.exact_fused = (ctx->exact_parallel && plan_ctas_hint(ctx, K) > 1) ? 2 : 1;
+    // the ordered path always runs inside this kernel: its plan makes room for it in the dynamic shared memory
+    const SplitLaunch plan = split2_plan(ctx->split_ctas, ctx->sm_count, K, exact_path);
+    if (exact_path) {
+      x.exact_fused = (ctx->exact_parallel && plan.grid > 1) ? 2 : 1;
       x.exact_src = sampling;
       x.exact_first_seen = ctx->d_map;
       x.exact_scratch = reinterpret_cast<unsigned char *>(ctx->d_exact.ptr);
       x.exact_f64 = ctx->d_ctl_f64.ptr;
       x.exact_i32 = ctx->d_ctl_i32.ptr;
-    } else if (exact_path) {
-      split_exact_launch(a, sampling, reinterpret_cast<unsigned char *>(ctx->d_exact.ptr), ctx->d_uniq.ptr, ctx->d_table, ctx->d_map, ctx->d_ctl_f64.ptr, ctx->d_ctl_i32.ptr, ctx->stream);
-      ctx->stats.kernel_launches += 2;
     }
-    split2_launch(a, x, split2_plan(ctx->split_ctas, ctx->sm_count, K, fuse), ctx->stream);
+    split2_launch(a, x, plan, ctx->stream);
   } else {
     if (exact_path) {
       split_exact_launch(a, sampling, reinterpret_cast<unsigned char *>(ctx->d_exact.ptr), ctx->d_uniq.ptr, ctx->d_table, ctx->d_map, ctx->d_ctl_f64.ptr, ctx->d_ctl_i32.ptr, ctx->stream);
       ctx->stats.kernel_launches += 2;
     }
-    if (collect_from_hist) {  // the generic kernel has no fused collect
+    if (hist) {  // the generic kernel has no fused collect
       hist_collect(ctx->d_uniq.ptr, &ctx->d_cb->ucount, point_capacity, ctx->d_table, ctx->d_pts0.ptr, true, ctx->sm_count, ctx->stream);
       ctx->stats.kernel_launches++;
     }
@@ -430,10 +425,7 @@ uint32_t run_split(dq_context *ctx, uint32_t point_capacity, double norm, uint32
   ctx->stats.kernel_launches++;
   ctx->pend.a = a;
   ctx->pend.use_v2 = use_v2;
-  ctx->pend.K = K;
-  ctx->pend.unaudited = weighted && !a.tie_audit && ctx->tie_policy != 0;
-  if (defer) return 0;  // the caller polls split_ready() and collects with run_split_finish()
-  return run_split_finish(ctx, colortable_out, records_out, mean_out, size_out);
+  ctx->pend.unaudited = hist && !a.tie_audit && ctx->tie_policy != 0;
 }
 
 // Has the split launched last on this context delivered its palette?  (non-blocking; true when there is nothing to poll)
@@ -444,11 +436,13 @@ bool split_ready(dq_context *ctx) {
   return cudaStreamQuery(ctx->stream) != cudaErrorNotReady;  // an error exit leaves the stream idle without the number
 }
 
-uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out, dq_split_record *records_out, double *mean_out,
-                          uint32_t *size_out) {
+// Collects the palette of the split launched last into colortable_out, and the records / means / sizes ctx->qs asks for.
+// Returns the number of palette entries.
+uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out) {
+  const dq_context::QuantState &q = ctx->qs;
   const SplitArgs &a = ctx->pend.a;
   const bool use_v2 = ctx->pend.use_v2;
-  const uint32_t K = ctx->pend.K;
+  const uint32_t K = q.K;
   ctx->ensure_small((size_t)K + 16);
   bool mailed = false;
   if (a.mailbox != nullptr) {
@@ -492,7 +486,7 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out, dq_split_re
     }
     abort();
   }
-  if (use_v2 && getenv("DQ_PROFILE_NARROW")) {
+  if (use_v2 && ctx->profile_narrow) {
     uint32_t prof[8];
     cudaMemcpy(prof, ctx->d_progress.ptr + 756, sizeof(prof), cudaMemcpyDeviceToHost);
     uint32_t wp[9];
@@ -517,10 +511,10 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out, dq_split_re
   ctx->stats.tie_flags = a.tie_audit ? ctx->h_cb->ctl[kCtlTie] : 0u;
   // exact-integer sums without an audit (the generic kernel beyond the ordered path's reach): say so
   if (ctx->pend.unaudited && ctx->h_cb->ucount > a.exact_small_max) ctx->stats.tie_flags |= (uint32_t)kTieUnaudited;
-  if (records_out && K > 1)
-    DQ_CUDA_CHECK(cudaMemcpy(records_out, ctx->d_records.ptr, (size_t)(K - 1) * sizeof(SplitRecord), cudaMemcpyDeviceToHost));
-  if (mean_out) DQ_CUDA_CHECK(cudaMemcpy(mean_out, ctx->d_cluster_mean.ptr, (size_t)3 * K * sizeof(double), cudaMemcpyDeviceToHost));
-  if (size_out) DQ_CUDA_CHECK(cudaMemcpy(size_out, ctx->d_cluster_size.ptr, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  if (q.records && K > 1)
+    DQ_CUDA_CHECK(cudaMemcpy(q.records, ctx->d_records.ptr, (size_t)(K - 1) * sizeof(SplitRecord), cudaMemcpyDeviceToHost));
+  if (q.mean_out) DQ_CUDA_CHECK(cudaMemcpy(q.mean_out, ctx->d_cluster_mean.ptr, (size_t)3 * K * sizeof(double), cudaMemcpyDeviceToHost));
+  if (q.size_out) DQ_CUDA_CHECK(cudaMemcpy(q.size_out, ctx->d_cluster_size.ptr, (size_t)K * sizeof(uint32_t), cudaMemcpyDeviceToHost));
   return actual;
 }
 
@@ -600,54 +594,6 @@ void check_quant_args(uint32_t n, uint32_t k, int num_bits) {
   }
 }
 
-// quant_varpart_fast on device-resident pixels; keeps the unique list (when one was built) valid for
-// a following table remap.  Returns true if such a unique list exists (d_uniq / d_cb->ucount).
-// First half: histogram (or points) and the split kernel are queued; nothing is waited for.
-void quantize_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t rows, uint32_t cols, uint32_t K, int num_bits,
-                    int dec, int max_iters, int all_unique, dq_split_record *records, double *mean_out, uint32_t *size_out) {
-  check_quant_args(n, K, num_bits);
-  reset_control(ctx);
-  ctx->mark(0);
-  bool table_dirty = false;
-  double norm;
-  uint32_t point_cap;
-  if (all_unique && num_bits == 8 && dec == 1) {
-    // uniform weight: every pixel is a point (DivQuantCluster.cpp:1130-1132)
-    ctx->d_pts0.ensure(n);
-    ctx->mark(1);
-    points_from_pixels(d_in, n, ctx->d_pts0.ptr, ctx->sm_count, ctx->stream);
-    ctx->stats.kernel_launches++;
-    ctx->h_cb->ucount = n;
-    DQ_CUDA_CHECK(cudaMemcpyAsync(&ctx->d_cb->ucount, &ctx->h_cb->ucount, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    norm = sample_norm(1, n, 1);
-    point_cap = n;
-  } else {
-    if (dec <= 0) {
-      fprintf(stderr, "Decimation factor ( %d ) should be positive !\n", dec);
-      abort();  // the reference dereferences the NULL it gets back (:1136); fail loudly instead
-    }
-    const uint32_t samples = ((rows + dec - 1) / dec) * ((cols + dec - 1) / dec);
-    ctx->d_pts0.ensure(samples);
-    run_histogram(ctx, d_in, n, rows, cols, (uint32_t)dec, num_bits);
-    ctx->mark(1);
-    table_dirty = true;  // (= a unique list exists; the split kernel's first pass turns it into points and zeroes the counters)
-    norm = sample_norm(rows, cols, dec);
-    point_cap = samples;
-  }
-  const ExactSource src = {d_in, rows, cols, (uint32_t)dec, num_bits};
-  uint32_t unused = 0;
-  run_split(ctx, point_cap, norm, K, max_iters, num_bits, &unused, records, mean_out, size_out, table_dirty,
-            table_dirty ? &src : nullptr, table_dirty, /*defer=*/true);
-  dq_context::QuantState &q = ctx->qs;
-  q.n = n, q.rows = rows, q.cols = cols, q.K = K, q.point_cap = point_cap, q.d_in = d_in;
-  q.num_bits = num_bits, q.dec = dec, q.max_iters = max_iters, q.norm = norm, q.table_dirty = table_dirty;
-  q.records = records, q.mean_out = mean_out, q.size_out = size_out;
-  q.phase = 0;
-  q.flags = q.flags_all = q.tie_count = q.cut_count = q.k_first = q.resplits = 0;
-  q.merged = dq_context::QuantState::Merged();
-  ctx->n_ovr = 0;
-}
-
 // The merged histogram of a row-sharded image in the direct table, and the whole image's first-seen index of every colour
 // in d_map (what the resolver reads); leaves U in d_cb->ucount.
 void run_merge(dq_context *ctx, const dq_context::QuantState::Merged &m) {
@@ -655,6 +601,61 @@ void run_merge(dq_context *ctx, const dq_context::QuantState::Merged &m) {
              ctx->d_map);
   hist_merge_first(m.colours, m.counts, m.first, m.cap, m.world, ctx->d_map, ctx->sm_count, ctx->stream);
   ctx->stats.kernel_launches += 2;
+}
+
+// Control block cleared and the histogram of ctx->qs's source built again: the sampled pixels of q.d_in or, in a
+// row-sharded call (whose other shards' pixels are not here), the gathered lists.  Leaves U in d_cb->ucount.
+void rebuild_histogram(dq_context *ctx) {
+  const dq_context::QuantState &q = ctx->qs;
+  reset_control(ctx);
+  if (q.merged.colours != nullptr) run_merge(ctx, q.merged);
+  else run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
+}
+
+// Queues the first run of the quantize call that the caller has described in ctx->qs: the points (the histogram of its
+// source, or one per pixel of q.d_in), then the split.  Nothing is waited for.
+void quantize_launch(dq_context *ctx) {
+  const dq_context::QuantState &q = ctx->qs;
+  ctx->mark(0);
+  ctx->d_pts0.ensure(q.point_cap);
+  if (q.table_dirty) {
+    rebuild_histogram(ctx);
+    ctx->mark(1);
+  } else {
+    reset_control(ctx);
+    ctx->mark(1);
+    points_from_pixels(q.d_in, q.n, ctx->d_pts0.ptr, ctx->sm_count, ctx->stream);
+    ctx->stats.kernel_launches++;
+    ctx->h_cb->ucount = q.n;
+    DQ_CUDA_CHECK(cudaMemcpyAsync(&ctx->d_cb->ucount, &ctx->h_cb->ucount, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  }
+  run_split(ctx, SplitRun::kFirst);
+}
+
+// quant_varpart_fast on device-resident pixels.  First half: histogram (or points) and the split kernel are queued;
+// nothing is waited for.
+void quantize_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t rows, uint32_t cols, uint32_t K, int num_bits,
+                    int dec, int max_iters, int all_unique, dq_split_record *records, double *mean_out, uint32_t *size_out) {
+  check_quant_args(n, K, num_bits);
+  dq_context::QuantState &q = ctx->qs;
+  q = dq_context::QuantState();
+  q.n = n, q.rows = rows, q.cols = cols, q.K = K, q.d_in = d_in;
+  q.num_bits = num_bits, q.dec = dec, q.max_iters = max_iters;
+  q.records = records, q.mean_out = mean_out, q.size_out = size_out;
+  if (all_unique && num_bits == 8 && dec == 1) {
+    // uniform weight: every pixel is a point (DivQuantCluster.cpp:1130-1132)
+    q.point_cap = n;
+    q.norm = sample_norm(1, n, 1);
+  } else {
+    if (dec <= 0) {
+      fprintf(stderr, "Decimation factor ( %d ) should be positive !\n", dec);
+      abort();  // the reference dereferences the NULL it gets back (:1136); fail loudly instead
+    }
+    q.point_cap = ((rows + dec - 1) / dec) * ((cols + dec - 1) / dec);
+    q.norm = sample_norm(rows, cols, dec);
+    q.table_dirty = true;
+  }
+  quantize_launch(ctx);
 }
 
 // Second half, as a small state machine so that a host thread that drives several contexts never has to wait inside it:
@@ -694,18 +695,12 @@ bool quantize_pending_ready(dq_context *ctx) {
 QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colortable) {
   dq_context::QuantState &q = ctx->qs;
   const uint32_t K = q.K;
-  const ExactSource src = {q.d_in, q.rows, q.cols, (uint32_t)q.dec, q.num_bits};
   auto queue_rerun = [&]() {
     // Some decision of the exact-integer split sits inside the rounding noise of the reference's sequential sums:
     // the reference's own summation order decides.  The count table is all-zero again (the split kernel zeroed what
     // it collected), so the frame simply goes through the histogram and the split once more, on the ordered path.
-    const uint32_t keep = ctx->exact_max_points;
-    ctx->exact_max_points = kExactMaxPoints;
-    reset_control(ctx);
-    run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
-    uint32_t unused = 0;
-    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true, &src, true, /*defer=*/true);
-    ctx->exact_max_points = keep;
+    rebuild_histogram(ctx);
+    run_split(ctx, SplitRun::kOrdered);
     q.phase = 2;
   };
   auto queue_resplit = [&]() {
@@ -713,16 +708,9 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     // what the reference's mean is): the exact-integer split runs again with that node cut where the reference cuts it
     // (SplitArgs::cut_overrides).  Everything outside the node's subtree comes out as before.
     ctx->d_ovr.ensure(kCutOverrideCap * sizeof(CutOverride) / sizeof(uint32_t));
-    DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_ovr.ptr, ctx->h_ovr, ctx->n_ovr * sizeof(CutOverride), cudaMemcpyHostToDevice, ctx->stream));
-    reset_control(ctx);
-    const bool merged = q.merged.colours != nullptr;
-    if (merged) run_merge(ctx, q.merged);  // (the shards' pixels are not here: merge the gathered lists again)
-    else run_histogram(ctx, q.d_in, q.n, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
-    uint32_t unused = 0;
-    ctx->ovr_active = true;
-    run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &unused, q.records, q.mean_out, q.size_out, true,
-              merged ? nullptr : &src, true, /*defer=*/true);
-    ctx->ovr_active = false;
+    DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_ovr.ptr, q.h_ovr, q.n_ovr * sizeof(CutOverride), cudaMemcpyHostToDevice, ctx->stream));
+    rebuild_histogram(ctx);
+    run_split(ctx, SplitRun::kForcedCuts);
     q.resplits++;
     q.phase = 0;
   };
@@ -756,11 +744,11 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
   const bool can_rerun = ctx->tie_policy == 2 && q.table_dirty && ctx->exact_small && K <= kExactMaxColors && K <= kSplit2MaxColors &&
                          ctx->split_version == 2 && q.merged.colours == nullptr;
   if (q.phase == 0) {
-    *k_inout = run_split_finish(ctx, colortable, q.records, q.mean_out, q.size_out);
+    *k_inout = run_split_finish(ctx, colortable);
     q.flags = ctx->stats.tie_flags;
     q.flags_all |= q.flags;
     ctx->stats.tie_flags = q.flags_all;  // (a frame that needed forced cuts stays marked as flagged)
-    ctx->stats.cut_overrides = ctx->n_ovr;
+    ctx->stats.cut_overrides = q.n_ovr;
     if (q.flags == 0u) return kQuantDone;
     if ((q.flags & ~(uint32_t)(kTieRound | kTieCut)) == 0u && ctx->tie_policy == 2 && q.table_dirty && ctx->exact_small &&
         q.records == nullptr && q.mean_out == nullptr) {
@@ -826,7 +814,7 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
       CutOverride rec[kTieListCap];  // (copied out: K odd leaves the doubles inside h_small unaligned)
       memcpy(rec, ctx->h_small + K + 2 * kTieListCap, q.cut_count * sizeof(CutOverride));
       const uint32_t *st = ctx->h_small + K + q.tie_count;
-      const uint32_t added = select_cut_overrides(rec, st, q.cut_count, ctx->h_ovr, &ctx->n_ovr, kCutOverrideCap);
+      const uint32_t added = select_cut_overrides(rec, st, q.cut_count, q.h_ovr, &q.n_ovr, kCutOverrideCap);
       if (added) {
         queue_resplit();
         return kQuantPending;
@@ -844,7 +832,7 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
   }
   // phase 2
   const uint32_t launches = ctx->stats.kernel_launches;
-  *k_inout = run_split_finish(ctx, colortable, q.records, q.mean_out, q.size_out);
+  *k_inout = run_split_finish(ctx, colortable);
   ctx->stats.kernel_launches = launches;
   ctx->stats.tie_flags = q.flags;
   ctx->stats.ordered_rerun = 1;
@@ -873,23 +861,15 @@ void recurse_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t K
   quantize_begin(ctx, n, d_in, 1, n, K, 8, 1, 10, all_unique, nullptr, nullptr, nullptr);
 }
 
-void recurse_remap_tail(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable);
-
-void recurse_remap(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable,
-                   std::chrono::steady_clock::time_point *t_palette = nullptr) {
-  quantize_finish(ctx, k_inout, colortable);
-  if (t_palette) *t_palette = std::chrono::steady_clock::now();
-  recurse_remap_tail(ctx, n, d_in, d_out, k_inout, colortable);
-}
-
-// The palette is final: the reference's host handling of it and the remap kernels (queued, not waited for).
-void recurse_remap_tail(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable) {
-  const bool dirty = ctx->qs.table_dirty;
+// The palette is final: the reference's host handling of it and the remap of d_in's n pixels (queued, not waited for).
+// through_table: the unique list of the quantize (d_uniq / d_cb->ucount, mapped through d_map) holds every colour of d_in.
+void remap_quantized(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable,
+                     bool through_table) {
   uint32_t k = dedup_palette(colortable, *k_inout);
   *k_inout = k;
   ctx->stats.actual_colors = k;
+  if (n == 0) return;  // (a row shard without rows)
   const uint32_t U = ctx->stats.num_points;
-  const bool through_table = dirty && (uint64_t)U * 2 <= n;
   if (through_table && k <= 256) {
     // the tables ride in the kernel's parameter block: no upload
     MapTablesParam tables;
@@ -911,6 +891,19 @@ void recurse_remap_tail(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint3
     upload_search_tables(ctx, colortable, (int)k);
     remap_bruteforce(ctx, d_in, n, d_out, (int)k);
   }
+}
+
+// quant_recurse's remap: through the table when there are at most half as many unique colours as pixels.
+void recurse_remap_tail(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable) {
+  const bool through_table = ctx->qs.table_dirty && (uint64_t)ctx->stats.num_points * 2 <= n;
+  remap_quantized(ctx, n, d_in, d_out, k_inout, colortable, through_table);
+}
+
+void recurse_remap(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout, uint32_t *colortable,
+                   std::chrono::steady_clock::time_point *t_palette = nullptr) {
+  quantize_finish(ctx, k_inout, colortable);
+  if (t_palette) *t_palette = std::chrono::steady_clock::now();
+  recurse_remap_tail(ctx, n, d_in, d_out, k_inout, colortable);
 }
 
 void quant_recurse_device_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t *d_out, uint32_t *k_inout,
@@ -1259,6 +1252,7 @@ dq_context *dq_context_create(int device) {
   if (const char *e = getenv("DIVQUANT_B200_EXACT_SMALL")) ctx->exact_small = (e[0] != '0');
   if (const char *e = getenv("DIVQUANT_B200_EXACT_PARALLEL")) ctx->exact_parallel = (e[0] != '0');
   if (const char *e = getenv("DIVQUANT_B200_EXACT_MAX")) ctx->exact_max_points = (uint32_t)std::min<long>(std::max<long>(atol(e), 0), kExactMaxPoints);
+  ctx->profile_narrow = getenv("DQ_PROFILE_NARROW") != nullptr;
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
   return ctx;
 }
@@ -1725,53 +1719,6 @@ void dq_colortable_indexes(const uint32_t *quantPixels, uint32_t numPixels, cons
   DQ_CUDA_CHECK(cudaMemcpy(labelsOut, ctx->d_out.ptr, (size_t)numPixels * sizeof(uint32_t), cudaMemcpyDeviceToHost));
 }
 
-// ---- pixel-row sharding of one image ----
-
-uint32_t dq_shard_histogram(dq_context *ctx, const uint32_t *d_shard, uint32_t n_shard, uint32_t *d_colours, uint32_t *d_counts) {
-  require_device(ctx);
-  memset(&ctx->stats, 0, sizeof(ctx->stats));
-  ctx->stats.num_pixels = n_shard;
-  if (n_shard == 0) return 0;
-  reset_control(ctx);
-  ctx->d_pts0.ensure(n_shard);
-  run_histogram(ctx, d_shard, n_shard, 1, n_shard, 1, 8);
-  hist_collect(ctx->d_uniq.ptr, &ctx->d_cb->ucount, n_shard, ctx->d_table, ctx->d_pts0.ptr, true, ctx->sm_count, ctx->stream);
-  hist_export(ctx->d_pts0.ptr, &ctx->d_cb->ucount, n_shard, d_colours, d_counts, ctx->sm_count, ctx->stream);
-  ctx->stats.kernel_launches += 2;
-  DQ_CUDA_CHECK(cudaMemcpyAsync(&ctx->h_cb->ucount, &ctx->d_cb->ucount, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-  ctx->stats.num_points = ctx->h_cb->ucount;
-  return ctx->h_cb->ucount;
-}
-
-void dq_shard_quantize_map(dq_context *ctx, const uint32_t *d_all_colours, const uint32_t *d_all_counts, uint32_t num_entries,
-                           uint64_t total_pixels, const uint32_t *d_shard, uint32_t n_shard, uint32_t *d_out_shard,
-                           uint32_t *numClustersPtr, uint32_t *outColortablePtr) {
-  require_device(ctx);
-  memset(&ctx->stats, 0, sizeof(ctx->stats));
-  ctx->stats.num_pixels = n_shard;
-  const uint32_t K = *numClustersPtr;
-  if (total_pixels == 0 || total_pixels > 0x7fffffffull || K == 0 || num_entries == 0) {
-    fprintf(stderr, "divquant_b200: row-sharded call needs 0 < total_pixels < 2^31, K > 0 and a non-empty histogram\n");
-    abort();
-  }
-  reset_control(ctx);
-  // merged histogram: at most min(num_entries, 2^24) unique colours
-  ctx->d_uniq.ensure(num_entries);
-  ctx->d_pts0.ensure(num_entries);
-  hist_merge(d_all_colours, d_all_counts, num_entries, ctx->d_table, ctx->d_uniq.ptr, &ctx->d_cb->ucount, ctx->sm_count, ctx->stream);
-  ctx->stats.kernel_launches += 1;
-  const double norm = sample_norm(1, (uint32_t)total_pixels, 1);  // 1 / N of the WHOLE image (:172)
-  uint32_t k = run_split(ctx, num_entries, norm, K, 10, 8, outColortablePtr, nullptr, nullptr, nullptr, true, nullptr, true);
-  k = dedup_palette(outColortablePtr, k);
-  *numClustersPtr = k;
-  ctx->stats.actual_colors = k;
-  upload_search_tables(ctx, outColortablePtr, (int)k);
-  // every colour of this rank's rows is in the merged list, so the table path serves the shard
-  if (n_shard) remap_through_table(ctx, d_shard, n_shard, d_out_shard, (int)k, ctx->stats.num_points);
-  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-}
-
 // ---- frame pipeline ----
 
 }  // extern "C"
@@ -2071,6 +2018,12 @@ uint32_t dq_debug_split_points(dq_context *ctx, const uint32_t *colours, const u
   require_device(ctx);
   memset(&ctx->stats, 0, sizeof(ctx->stats));
   static_assert(sizeof(dq_split_record) == sizeof(SplitRecord), "record layouts must match");
+  // host points, no histogram: unweighted (no tie audit), and with records requested no mailbox
+  dq_context::QuantState &q = ctx->qs;
+  q = dq_context::QuantState();
+  q.n = num_points, q.K = num_colors, q.point_cap = num_points;
+  q.num_bits = num_bits, q.max_iters = max_iters, q.norm = norm;
+  q.records = records, q.mean_out = cluster_mean, q.size_out = cluster_size;
   std::vector<uint2> pts(num_points);
   for (uint32_t i = 0; i < num_points; ++i) pts[i] = make_uint2(colours[i] & 0x00FFFFFFu, counts ? counts[i] : 1u);
   ctx->d_pts0.ensure(num_points);
@@ -2079,8 +2032,8 @@ uint32_t dq_debug_split_points(dq_context *ctx, const uint32_t *colours, const u
   ctx->h_cb->ucount = num_points;
   DQ_CUDA_CHECK(cudaMemcpyAsync(&ctx->d_cb->ucount, &ctx->h_cb->ucount, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
-  return run_split(ctx, num_points, norm, num_colors, max_iters, num_bits, colortable,
-                   reinterpret_cast<dq_split_record *>(records), cluster_mean, cluster_size);
+  run_split(ctx, SplitRun::kFirst);
+  return run_split_finish(ctx, colortable);
 }
 
 uint32_t dq_debug_histogram(dq_context *ctx, const uint32_t *inPixels, uint32_t numPixels, uint32_t *colours, uint32_t *counts) {
@@ -2299,31 +2252,12 @@ void dq_rows_quant_recurse(dq_rows *r, const uint32_t *d_shard, uint32_t n_shard
   q.n = (uint32_t)total_pixels, q.rows = 1, q.cols = (uint32_t)total_pixels, q.K = K, q.point_cap = (uint32_t)entries;
   q.norm = sample_norm(1, (uint32_t)total_pixels, 1);  // 1 / N of the WHOLE image (:172)
   q.table_dirty = true;
-  ctx->n_ovr = 0;
-  reset_control(ctx);
-  run_merge(ctx, q.merged);
-  uint32_t k = 0;
-  run_split(ctx, q.point_cap, q.norm, K, q.max_iters, q.num_bits, &k, nullptr, nullptr, nullptr, true, nullptr, true, /*defer=*/true);
-  k = K;
+  quantize_launch(ctx);
+  uint32_t k = K;
   quantize_finish(ctx, &k, outColortablePtr);
-  k = dedup_palette(outColortablePtr, k);
+  // every colour of this rank's rows is in the merged list, so the table path serves the shard
+  remap_quantized(ctx, n_shard, d_shard, d_out_shard, &k, outColortablePtr, true);
   *numClustersPtr = k;
-  ctx->stats.actual_colors = k;
-  if (n_shard) {
-    if (k <= 256) {
-      MapTablesParam tables;
-      int lut[kLutEntries];
-      build_search_tables(outColortablePtr, (int)k, tables.sorted, lut);
-      for (int i = 0; i < kLutEntries; ++i) tables.lut[i] = (uint16_t)lut[i];
-      map_unique_params(tables, ctx->d_uniq.ptr, &ctx->d_cb->ucount, ctx->stats.num_points, ctx->d_map, (int)k, ctx->sm_count, ctx->stream);
-      map_gather(d_shard, n_shard, d_out_shard, ctx->d_map, ctx->sm_count, ctx->stream);
-      ctx->stats.kernel_launches += 2;
-      ctx->stats.remap_path = 2;
-    } else {
-      upload_search_tables(ctx, outColortablePtr, (int)k);
-      remap_through_table(ctx, d_shard, n_shard, d_out_shard, (int)k, ctx->stats.num_points);
-    }
-  }
   uint32_t overflow = 0;
   DQ_CUDA_CHECK(cudaMemcpyAsync(&overflow, r->d_overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));

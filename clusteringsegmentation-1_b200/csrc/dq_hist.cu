@@ -188,17 +188,6 @@ __global__ void __launch_bounds__(256) order_emit_kernel(const uint2 *__restrict
   }
 }
 
-// (colour, count) points -> two plain arrays (the exchange format of the row-sharded path)
-__global__ void __launch_bounds__(256) hist_export_kernel(const uint2 *__restrict__ pts, const uint32_t *ucount,
-                                                         uint32_t *colours, uint32_t *counts) {
-  const uint32_t u = *ucount;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < u; i += gridDim.x * blockDim.x) {
-    const uint2 p = pts[i];
-    colours[i] = p.x;
-    counts[i] = p.y;
-  }
-}
-
 // Same into a fixed-capacity slice of the exchange buffers: entries beyond the shard's U get count 0 (the merge skips
 // them), a shard with more than `cap` colours raises *overflow (the caller sized the exchange too small).
 // With `first` (cap + 1 words): first[i] = the shard-local first-seen index of colour i (read from first_table), and
@@ -342,12 +331,6 @@ void order_sort_emit(const uint2 *d_pts, uint32_t u, uint64_t *d_keys, uint32_t 
   if (u == 0) return;
   order_sort(d_keys, d_vals, u, sm_count, st);
   order_emit_kernel<<<blocks_for(u, 256, sm_count, 8), 256, 0, st>>>(d_pts, d_vals, u, norm, d_colours, d_weights);
-  DQ_CUDA_CHECK(cudaGetLastError());
-}
-
-void hist_export(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_colours, uint32_t *d_counts,
-                 int sm_count, cudaStream_t st) {
-  hist_export_kernel<<<blocks_for(u_hint, 256, sm_count, 8), 256, 0, st>>>(d_pts, d_ucount, d_colours, d_counts);
   DQ_CUDA_CHECK(cudaGetLastError());
 }
 

@@ -24,8 +24,6 @@ void order_keys(const uint32_t *d_in, uint32_t num_rows, uint32_t num_cols, uint
 void order_sort(uint64_t *d_keys, uint32_t *d_vals, uint32_t u, int sm_count, cudaStream_t st);
 void order_sort_emit(const uint2 *d_pts, uint32_t u, uint64_t *d_keys, uint32_t *d_vals, double norm, uint32_t *d_colours,
                      double *d_weights, int sm_count, cudaStream_t st);
-void hist_export(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t u_hint, uint32_t *d_colours, uint32_t *d_counts,
-                 int sm_count, cudaStream_t st);
 // d_first (optional, cap + 1 words): the shard-local first-seen index of every exported colour (from d_first_table), then
 // n_shard
 void hist_export_padded(const uint2 *d_pts, const uint32_t *d_ucount, uint32_t cap, uint32_t *d_colours, uint32_t *d_counts,

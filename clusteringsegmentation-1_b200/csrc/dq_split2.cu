@@ -33,10 +33,7 @@
 namespace dq {
 namespace {
 
-#ifndef DQ_SPLIT_WARPS
-#define DQ_SPLIT_WARPS 16
-#endif
-constexpr int kWarps = DQ_SPLIT_WARPS;
+constexpr int kWarps = 16;
 constexpr int T = 32 * kWarps;  // 16 warps, up to 128 registers per thread: points stay in registers without spills
 constexpr uint32_t kWideTile = 1024;  // points per wide tile
 constexpr int kWidePPT = 2;           // points per thread when a CTA classifies its share of a wide job
@@ -1675,7 +1672,7 @@ SplitLaunch split2_plan(int requested_ctas, int sm_count, uint32_t num_colors, b
   plan.grid = (requested_ctas >= 1 && requested_ctas <= cap) ? requested_ctas : cap;
   plan.smem_bytes = split2_smem_bytes(num_colors, 8 * num_colors + 16);
   // the small-input body lives in the same dynamic shared memory (one CTA per SM either way: 128 registers x 512)
-  if (exact_fused && kWarps == 16) plan.smem_bytes = std::max(plan.smem_bytes, split_exact_smem_bytes());
+  if (exact_fused) plan.smem_bytes = std::max(plan.smem_bytes, split_exact_smem_bytes());
   return plan;
 }
 

@@ -222,29 +222,11 @@ void dq_colortable_indexes_device(dq_context *ctx, const uint32_t *d_quantPixels
 /* ------------------------------------------------------------------------------------------------
  * 2a. Pixel-row sharding of ONE image over several GPUs (BASELINE.json config 3; one process per GPU).
  *     Counts are additive over shards and every sum of the divisive phase is an exact integer, so the
- *     palette is independent of the number of shards.  The library does the per-device work; the caller
- *     owns the one exchange (an all-gather of the per-shard (colour, count) lists, e.g. NCCL through
- *     torch.distributed):
- *       1. U_r = dq_shard_histogram(ctx, d_shard, n_r, d_colours_r, d_counts_r)        on every rank r
- *       2. all-gather the lists -> d_all_colours / d_all_counts (M = sum of U_r entries)
- *       3. dq_shard_quantize_map(ctx, d_all_colours, d_all_counts, M, N_total, d_shard, n_r, d_out_r, &K, palette)
- *     Step 3 merges the lists in the direct table, runs the split on the merged histogram (replicated:
- *     every rank takes identical decisions from identical integers) and remaps the rank's own rows.
- *     Result: dq_quant_recurse of the whole image when dq_call_stats::tie_flags is 0.  This form does NOT resolve
- *     flagged frames (no first-seen indexes travel in its exchange): a frame whose decision sat inside the reference's
- *     rounding noise (about 1 % of 1080p / 4K G1 frames) is reported in tie_flags and may differ from the reference by
- *     one LSB in a palette entry.  dq_rows_* below resolves them.
+ *     palette is independent of the number of shards.  The one exchange runs inside the library (NCCL over NVLink, looked
+ *     up with dlopen("libnccl.so.2") at run time, so the copy the process already has -- e.g. PyTorch's -- is used and the
+ *     library has no link-time dependency on it).
  * ---------------------------------------------------------------------------------------------- */
-/* Unique colours and counts of a shard into caller-provided DEVICE arrays (capacity n_shard each). */
-uint32_t dq_shard_histogram(dq_context *ctx, const uint32_t *d_shard, uint32_t n_shard, uint32_t *d_colours,
-                            uint32_t *d_counts);
-void dq_shard_quantize_map(dq_context *ctx, const uint32_t *d_all_colours, const uint32_t *d_all_counts, uint32_t num_entries,
-                           uint64_t total_pixels, const uint32_t *d_shard, uint32_t n_shard, uint32_t *d_out_shard,
-                           uint32_t *numClustersPtr, uint32_t *outColortablePtr);
-
-/* The same with the exchange INSIDE the library (NCCL over NVLink, looked up with dlopen("libnccl.so.2") at run time, so
- * the copy the process already has -- e.g. PyTorch's -- is used and the library has no link-time dependency on it).
- *   rank 0:      dq_rows_unique_id(id)            -> hand the 128 bytes to every rank (any side channel)
+/*   rank 0:      dq_rows_unique_id(id)            -> hand the 128 bytes to every rank (any side channel)
  *   every rank:  rows = dq_rows_create(ctx, world, rank, id, list_capacity)          (collective: ncclCommInitRank)
  *   per image:   dq_rows_quant_recurse(rows, d_shard, n_shard, N_total, d_out_shard, &K, palette)
  * One grouped ncclAllGather per image on the context's stream of three fixed-capacity slices per rank: colours, counts

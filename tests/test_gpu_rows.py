@@ -1,7 +1,6 @@
 """GPU test of the pixel-row sharded path (BASELINE.json config 3): histogram per shard, one all-gather of the
 (colour, count) lists, merged split replicated on every rank, shard-local remap -- bit-exact against the
-single-GPU quant_recurse of the whole image.  Uses as many GPUs as the box has (1 GPU still exercises the
-dq_shard_* entry points; 2+ GPUs go through NCCL)."""
+single-GPU quant_recurse of the whole image.  Uses as many GPUs as the box has (2+ GPUs go through NCCL)."""
 import os
 import subprocess
 import sys

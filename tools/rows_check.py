@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Row-sharded quant_recurse of one image over the ranks of a torchrun job, checked against the single-GPU result of the
-whole image and timed next to it.  Two forms: the in-library exchange (dq_rows_*, one grouped ncclAllGather per image,
-no host wait before the palette) and the caller-owned exchange (dq_shard_* + torch.distributed all-gather).
+"""Row-sharded quant_recurse of one image over the ranks of a torchrun job (dq_rows_*: one grouped ncclAllGather per
+image inside the library, no host wait before the palette), checked against the single-GPU result of the whole image and
+timed next to it.
 With a seed, the image is G1 of that seed; where tests/golden/frames.npz holds the compiled reference's fingerprint of that
 image (1920x1080 K=64, 3840x2160 K=256), the single-GPU result is checked against it as well.
 usage: torchrun --nproc-per-node N tools/rows_check.py [w h K reps [seed]]"""
@@ -34,9 +34,6 @@ shard = torch.from_numpy(img[r0 * w:r1 * w].view(np.int32).copy()).cuda()
 d = dist if world > 1 else None
 rows = pkg.RowShards(lib, ctx, d, list_capacity=1 << 18)
 out, pal = rows.quant_recurse(shard, w * h, k)
-out_py, pal_py = pkg.row_sharded_quant_recurse(lib, ctx, shard, w * h, k, d)
-st_py = pkg.CallStats()
-lib.dq_context_last_stats(ctx, C.byref(st_py))
 # reference: the whole image on this GPU alone
 full = torch.from_numpy(img.view(np.int32)).cuda()
 full_out = torch.empty_like(full)
@@ -52,9 +49,6 @@ def single():
 
 single()
 ok = np.array_equal(pal, ct[:nk.value]) and torch.equal(out, full_out[r0 * w:r1 * w])
-# the caller-owned exchange (dq_shard_*) does not resolve flagged frames: it has to match unless it reports the frame
-ok_py = np.array_equal(pal_py, ct[:nk.value]) and torch.equal(out_py, full_out[r0 * w:r1 * w])
-ok = ok and (ok_py or st_py.tie_flags != 0)
 golden = None
 tag = {(1920, 1080, 64): "c4", (3840, 2160, 256): "bench"}.get((w, h, k))
 if tag:
@@ -87,9 +81,7 @@ def timed(fn):
     return float(ms.item())
 
 
-ws = {}
 ms_lib = timed(lambda: rows.quant_recurse(shard, w * h, k, out))
-ms_py = timed(lambda: pkg.row_sharded_quant_recurse(lib, ctx, shard, w * h, k, d, ws))
 ms_one = timed(single)
 flag = torch.tensor([1 if ok else 0], device="cuda")
 if d:
@@ -97,10 +89,8 @@ if d:
 if rank == 0:
     verdict = "bit-exact vs single GPU" if flag.item() else "MISMATCH"
     verdict += {None: "", True: ", reference fingerprint ok", False: ", reference fingerprint MISMATCH"}[golden]
-    if not ok_py:
-        verdict += f" (caller-owned exchange reports tie_flags {st_py.tie_flags} and is not resolved)"
-    print(f"rows x{world} {w}x{h} K={k} seed {seed}: {verdict}; in-library exchange {ms_lib:.3f} ms/image, "
-          f"caller-owned exchange {ms_py:.3f}, one GPU alone {ms_one:.3f}", flush=True)
+    print(f"rows x{world} {w}x{h} K={k} seed {seed}: {verdict}; {ms_lib:.3f} ms/image, one GPU alone {ms_one:.3f}",
+          flush=True)
 rows.close()
 if d:
     d.destroy_process_group()

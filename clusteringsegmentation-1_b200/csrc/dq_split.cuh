@@ -76,7 +76,7 @@ struct SplitRecord {
 };
 
 // timeline tags
-enum TraceTag { kTraceRoundBegin = 1, kTracePhaseA = 2, kTracePhaseB = 3, kTracePhaseC = 4, kTraceCtlBarrier = 5, kTracePass = 6, kTracePartition = 7, kTraceRoot = 8, kTraceBegin = 9, kTraceCollected = 10, kTraceReduced = 11, kTraceRootBarrier = 12 };
+enum TraceTag { kTraceRoundBegin = 1, kTracePhaseA = 2, kTracePhaseB = 3, kTracePhaseC = 4, kTraceCtlBarrier = 5, kTracePass = 6, kTracePartition = 7, kTraceRoot = 8, kTraceBegin = 9, kTraceCollected = 10, kTraceReduced = 11, kTraceRootBarrier = 12, kTraceNarrowJob = 13 };
 
 enum CtlSlot {
   kCtlJobs = 0,    // jobs in the current round

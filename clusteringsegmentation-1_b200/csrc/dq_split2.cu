@@ -39,6 +39,10 @@ constexpr uint32_t kWideTile = 1024;  // points per wide tile
 constexpr int kWidePPT = 2;           // points per thread when a CTA classifies its share of a wide job
 constexpr int kNarrowPPT = 8;         // points per thread of a narrow job (kept in registers for all passes)
 constexpr uint32_t kNarrowMax = kNarrowPPT * T;
+constexpr int kGroupWarps = 8;                 // warps of a narrow-job group
+constexpr int kGroups = kWarps / kGroupWarps;  // narrow jobs a CTA runs side by side
+constexpr int kGroupT = 32 * kGroupWarps;
+constexpr uint32_t kGroupMax = kNarrowPPT * kGroupT;  // largest narrow job a group holds in registers
 constexpr int kWideCache = 4;         // wide jobs whose constants a CTA keeps in shared memory
 constexpr unsigned long long kValueMask = (1ull << 48) - 1ull;
 
@@ -53,6 +57,20 @@ struct JobAudit {
   double eW, eS, eM, m1;  // m1 = max |tm_c|
 };
 constexpr int kAudCache = 32;  // wide jobs of a CTA whose audit constants are kept (more than that: flagged wholesale)
+
+// A narrow job in flight in a group of kGroupWarps warps: the fields of Shared2 that one narrow job uses, under the same names.
+struct NarrowGroup {
+  uint64_t red[kGroupWarps][kAccWords];
+  uint64_t tot[kAccWords];
+  PassParams pp;
+  tie::PassExt ext;
+  JobAudit aud;
+  SplitNode cur;
+  uint64_t prev_tot[4];
+  int32_t converged;
+  uint32_t near, job_tie, cur_old, cur_new;
+  int32_t next;  // the group's next entry of mynarrow
+};
 
 struct Shared2 {
   uint64_t red[32][kAccWords];
@@ -78,12 +96,23 @@ struct Shared2 {
   tie::PassExt ext;   // tie audit: centres and bounds behind S.pp (written with it)
   JobAudit aud;       // tie audit: constants of the narrow job in flight
   JobAudit wide_aud[kAudCache];
-  uint32_t near;      // tie audit: points of the pass just reduced / gathered that sit inside the noise bound
+  uint32_t near;     // tie audit: points of the pass just reduced / gathered that sit inside the noise bound
   uint32_t job_tie;   // TieBit mask of the narrow job in flight
   uint32_t tie_total; // TieBit mask of the frame (CTA 0, final assignment + palette)
   uint32_t cut_count; // consumed splits whose cut is flagged (kTieCut): entries of the second list of SplitArgs::tie_list
   CutOverride ovr[kCutOverrideCap];  // SplitArgs::cut_overrides, staged
   uint32_t n_ovr;
+  NarrowGroup grp[kGroups];
+  int32_t narrow_next;  // entries of mynarrow handed to the groups so far
+};
+
+// Barriers of the helpers that run either on the whole CTA or on one narrow-job group (named barrier 1 + group).
+struct CtaSync {
+  __device__ __forceinline__ void operator()() const { __syncthreads(); }
+};
+struct GroupSync {
+  int id;
+  __device__ __forceinline__ void operator()() const { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(kGroupT) : "memory"); }
 };
 
 struct Arrays {
@@ -104,6 +133,10 @@ struct Arrays {
   double *terr;        // [cap]  tie audit: bound of the node's TSE
   int32_t *byrank;     // [cap]  tie audit: node of every TSE rank (final assignment)
   uint8_t *jobtie;     // [K]    tie audit: TieBit mask of this round's wide jobs (owner CTA)
+  // Fixed-point exit of this CTA's wide jobs, indexed like mywide.  Only the controller's selection uses rank[] and cand[],
+  // so these two live in their memory.
+  uint64_t (*wprev)[4];  // [K]  {cnt, R, G, B} of the last pass gathered (in rank[], cap * 4 >= K * 32 bytes)
+  int32_t *wfin;         // [K]  1 + the pass that ran as the job's final one, 0 while it runs (in cand[])
 };
 
 __device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long *p) {
@@ -206,9 +239,9 @@ __device__ __forceinline__ uint64_t warp_sum_redux(uint64_t v) {
 // the usual case) or two 24/26-bit limbs are needed: the REDUX unit, not latency, bounds this stage
 // (tools/microbench/classify_mb.cu: 340 cycles against 500 with a vote per word and 1000 with two limbs always).
 // Ends with a barrier.
-template <int WORDS>
-__device__ __forceinline__ void reduce_stage1(Shared2 &S, const uint64_t (&v)[kAccWords], int warps) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+template <int WORDS, typename St, typename Sync = CtaSync>
+__device__ __forceinline__ void reduce_stage1(St &S, const uint64_t (&v)[kAccWords], int warps, int t = threadIdx.x, Sync sync = Sync()) {
+  const int lane = t & 31, warp = t >> 5;
   if (warp < warps) {
     uint64_t all = 0;
 #pragma unroll
@@ -230,13 +263,13 @@ __device__ __forceinline__ void reduce_stage1(Shared2 &S, const uint64_t (&v)[kA
       for (int w = 0; w < WORDS; ++w) S.red[warp][w] = s[w];
     }
   }
-  __syncthreads();
+  sync();
 }
 
 // Stage 2, executed by warp 0 only: sums rows 0..rows-1 (<= 32) of S.red (values below 2^54) into
 // S.tot with two 27-bit limbs per word.  Totals are visible to warp 0 on return (no CTA barrier).
-template <int WORDS>
-__device__ __forceinline__ void reduce_stage2_warp0(Shared2 &S, int rows) {
+template <int WORDS, typename St>
+__device__ __forceinline__ void reduce_stage2_warp0(St &S, int rows) {
   const int lane = threadIdx.x & 31;
   uint64_t x[WORDS];
 #pragma unroll
@@ -253,8 +286,9 @@ __device__ __forceinline__ void reduce_stage2_warp0(Shared2 &S, int rows) {
 // Tie audit: the classification adds (near ? 1 : 0) << 32 per thread to the point counter (kAccPts), so the number of
 // threads that saw a point inside the noise bound rides through every reduction and exchange for free.  Warp 0 calls
 // this once the totals are in S.tot: S.near = that number, S.tot[kAccPts] = the plain point count again.
-__device__ __forceinline__ void split_near_warp0(Shared2 &S) {
-  if (threadIdx.x == 0) {
+template <typename St>
+__device__ __forceinline__ void split_near_warp0(St &S, int t = threadIdx.x) {
+  if (t == 0) {
     S.near = (uint32_t)(S.tot[kAccPts] >> 32);
     S.tot[kAccPts] &= 0xFFFFFFFFull;
   }
@@ -344,9 +378,10 @@ __device__ __forceinline__ SplitNode load_node(const SplitArgs &A, const Shared2
 
 // Classification parameters of the next pass from the totals in S.tot, computed by warp 0
 // (one lane per channel), left in S.pp.  Caller synchronises afterwards.
-__device__ __forceinline__ void derive_params_warp0(Shared2 &S, const JobConst &jc, double norm) {
-  if (threadIdx.x < 32) {  // uniform per warp
-    const int c = min((int)threadIdx.x, 2);
+template <typename St>
+__device__ __forceinline__ void derive_params_warp0(St &S, const JobConst &jc, double norm, int t = threadIdx.x) {
+  if (t < 32) {  // uniform per warp
+    const int c = min(t, 2);
     const double nw = fmul(u52_to_double(S.tot[kAccCnt]), norm);
     const double nm = fdiv(fmul(u52_to_double(S.tot[kAccR + c]), norm), nw);
     const double ow = fsub(jc.tw, nw);
@@ -354,12 +389,12 @@ __device__ __forceinline__ void derive_params_warp0(Shared2 &S, const JobConst &
     const double a = fsq(om), b = fsq(nm);
     const double a1 = __shfl_sync(0xffffffffu, a, 1), b1 = __shfl_sync(0xffffffffu, b, 1);
     const double a2 = __shfl_sync(0xffffffffu, a, 2), b2 = __shfl_sync(0xffffffffu, b, 2);
-    if (threadIdx.x < 3) {
+    if (t < 3) {
       S.pp.r[c] = fsub(om, nm);
       S.ext.om[c] = om;  // (tie audit: the centres themselves, for the cold per-point re-check)
       S.ext.nm[c] = nm;
     }
-    if (threadIdx.x == 0) {
+    if (t == 0) {
       double l = fsub(a, b);  // (:616-619), left to right
       l = fadd(l, a1);
       l = fsub(l, b1);
@@ -377,15 +412,18 @@ __device__ __forceinline__ void derive_params_warp0(Shared2 &S, const JobConst &
 // Tie audit, next to derive_params_warp0 and at the same time: WARP 1 sums the rows of S.red itself (the totals warp 0
 // is reducing into S.tot), derives the same centres and from them the tolerance of the next pass's hyperplane test
 // (dq_tie.cuh), so that the bound costs the split's critical path nothing.  Writes S.pp.tol_hi and S.ext only.
-__device__ __forceinline__ uint64_t warp_total_row(const Shared2 &S, int lane, int rows, int w) {
+template <typename St>
+__device__ __forceinline__ uint64_t warp_total_row(const St &S, int lane, int rows, int w) {
   const uint64_t x = lane < rows ? S.red[lane][w] : 0ull;
   const unsigned lo = __reduce_add_sync(0xffffffffu, (unsigned)(x & 0x7FFFFFFu));
   const unsigned hi = __reduce_add_sync(0xffffffffu, (unsigned)(x >> 27));
   return (uint64_t)lo + ((uint64_t)hi << 27);
 }
-__device__ __forceinline__ void derive_audit_warp1(Shared2 &S, const JobConst &jc, const JobAudit *aud, double norm, int rows) {
-  if (threadIdx.x >= 32 && threadIdx.x < 64) {  // uniform per warp
-    const int lane = threadIdx.x & 31;
+template <typename St>
+__device__ __forceinline__ void derive_audit_warp1(St &S, const JobConst &jc, const JobAudit *aud, double norm, int rows,
+                                                   int t = threadIdx.x) {
+  if (t >= 32 && t < 64) {  // uniform per warp
+    const int lane = t & 31;
     const double eM = aud ? aud->eM : 0.0;
     if (eM < 0.0) {  // audit off
       if (lane == 0) S.pp.tol_hi = -1;
@@ -415,21 +453,23 @@ __device__ __forceinline__ void derive_audit_warp1(Shared2 &S, const JobConst &j
   }
 }
 
-__device__ __forceinline__ void set_split_params(Shared2 &S, const JobConst &jc, const JobAudit *aud) {
-  if (threadIdx.x == 0) {
-    S.pp.a = jc.cut;
+template <typename St>
+__device__ __forceinline__ void set_split_params(const Shared2 &S, St &G, const JobConst &jc, const JobAudit *aud,
+                                                 int t = threadIdx.x) {
+  if (t == 0) {
+    G.pp.a = jc.cut;
     // a cut taken from SplitArgs::cut_overrides is the reference's own comparison: not audited
     bool forced = false;
     for (uint32_t i = 0; i < S.n_ovr; ++i)
       forced = forced || (S.ovr[i].begin == jc.begin && S.ovr[i].size == jc.size && S.ovr[i].mean_ref == jc.cut);
     const double eM = forced ? -1.0 : (aud ? aud->eM : __longlong_as_double(0x7ff0000000000000ll));
-    S.ext.tol = eM;  // tie audit of the cut test (:473): the cut is the node's mean (a forced cut is the reference's own)
-    S.pp.tol_hi = __double2hiint(eM) + (eM >= 0.0 ? 1 : 0);
-    S.pp.r[0] = S.pp.r[1] = S.pp.r[2] = 0.0;
-    S.pp.axis = jc.axis;
-    S.pp.buf = jc.buf;
-    S.pp.begin = jc.begin;
-    S.pp.size = jc.size;
+    G.ext.tol = eM;  // tie audit of the cut test (:473): the cut is the node's mean (a forced cut is the reference's own)
+    G.pp.tol_hi = __double2hiint(eM) + (eM >= 0.0 ? 1 : 0);
+    G.pp.r[0] = G.pp.r[1] = G.pp.r[2] = 0.0;
+    G.pp.axis = jc.axis;
+    G.pp.buf = jc.buf;
+    G.pp.begin = jc.begin;
+    G.pp.size = jc.size;
   }
 }
 
@@ -476,9 +516,10 @@ __device__ __forceinline__ void add_point(uint64_t (&v)[kAccWords], uint2 p, boo
 }
 
 // Owner of a finished split writes its two children (totals of the last pass in S.tot, parent in S.cur).
-__device__ __forceinline__ void write_children(const SplitArgs &A, Shared2 &S, int node_id, int child0, const JobConst &jc,
-                                               uint32_t tie_bits) {
-  if (threadIdx.x == 0) {
+template <typename St>
+__device__ __forceinline__ void write_children(const SplitArgs &A, St &S, int node_id, int child0, const JobConst &jc,
+                                               uint32_t tie_bits, int t = threadIdx.x) {
+  if (t == 0) {
     SplitNode o, n;
     make_children(S.cur, node_id, child0, A.norm, S.tot, o, n, A.tie_audit != 0u);
     A.nodes[child0] = o;
@@ -889,9 +930,9 @@ __device__ void sequential_controller(const SplitArgs &A, Shared2 &S, const Arra
 // One pass of a narrow job: classify the (register-resident) points, reduce, and -- except after the
 // last pass -- derive the next pass's parameters.  SPLIT: cut test of pass 0; FINAL: last LKM pass
 // (also sums count*c*c).  Returns the membership mask of this thread's points.
-template <bool SPLIT, bool FINAL>
-__device__ __forceinline__ unsigned narrow_pass(Shared2 &S, const uint2 (&p)[kNarrowPPT], unsigned validmask, int ppt,
-                                                int nwarps, const JobConst &jc, double norm) {
+template <bool SPLIT, bool FINAL, typename St, typename Sync>
+__device__ __forceinline__ unsigned narrow_pass(St &S, const uint2 (&p)[kNarrowPPT], unsigned validmask, int ppt, int nwarps,
+                                                const JobConst &jc, double norm, int t, Sync sync) {
   // (tie audit constants of the narrow job in flight: S.aud)
   const PassParams pp = S.pp;
   AccD acc = acc_zero();
@@ -916,16 +957,16 @@ __device__ __forceinline__ unsigned narrow_pass(Shared2 &S, const uint2 (&p)[kNa
   acc_words(acc, v);
   v[kAccPts] += (uint64_t)near << 32;  // tie audit (split_near_warp0)
   constexpr int WORDS = FINAL ? kAccWords : 5;
-  reduce_stage1<WORDS>(S, v, nwarps);
-  if (threadIdx.x < 32) {
+  reduce_stage1<WORDS>(S, v, nwarps, t, sync);
+  if (t < 32) {
     reduce_stage2_warp0<WORDS>(S, nwarps);
-    split_near_warp0(S);
-    if (threadIdx.x == 0 && S.near) S.job_tie |= SPLIT ? (uint32_t)kTieCut : (uint32_t)kTieHyperplane;
+    split_near_warp0(S, t);
+    if (t == 0 && S.near) S.job_tie |= SPLIT ? (uint32_t)kTieCut : (uint32_t)kTieHyperplane;
     if (!FINAL) {
       // Fixed point of the local 2-means: the next pass's parameters are a function of {cnt, R, G, B} only, so
       // equal sums in two consecutive passes mean every later pass repeats this one exactly -- the remaining
       // iterations can be skipped without changing a bit of the result (the caller goes straight to the last pass).
-      if (threadIdx.x == 0) {
+      if (t == 0) {
         bool same = !SPLIT;
 #pragma unroll
         for (int w = 0; w < 4; ++w) {
@@ -934,12 +975,12 @@ __device__ __forceinline__ unsigned narrow_pass(Shared2 &S, const uint2 (&p)[kNa
         }
         S.converged = same ? 1 : 0;
       }
-      derive_params_warp0(S, jc, norm);
+      derive_params_warp0(S, jc, norm, t);
     }
   } else if (!FINAL) {
-    derive_audit_warp1(S, jc, &S.aud, norm, nwarps);
+    derive_audit_warp1(S, jc, &S.aud, norm, nwarps, t);
   }
-  __syncthreads();
+  sync();
   return newmask;
 }
 
@@ -987,6 +1028,80 @@ __device__ __forceinline__ void wide_classify(const PassParams &pp, const tie::P
   v[kAccPts] += (uint64_t)near << 32;  // tie audit (split_near_warp0)
 }
 
+// One narrow job, start to finish, on GT threads (the CTA, or one group): load its points into registers, run its passes
+// to the fixed point, partition, write the children.  St = the job's state (Shared2 or a NarrowGroup), t = this thread's
+// index among the GT, sync = their barrier.
+template <int GT, typename St, typename Sync>
+__device__ __forceinline__ void narrow_job(const SplitArgs &A, const Shared2 &S, St &G, const Arrays &R, int j, int child_base,
+                                           int P, int t, Sync sync) {
+  const int lane = t & 31;
+  const int node = R.jobnode[j];
+  if (t == 0) {
+    const bool audit = A.tie_audit != 0u;
+    G.cur = load_node(A, S, node);
+    G.cur_old = 0;
+    G.cur_new = 0;
+    G.aud = job_audit_of(G.cur, audit);
+    G.job_tie = (audit && tie::axis_tie(G.cur.tv, G.cur.eV)) ? (uint32_t)kTieAxis : 0u;  // D1 (:388-403)
+  }
+  sync();
+  const JobConst jc = job_const_of(S, G.cur);
+  // all warps the job has points for; up to kNarrowPPT points per thread, held in registers for every pass
+  const uint32_t nthr = min((uint32_t)GT, max(32u, (jc.size + 31u) & ~31u));
+  const int nwarps = (int)(nthr >> 5);
+  uint2 p[kNarrowPPT];
+  unsigned validmask = 0;
+#pragma unroll
+  for (int k = 0; k < kNarrowPPT; ++k) {
+    const uint32_t off = (uint32_t)k * nthr + (uint32_t)t;
+    p[k] = make_uint2(0, 0);
+    if ((uint32_t)t < nthr && off < jc.size) {
+      p[k] = ld_cg_u2(A.pts[jc.buf] + jc.begin + off);
+      validmask |= 1u << k;
+    }
+  }
+  set_split_params(S, G, jc, &G.aud, t);
+  sync();
+  const int ppt = (int)((jc.size + nthr - 1) / nthr);
+  unsigned newmask = narrow_pass<true, false>(G, p, validmask, ppt, nwarps, jc, A.norm, t, sync);
+  int pass = 1;
+  for (; pass < P; ++pass) {
+    newmask = narrow_pass<false, false>(G, p, validmask, ppt, nwarps, jc, A.norm, t, sync);
+    if (G.converged) {  // uniform in the group: written before the barrier that ends the pass
+      ++pass;
+      break;
+    }
+  }
+  newmask = narrow_pass<false, true>(G, p, validmask, ppt, nwarps, jc, A.norm, t, sync);
+  trace2(A, kTraceNarrowJob, pass + 1);  // passes run, the cut pass and the final one included
+  // G.tot = totals of the last pass; newmask = membership decided by it
+  const uint32_t size_old = jc.size - (uint32_t)G.tot[kAccPts];
+  if ((uint32_t)t < nthr) {
+#pragma unroll
+    for (int k = 0; k < kNarrowPPT; ++k) {
+      const bool valid = (validmask >> k) & 1u;
+      const bool to_new = (newmask >> k) & 1u;
+      const unsigned m_new = __ballot_sync(0xffffffffu, to_new);
+      const unsigned m_old = __ballot_sync(0xffffffffu, valid && !to_new);
+      uint32_t base_new = 0, base_old = 0;
+      if (lane == 0) {
+        if (m_new) base_new = atomicAdd(&G.cur_new, (uint32_t)__popc(m_new));
+        if (m_old) base_old = atomicAdd(&G.cur_old, (uint32_t)__popc(m_old));
+      }
+      base_new = __shfl_sync(0xffffffffu, base_new, 0);
+      base_old = __shfl_sync(0xffffffffu, base_old, 0);
+      if (valid) {
+        const unsigned below = (1u << lane) - 1u;
+        const uint32_t dst = to_new ? jc.begin + size_old + base_new + __popc(m_new & below)
+                                    : jc.begin + base_old + __popc(m_old & below);
+        A.pts[jc.buf ^ 1][dst] = p[k];
+      }
+    }
+  }
+  write_children(A, G, node, child_base + 2 * j, jc, G.job_tie, t);
+  sync();
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // The kernel
 // ---------------------------------------------------------------------------------------------------------
@@ -1011,12 +1126,14 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
     R.parent = reinterpret_cast<int32_t *>(cur);
     cur += (size_t)cap * 4;
     R.rank = reinterpret_cast<int32_t *>(cur);
+    R.wprev = reinterpret_cast<uint64_t(*)[4]>(cur);
     cur += (size_t)cap * 4;
     R.jobnode = reinterpret_cast<int32_t *>(cur);
     cur += (size_t)K * 4;
     R.cnode = reinterpret_cast<int32_t *>(cur);
     cur += (size_t)K * 4;
     R.cand = reinterpret_cast<int32_t *>(cur);
+    R.wfin = R.cand;
     cur += (size_t)K * 4;
     R.tile0 = reinterpret_cast<uint32_t *>(cur);
     cur += (size_t)(K + 1) * 4;
@@ -1320,6 +1437,7 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       }
     }
     const int n_mywide = S.n_mywide, n_mynarrow = S.n_mynarrow;
+    for (int mw = tid; mw < n_mywide; mw += T) R.wfin[mw] = 0;
     for (int mw = tid; mw < min(n_mywide, kAudCache); mw += T) {
       // (executed by a few threads) constants of the first few wide jobs stay in shared memory
       const SplitNode nd = load_node(A, S, R.jobnode[R.mywide[mw]]);
@@ -1372,10 +1490,17 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
         if ((uint32_t)tid < nthr && q < n_my) pre0[k] = ld_cg_u2(A.pts[jc.buf] + jc.begin + sh.first_point + q);
       }
     }
-    for (int pass = 0; pass <= P; ++pass) {
+    // Fixed-point exit: every participant gathers the same totals, so each of them finds on its own
+    // that {cnt, R, G, B} repeat the previous pass's -- the next parameters, and so every later classification, repeat
+    // that pass exactly -- and runs this pass as the final one, as a narrow job does.  The participants therefore all
+    // publish their final sums in the same pass and nobody writes the job's slots afterwards: the two slot buffers stay
+    // enough, the final sums simply sit in the buffer and under the tag of that pass (R.wfin).
+    int n_running = n_mywide;  // CTA-uniform
+    for (int pass = 0; pass <= P && n_running > 0; ++pass) {
       unsigned long long *slots_w = X.slots + (size_t)(pass & 1) * X.slot_cap * kAccWords;
       const unsigned long long *slots_r = X.slots + (size_t)((pass & 1) ^ 1) * X.slot_cap * kAccWords;
       for (int mw = 0; mw < n_mywide; ++mw) {
+        if (R.wfin[mw] != 0) continue;
         const int j = R.mywide[mw];
         const JobConst jc = wide_const(mw);
         const Share sh = share_of(j, jc.size);
@@ -1400,7 +1525,7 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
 #endif
         const JobAudit *aud = (mw < kAudCache) ? &S.wide_aud[mw] : nullptr;
         if (pass == 0) {
-          set_split_params(S, jc, aud);
+          set_split_params(S, S, jc, aud);
         } else {
           gather(A, S, slots_r, R.slot0[j], m, 5, (seq0 + pass - 1) & 0xFFFFu);
           if (tid == 0 && S.near) R.jobtie[j] |= (pass == 1) ? (uint8_t)kTieCut : (uint8_t)kTieHyperplane;
@@ -1409,24 +1534,36 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
 #endif
           derive_params_warp0(S, jc, A.norm);
           derive_audit_warp1(S, jc, aud, A.norm, kWarps);
+          if (tid == 0 && pass < P) {
+            bool same = pass >= 2;  // (pass 1 gathers the cut pass's sums)
+#pragma unroll
+            for (int w = 0; w < 4; ++w) {
+              same = same && (R.wprev[mw][w] == S.tot[w]);
+              R.wprev[mw][w] = S.tot[w];
+            }
+            S.converged = same ? 1 : 0;
+          }
         }
         __syncthreads();
 #ifdef DQ_PROFILE_NARROW
         const long long w2 = clock64();
 #endif
+        const bool fin = pass == P || (pass >= 2 && S.converged != 0);  // CTA-uniform
         const PassParams pp = S.pp;
         uint64_t v[kAccWords];
         {
           const uint2 *seg = A.pts[jc.buf] + jc.begin;
           auto off = [&](uint32_t q) { return sh.first_point + q; };
           if (pass == 0) wide_classify<true, false>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
-          else if (pass == P) wide_classify<false, true>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
+          else if (fin) wide_classify<false, true>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
           else wide_classify<false, false>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
         }
 #ifdef DQ_PROFILE_NARROW
         const long long w3 = clock64();
 #endif
-        if (pass == P) {
+        if (fin) {
+          --n_running;
+          if (tid == 0) R.wfin[mw] = pass + 1;
           if (tid == 0 && mw < kWideCache) S.wide_pp[mw] = pp;
           reduce_stage1<kAccWords>(S, v, (int)(nthr >> 5));
           if (tid < 32) {
@@ -1480,15 +1617,17 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       const Share sh = share_of(j, jc.size);
       const int m = (int)sh.m;
       const uint32_t me = sh.me;
-      // classification of the last pass (parameters from the totals of pass P-1)
+      const int pf = R.wfin[mw] - 1;  // the job's final pass
+      // classification of the final pass (parameters from the totals of pass pf-1)
       if (mw >= kWideCache) {
-        gather(A, S, X.slots + (size_t)((P - 1) & 1) * X.slot_cap * kAccWords, R.slot0[j], m, 5, (seq0 + P - 1) & 0xFFFFu);
+        gather(A, S, X.slots + (size_t)((pf - 1) & 1) * X.slot_cap * kAccWords, R.slot0[j], m, 5, (seq0 + pf - 1) & 0xFFFFu);
         derive_params_warp0(S, jc, A.norm);  // (only the partition's re-classification follows: no audit)
         __syncthreads();
       }
       const PassParams pp = (mw < kWideCache) ? S.wide_pp[mw] : S.pp;
       __syncthreads();
-      gather(A, S, X.slots + (size_t)(P & 1) * X.slot_cap * kAccWords, R.slot0[j], m, kAccWords, (seq0 + P) & 0xFFFFu);
+      const unsigned long long *slots_p = X.slots + (size_t)(pf & 1) * X.slot_cap * kAccWords;
+      gather(A, S, slots_p, R.slot0[j], m, kAccWords, (seq0 + pf) & 0xFFFFu);
       if (tid == 0 && S.near) R.jobtie[j] |= (uint8_t)kTieHyperplane;
       __syncthreads();
       if (S.tot[kAccPts] > jc.size) continue;  // only after an expired wait: never scatter out of the segment
@@ -1499,7 +1638,6 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       {
         // (shares are contiguous and in CTA order: the points before mine are simply those of the tiles before mine)
         uint32_t before_new = 0;
-        const unsigned long long *slots_p = X.slots + (size_t)(P & 1) * X.slot_cap * kAccWords;
         for (uint32_t i = (uint32_t)tid; i < me; i += T)
           before_new += (uint32_t)(ld_relaxed_u64(slots_p + (size_t)(R.slot0[j] + i) * kAccWords + kAccPts) & kValueMask);
         before_new = __reduce_add_sync(0xffffffffu, before_new);
@@ -1559,66 +1697,31 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
     DQ_PROGRESS(round * 10000 + 3000);
 
     // ================= narrow jobs: everything inside this CTA =================
+    // Jobs of more than kGroupMax points take the whole CTA, one after the other; the others run kGroups at a time, one per
+    // group of kGroupWarps warps, each group taking the CTA's next such job as soon as it is free.
     for (int mn = 0; mn < n_mynarrow; ++mn) {
       const int j = R.mynarrow[mn];
-      const int node = R.jobnode[j];
-      if (tid == 0) {
-        S.cur = load_node(A, S, node);
-        S.cur_old = 0;
-        S.cur_new = 0;
-        S.aud = job_audit_of(S.cur, audit);
-        S.job_tie = (audit && tie::axis_tie(S.cur.tv, S.cur.eV)) ? (uint32_t)kTieAxis : 0u;  // D1 (:388-403)
-      }
+      if (R.size[R.jobnode[j]] > kGroupMax) narrow_job<T>(A, S, S, R, j, child_base, P, tid, CtaSync());
+    }
+    if (n_mynarrow) {
+      if (tid == 0) S.narrow_next = 0;
       __syncthreads();
-      const JobConst jc = job_const_of(S, S.cur);
-      // all warps the job has points for; up to kNarrowPPT points per thread, held in registers for every pass
-      const uint32_t nthr = min((uint32_t)T, max(32u, (jc.size + 31u) & ~31u));
-      const int nwarps = (int)(nthr >> 5);
-      uint2 p[kNarrowPPT];
-      unsigned validmask = 0;
-#pragma unroll
-      for (int k = 0; k < kNarrowPPT; ++k) {
-        const uint32_t off = (uint32_t)k * nthr + tid;
-        p[k] = make_uint2(0, 0);
-        if ((uint32_t)tid < nthr && off < jc.size) {
-          p[k] = ld_cg_u2(A.pts[jc.buf] + jc.begin + off);
-          validmask |= 1u << k;
+      const int t = tid % kGroupT;
+      NarrowGroup &G = S.grp[tid / kGroupT];
+      const GroupSync gsync{1 + tid / kGroupT};
+      for (;;) {
+        if (t == 0) {
+          int k;
+          do {
+            k = atomicAdd(&S.narrow_next, 1);
+          } while (k < n_mynarrow && R.size[R.jobnode[R.mynarrow[k]]] > kGroupMax);
+          G.next = k;
         }
+        gsync();
+        const int k = G.next;  // (rewritten only after the job's closing barrier)
+        if (k >= n_mynarrow) break;
+        narrow_job<kGroupT>(A, S, G, R, R.mynarrow[k], child_base, P, t, gsync);
       }
-      set_split_params(S, jc, &S.aud);
-      __syncthreads();
-      const int ppt = (int)((jc.size + nthr - 1) / nthr);
-      unsigned newmask = narrow_pass<true, false>(S, p, validmask, ppt, nwarps, jc, A.norm);
-      for (int pass = 1; pass < P; ++pass) {
-        newmask = narrow_pass<false, false>(S, p, validmask, ppt, nwarps, jc, A.norm);
-        if (S.converged) break;  // CTA-uniform: written before the barrier that ends the pass
-      }
-      newmask = narrow_pass<false, true>(S, p, validmask, ppt, nwarps, jc, A.norm);
-      // S.tot = totals of the last pass; newmask = membership decided by it
-      const uint32_t size_old = jc.size - (uint32_t)S.tot[kAccPts];
-      if (tid < (int)nthr) {
-#pragma unroll
-        for (int k = 0; k < kNarrowPPT; ++k) {
-          const bool valid = (validmask >> k) & 1u;
-          const bool to_new = (newmask >> k) & 1u;
-          const unsigned m_new = __ballot_sync(0xffffffffu, to_new);
-          const unsigned m_old = __ballot_sync(0xffffffffu, valid && !to_new);
-          uint32_t base_new = 0, base_old = 0;
-          if (lane == 0) {
-            if (m_new) base_new = atomicAdd(&S.cur_new, (uint32_t)__popc(m_new));
-            if (m_old) base_old = atomicAdd(&S.cur_old, (uint32_t)__popc(m_old));
-          }
-          base_new = __shfl_sync(0xffffffffu, base_new, 0);
-          base_old = __shfl_sync(0xffffffffu, base_old, 0);
-          if (valid) {
-            const unsigned below = (1u << lane) - 1u;
-            const uint32_t dst = to_new ? jc.begin + size_old + base_new + __popc(m_new & below)
-                                        : jc.begin + base_old + __popc(m_old & below);
-            A.pts[jc.buf ^ 1][dst] = p[k];
-          }
-        }
-      }
-      write_children(A, S, node, child_base + 2 * j, jc, S.job_tie);
       __syncthreads();
     }
     if (n_mynarrow) trace2(A, kTracePartition, 1000 + n_mynarrow);

@@ -386,7 +386,8 @@ uint32_t dq_debug_histogram(dq_context *ctx, const uint32_t *inPixels, uint32_t 
  * its phase boundaries during the next calls.  Call again with pairs_out to fetch the last trace
  * (returns the number of pairs).  Tags: 1 round begin, 2 children finalised, 3 replay done, 4 jobs
  * issued, 5 barrier after controller, 6 pass done, 7 partition done, 8 root statistics done, 9 kernel entered,
- * 10 histogram collected, 11 root sums reduced, 12 root barrier passed. */
+ * 10 histogram collected, 11 root sums reduced, 12 root barrier passed, 13 narrow job done (arg = its passes,
+ * the final one included). */
 uint32_t dq_debug_split_timeline(dq_context *ctx, int enable, uint64_t *pairs_out, uint32_t capacity_pairs);
 
 /* Host-only pieces of the path (no device needed): the palette handling the shim does between the

@@ -99,6 +99,8 @@ def load_library(path=LIB_PATH):
         "dq_context_last_batch_stats": (None, [vp, C.POINTER(BatchStats)]),
         "dq_map_colors_batch_device": (None, [vp, C.c_uint32, _u32p, C.c_uint32, vp, vp, C.POINTER(C.c_int), _u32p, vp]),
         "dq_map_colors_batch_ctx": (None, [vp, C.c_uint32, _u32p, C.c_uint32, _u32p, _u32p, C.POINTER(C.c_int), _u32p, _u32p]),
+        "dq_quant_regions_device": (None, [vp, C.c_uint32, vp, vp, C.c_uint32, vp, _u32p, _u32p, vp]),
+        "dq_quant_regions_ctx": (None, [vp, C.c_uint32, _u32p, _u32p, C.c_uint32, _u32p, _u32p, _u32p, _u32p]),
         "dq_context_set_split_ctas": (None, [vp, C.c_int]),
         "dq_context_set_exact_small": (None, [vp, C.c_int]),
         "dq_context_set_exact_max_points": (None, [vp, C.c_uint32]),
@@ -156,7 +158,7 @@ EXPORTED_C_SYMBOLS = [
     "dq_pipeline_context", "dq_pipeline_kernel_launches", "dq_pipeline_flagged_frames",
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
     "dq_quant_recurse_batch_device", "dq_quant_recurse_batch_ctx", "dq_context_last_batch_stats",
-    "dq_map_colors_batch_device", "dq_map_colors_batch_ctx",
+    "dq_map_colors_batch_device", "dq_map_colors_batch_ctx", "dq_quant_regions_device", "dq_quant_regions_ctx",
     "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
     "dq_host_build_label_table",
 ]
@@ -287,6 +289,46 @@ class DivQuant:
                                                 flat.data_ptr(), out.data_ptr(), sizes.ctypes.data_as(C.POINTER(C.c_int)), _p(ct),
                                                 lab.data_ptr() if labels else None)
         return out, lab
+
+    def quant_regions(self, pixels, tags, ks, labels=False, ctx=None):
+        """quant_recurse of every region of a tag image, each to its own palette, in one call (dq_quant_regions_ctx).
+        Region r is pixels[tags == r] in raster order, quantized with ks[r] colours; pixels whose tag is >= len(ks) are
+        in no region and come back as 0 (label 0).  Returns (out, palettes, actual_k[, labels]): palettes is the uint32
+        array of sum(ks) words in which region r's palette starts at sum(ks[:r]) and holds actual_k[r] entries (0 for a
+        region with no pixels); out[tags == r] and its palette equal quant_recurse_batch's result for that region."""
+        px = _u32(pixels)
+        tg = _u32(tags)
+        nk = _u32(ks).copy()
+        if tg.size != px.size:
+            raise ValueError("one tag per pixel")
+        out = np.zeros_like(px)
+        lab = np.zeros_like(px) if labels else None
+        ct = np.zeros(max(int(nk.astype(np.int64).sum()), 1), np.uint32)
+        if nk.size:
+            self.lib.dq_quant_regions_ctx(ctx or self.lib.dq_default_context(), px.size, _p(px), _p(tg), nk.size, _p(out), _p(nk),
+                                          _p(ct), _p(lab) if labels else None)
+        return (out, ct, nk, lab) if labels else (out, ct, nk)
+
+    def quant_regions_device(self, pixels, tags, ks, labels=False, ctx=None, out=None, labels_out=None):
+        """Device form (dq_quant_regions_device): `pixels` and `tags` are contiguous CUDA tensors of 32-bit words, one tag
+        per pixel.  Writes out (and labels) at region pixels only: tensors passed as `out` / `labels_out` keep their other
+        pixels (a `labels_out` tensor implies labels=True).  Returns (out, palettes, actual_k[, labels]) as quant_regions."""
+        import torch
+        nk = _u32(ks).copy()
+        for t in (pixels, tags):
+            if t.dtype not in (torch.int32, torch.uint32) or not t.is_cuda or not t.is_contiguous():
+                raise ValueError("pixels and tags must be contiguous CUDA tensors of 32-bit words")
+        if tags.numel() != pixels.numel():
+            raise ValueError("one tag per pixel")
+        labels = labels or labels_out is not None
+        out = torch.zeros_like(pixels) if out is None else out
+        lab = (torch.zeros_like(pixels) if labels_out is None else labels_out) if labels else None
+        ct = np.zeros(max(int(nk.astype(np.int64).sum()), 1), np.uint32)
+        if nk.size:
+            torch.cuda.current_stream(pixels.device).synchronize()  # the library works on its context's stream
+            self.lib.dq_quant_regions_device(ctx or self.lib.dq_default_context(), pixels.numel(), pixels.data_ptr(), tags.data_ptr(),
+                                             nk.size, out.data_ptr(), _p(nk), _p(ct), lab.data_ptr() if labels else None)
+        return (out, ct, nk, lab) if labels else (out, ct, nk)
 
     def last_batch_stats(self, ctx=None):
         st = BatchStats()

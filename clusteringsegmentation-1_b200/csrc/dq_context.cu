@@ -191,6 +191,11 @@ struct dq_context {
   DevBuf<double> b_cluster_mean;
   PinnedBuf b_up, b_down, b_tab;
   dq_batch_stats batch_stats = {};
+  // quant_recurse of every region of a tag image (dq_regions.cu; quant_regions_impl below): the sort's (tag, index) pairs
+  // (2 x n, ping-pong), the pixels in sorted order [in | out | labels], [per-tile digit counts | digit totals | offsets]
+  DevBuf<uint2> r_pairs;
+  DevBuf<uint32_t> r_px, r_scratch;
+  PinnedBuf r_offsets;
   int use_mailbox = 1;  // DIVQUANT_B200_MAILBOX=0: always wait for the stream and copy
   void wait() {
     if (!blocking_wait) {
@@ -1009,9 +1014,10 @@ struct BatchRemap {
 // would split it on the ordered path in shared memory: weighted (all_unique = 0), K <= kSplit2MaxColors and at most
 // min(exact_max_points, kBatchMaxPoints) distinct colours with the ordered path on.  The histogram kernel finds U; any
 // other item goes through quant_recurse_device_impl, in item order between the batched items' palette handling, so that
-// the "# empty clusters" lines come out as a loop of single calls prints them.
+// the "# empty clusters" lines come out as a loop of single calls prints them.  d_labels (optional): every item's
+// dq_colortable_indexes (asGreyscale = 0) of its output in its deduped palette, the label image.
 void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, const uint32_t *d_in, uint32_t *d_out,
-                              uint32_t *ks, uint32_t *colortables, int all_unique) {
+                              uint32_t *ks, uint32_t *colortables, int all_unique, uint32_t *d_labels) {
   dq_batch_stats &bs = ctx->batch_stats;
   bs = dq_batch_stats();
   bs.items = num_items;
@@ -1075,7 +1081,7 @@ void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_
       if (empty) fprintf(stderr, "# empty clusters: %d\n", (int)empty);  // (:1067-1070)
       const uint32_t k = dedup_palette(ct, actual);
       ks[i] = k;
-      remap.add(ct, k, offsets[i] - base, n, false);
+      remap.add(ct, k, offsets[i] - base, n, d_labels != nullptr);
       bs.batched_items++;
       bs.empty_clusters += empty;
       host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1086,9 +1092,13 @@ void quant_recurse_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_
       launches += ctx->stats.kernel_launches;
       bs.empty_clusters += ctx->stats.empty_clusters;
       bs.single_call_items++;
+      if (d_labels != nullptr) {
+        dq_colortable_indexes_device(ctx, d_out + offsets[i], n, ct, (int)ks[i], d_labels + offsets[i], 0);
+        launches++;  // map_labels
+      }
     }
   }
-  launches += remap.run(ctx, d_in + base, d_out + base, nullptr);
+  launches += remap.run(ctx, d_in + base, d_out + base, d_labels != nullptr ? d_labels + base : nullptr);
   memset(&ctx->stats, 0, sizeof(ctx->stats));  // (dq_call_stats describes one frame: only the launches are kept)
   ctx->stats.kernel_launches = launches;
   bs.kernel_launches = launches;
@@ -1152,6 +1162,88 @@ void map_colors_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_t *
   ctx->stats.kernel_launches = launches;
   bs.kernel_launches = launches;
   bs.host_palette_ms = (float)host_ms;
+}
+
+// Fatal before any device work: more than 2^24 regions (the sort's three digit passes) and a region asking for K = 0.
+void check_regions_args(uint32_t num_regions, const uint32_t *ks) {
+  if (num_regions > (1u << 24)) {
+    fprintf(stderr, "divquant_b200: %u regions; dq_quant_regions takes at most 2^24\n", num_regions);
+    abort();
+  }
+  for (uint32_t r = 0; r < num_regions; ++r) {
+    if (ks[r] == 0) {
+      fprintf(stderr, "divquant_b200: region %u requests K = 0\n", r);
+      abort();  // assert(num_colors > 0) (:266)
+    }
+  }
+}
+
+// quant_recurse_batch_impl over the regions of a tag image: the pixels partitioned by tag on the device (dq_regions.cu),
+// the regions with pixels quantized as the batch's items in region order, the results scattered back to image layout.
+void quant_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                        uint32_t *d_out, uint32_t *ks, uint32_t *colortables, uint32_t *d_labels) {
+  uint32_t launches = 0, m = 0;
+  const uint2 *sorted = nullptr;
+  uint32_t *g_in = nullptr, *g_out = nullptr, *g_labels = nullptr;
+  ctx->r_offsets.ensure((size_t)num_regions + 1);
+  uint32_t *const off = ctx->r_offsets.ptr;
+  if (n == 0) {
+    memset(off, 0, ((size_t)num_regions + 1) * sizeof(uint32_t));
+  } else {
+    ctx->r_pairs.ensure(2 * (size_t)n);
+    ctx->r_px.ensure((d_labels != nullptr ? 3 : 2) * (size_t)n);
+    ctx->r_scratch.ensure(region_scratch_words(n, num_regions));
+    g_in = ctx->r_px.ptr;
+    g_out = g_in + n;
+    g_labels = d_labels != nullptr ? g_out + n : nullptr;
+    launches += region_partition(d_in, d_tags, n, num_regions, ctx->r_pairs.ptr, g_in, ctx->r_scratch.ptr, &sorted, ctx->stream);
+    DQ_CUDA_CHECK(cudaMemcpyAsync(off, region_offsets(ctx->r_scratch.ptr, n), ((size_t)num_regions + 1) * sizeof(uint32_t),
+                                  cudaMemcpyDeviceToHost, ctx->stream));
+    ctx->wait();
+    m = off[num_regions];
+  }
+  // the regions with pixels, in region order, are the batch's items; their palettes are packed by requested K
+  std::vector<uint32_t> item_off, item_k, item_region;
+  size_t item_pal = 0;
+  for (uint32_t r = 0; r < num_regions; ++r) {
+    if (off[r + 1] == off[r]) continue;
+    item_off.push_back(off[r]);
+    item_k.push_back(ks[r]);
+    item_region.push_back(r);
+    item_pal += ks[r];
+  }
+  item_off.push_back(m);
+  const uint32_t num_items = (uint32_t)item_region.size();
+  std::vector<uint32_t> pal(std::max<size_t>(item_pal, 1));
+  if (num_items > 0) {
+    quant_recurse_batch_impl(ctx, num_items, item_off.data(), g_in, g_out, item_k.data(), pal.data(), 0, g_labels);
+    launches += ctx->batch_stats.kernel_launches;
+  } else {
+    ctx->batch_stats = dq_batch_stats();
+  }
+  // palettes and actual K into the caller's packing (requested K of every region, the empty ones included)
+  size_t at = 0, from = 0;
+  for (uint32_t r = 0, i = 0; r < num_regions; ++r) {
+    const uint32_t requested = ks[r];
+    if (i < num_items && item_region[i] == r) {
+      memcpy(colortables + at, pal.data() + from, item_k[i] * sizeof(uint32_t));
+      from += requested;
+      ks[r] = item_k[i++];
+    } else {
+      ks[r] = 0;
+    }
+    at += requested;
+  }
+  if (m > 0) {
+    region_scatter_back(sorted, m, g_out, g_labels, d_out, d_labels, ctx->stream);
+    launches++;
+    ctx->wait();
+  }
+  dq_batch_stats &bs = ctx->batch_stats;
+  bs.items = num_regions;
+  bs.kernel_launches = launches;
+  memset(&ctx->stats, 0, sizeof(ctx->stats));  // (as after a quant_recurse batch: only the launches are kept)
+  ctx->stats.kernel_launches = launches;
 }
 
 std::mutex g_default_mutex;
@@ -1306,6 +1398,10 @@ void dq_context_destroy(dq_context *ctx) {
   ctx->b_up.release();
   ctx->b_down.release();
   ctx->b_tab.release();
+  ctx->r_pairs.release();
+  ctx->r_px.release();
+  ctx->r_scratch.release();
+  ctx->r_offsets.release();
   cudaFree(ctx->d_table);
   cudaFree(ctx->d_map);
   cudaFree(ctx->d_cb);
@@ -1410,7 +1506,7 @@ void dq_quant_recurse_batch_device(dq_context *ctx, uint32_t num_items, const ui
   if (num_items == 0) return;
   require_device(ctx);
   check_batch_args(num_items, offsets, numPixels, numClusters);
-  quant_recurse_batch_impl(ctx, num_items, offsets, d_in, d_out, numClusters, colortables, allPixelsUnique);
+  quant_recurse_batch_impl(ctx, num_items, offsets, d_in, d_out, numClusters, colortables, allPixelsUnique, nullptr);
 }
 
 void dq_map_colors_batch_device(dq_context *ctx, uint32_t num_items, const uint32_t *offsets, uint32_t numPixels, const uint32_t *d_in,
@@ -1419,6 +1515,14 @@ void dq_map_colors_batch_device(dq_context *ctx, uint32_t num_items, const uint3
   require_device(ctx);
   check_map_batch_args(num_items, offsets, numPixels, colormapSizes, d_labels != nullptr);
   map_colors_batch_impl(ctx, num_items, offsets, d_in, d_out, colormapSizes, colortables, d_labels);
+}
+
+void dq_quant_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                             uint32_t *d_out, uint32_t *ks, uint32_t *colortables, uint32_t *d_labels) {
+  if (num_regions == 0) return;
+  require_device(ctx);
+  check_regions_args(num_regions, ks);
+  quant_regions_impl(ctx, numPixels, d_in, d_tags, num_regions, d_out, ks, colortables, d_labels);
 }
 
 void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out) { *out = ctx->batch_stats; }
@@ -1437,7 +1541,8 @@ void dq_quant_recurse_batch_ctx(dq_context *ctx, uint32_t num_items, const uint3
   ctx->d_in.ensure(total);
   ctx->d_out.ensure(total);
   DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels + base, (size_t)total * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  quant_recurse_batch_impl(ctx, num_items, local.data(), ctx->d_in.ptr, ctx->d_out.ptr, numClusters, colortables, allPixelsUnique);
+  quant_recurse_batch_impl(ctx, num_items, local.data(), ctx->d_in.ptr, ctx->d_out.ptr, numClusters, colortables, allPixelsUnique,
+                           nullptr);
   DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels + base, ctx->d_out.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
 }
@@ -1460,6 +1565,26 @@ void dq_map_colors_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t
   DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels + base, ctx->d_out.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   if (labels != nullptr)
     DQ_CUDA_CHECK(cudaMemcpyAsync(labels + base, ctx->b_labels.ptr, (size_t)total * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+}
+
+void dq_quant_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixels, const uint32_t *tags, uint32_t num_regions,
+                          uint32_t *outPixels, uint32_t *ks, uint32_t *colortables, uint32_t *labels) {
+  if (num_regions == 0) return;
+  require_device(ctx);
+  check_regions_args(num_regions, ks);
+  // d_in = [pixels | tags], d_out = [out | labels]; out and labels go up too, so that pixels in no region keep them
+  const size_t n = numPixels, bytes = n * sizeof(uint32_t);
+  ctx->d_in.ensure(2 * n);
+  ctx->d_out.ensure(2 * n);
+  uint32_t *const d_out = ctx->d_out.ptr, *const d_labels = labels != nullptr ? d_out + n : nullptr;
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr + n, tags, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  DQ_CUDA_CHECK(cudaMemcpyAsync(d_out, outPixels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(d_labels, labels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  quant_regions_impl(ctx, numPixels, ctx->d_in.ptr, ctx->d_in.ptr + n, num_regions, d_out, ks, colortables, d_labels);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels, d_out, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(labels, d_labels, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
 }
 

@@ -87,10 +87,28 @@ void batch_remap_launch(const uint32_t *d_in, uint32_t *d_out, const BatchTile *
                         cudaStream_t st);
 
 // ---- dq_srm.cu ----
+// The stable counting sorts over tiles (SRM's edges, dq_regions.cu's tags) run 256 threads a CTA, one per bin.
+constexpr int kSortThreads = 256;
+// counts[bin][0 .. num_tiles) of num_bins bins: every row scanned (exclusive) in place, its total to row_total[bin]
+void tile_rowscan_launch(uint32_t num_bins, uint32_t num_tiles, uint32_t *counts, uint32_t *row_total, cudaStream_t st);
 uint32_t srm_num_pairs(uint32_t width, uint32_t height);
 size_t srm_scratch_words(uint32_t width, uint32_t height);
 // Returns the number of kernels launched.  d_pairs: 3 words per edge (r1, r2, diff) in merge order.
 int srm_sorted_edges(const uint8_t *d_in, uint32_t width, uint32_t height, uint32_t channels, uint32_t width_step,
                      uint32_t *d_pairs, uint32_t *d_scratch, cudaStream_t st);
+
+// ---- dq_regions.cu: stable partition of a tag image by region (dq_quant_regions_*) ----
+uint32_t region_passes(uint32_t num_regions);  // digit passes of the sort: 1 up to 256 regions, 2 up to 65 536, 3 above
+// d_scratch words for n pixels (n >= 1): per-tile digit counts, digit totals, the num_regions + 1 region offsets
+size_t region_scratch_words(uint32_t n, uint32_t num_regions);
+// Sorts the pixels with tags[p] < num_regions by tag, stable, in d_pairs (2 n pairs, ping-pong); *d_sorted = the m sorted
+// (tag, index) pairs, d_gathered[j] = d_in[index of pair j], region_offsets(d_scratch, n) = num_regions + 1 offsets of the
+// regions in that order (the last is m).  Returns the number of kernels launched.
+int region_partition(const uint32_t *d_in, const uint32_t *d_tags, uint32_t n, uint32_t num_regions, uint2 *d_pairs,
+                     uint32_t *d_gathered, uint32_t *d_scratch, const uint2 **d_sorted, cudaStream_t st);
+const uint32_t *region_offsets(const uint32_t *d_scratch, uint32_t n);
+// d_out[index of pair j] = d_g_out[j] and, with d_labels, d_labels[index] = d_g_labels[j] for j < m (one launch)
+void region_scatter_back(const uint2 *d_sorted, uint32_t m, const uint32_t *d_g_out, const uint32_t *d_g_labels, uint32_t *d_out,
+                         uint32_t *d_labels, cudaStream_t st);
 
 }  // namespace dq

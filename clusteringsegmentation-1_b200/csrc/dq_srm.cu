@@ -9,7 +9,7 @@
 //
 // Three kernels over tiles of 2048 consecutive edges:
 //   count    per-tile histogram of diff                      -> counts[bin][tile]
-//   rowscan  exclusive scan of every bin's row + row total   (one CTA per bin)
+//   rowscan  exclusive scan of every bin's row + row total   (one CTA per bin; tile_rowscan_launch, also dq_regions.cu's)
 //   scatter  rank of an edge = bins before it + same-bin edges of earlier tiles + same-bin edges before it in its
 //            tile (warp match -> per-segment counts -> per-bin running prefix over the tile's 64 segments)
 // 12 bytes written per edge, 2 x 3..4 bytes read per edge and pass (neighbouring reads hit L1/L2).
@@ -18,7 +18,7 @@
 namespace dq {
 namespace {
 
-constexpr int kSrmThreads = 256;
+constexpr int kSrmThreads = kSortThreads;
 constexpr int kSrmSegs = 64;                 // segments of 32 consecutive edges per tile
 constexpr int kSrmTile = 32 * kSrmSegs;      // 2048 edges
 constexpr int kSrmSegsPerWarp = kSrmSegs / (kSrmThreads / 32);
@@ -72,7 +72,7 @@ __global__ void __launch_bounds__(kSrmThreads) srm_count_kernel(const SrmShape s
 }
 
 // one CTA per bin: exclusive scan of counts[bin][0..num_tiles) in place, total to row_total[bin]
-__global__ void __launch_bounds__(kSrmThreads) srm_rowscan_kernel(uint32_t num_tiles, uint32_t *counts, uint32_t *row_total) {
+__global__ void __launch_bounds__(kSrmThreads) tile_rowscan_kernel(uint32_t num_tiles, uint32_t *counts, uint32_t *row_total) {
   __shared__ uint32_t warp_sum[kSrmThreads / 32];
   __shared__ uint32_t carry;
   uint32_t *row = counts + (size_t)blockIdx.x * num_tiles;
@@ -168,6 +168,10 @@ __global__ void __launch_bounds__(kSrmThreads) srm_scatter_kernel(const SrmShape
 
 }  // namespace
 
+void tile_rowscan_launch(uint32_t num_bins, uint32_t num_tiles, uint32_t *counts, uint32_t *row_total, cudaStream_t st) {
+  tile_rowscan_kernel<<<num_bins, kSrmThreads, 0, st>>>(num_tiles, counts, row_total);
+}
+
 uint32_t srm_num_pairs(uint32_t width, uint32_t height) {
   return 2u * (width - 1u) * (height - 1u) + (height - 1u) + (width - 1u);  // srm.c:58
 }
@@ -191,7 +195,7 @@ int srm_sorted_edges(const uint8_t *d_in, uint32_t width, uint32_t height, uint3
   const uint32_t tiles = (s.n_pairs + kSrmTile - 1) / kSrmTile;
   uint32_t *counts = d_scratch, *row_total = d_scratch + (size_t)256 * tiles;
   srm_count_kernel<<<tiles, kSrmThreads, 0, st>>>(s, d_in, tiles, counts);
-  srm_rowscan_kernel<<<256, kSrmThreads, 0, st>>>(tiles, counts, row_total);
+  tile_rowscan_launch(256, tiles, counts, row_total, st);
   srm_scatter_kernel<<<tiles, kSrmThreads, 0, st>>>(s, d_in, tiles, counts, row_total, d_pairs);
   DQ_CUDA_CHECK(cudaGetLastError());
   return 3;

@@ -357,6 +357,32 @@ void dq_map_colors_batch_ctx(dq_context *ctx, uint32_t num_items, const uint32_t
                              const uint32_t *inPixels, uint32_t *outPixels, const int *colormapSizes,
                              const uint32_t *colortables, uint32_t *labels);
 
+/* quant_recurse of every region of a tag image, each region to its own palette (the per-region quant_recurse calls of
+ * ClusteringSegmentation.cpp:758, :1803, :2789, :3152), optionally with the label image of the result.
+ * Region r = the pixels p with tags[p] == r, in index (raster) order; tags[p] >= num_regions = in no region.  With
+ * item_r = in at region r's pixels, every region with pixels gets exactly what dq_quant_recurse_batch_device on this
+ * context returns for the items item_r in region order with the same K (allPixelsUnique = 0): its palette, its actual K,
+ * out at its pixels and the same "# empty clusters: n" lines in the same order.
+ *   ks:          HOST, num_regions words, in = requested K (>= 1 for every region), out = actual K (0 for a region with no
+ *                pixels, which prints nothing and leaves its palette slot untouched).
+ *   colortables: HOST, sum(ks) words; region r's palette starts at the sum of the requested K of regions < r (the batch
+ *                packing).
+ *   out / labels: written at region pixels only; pixels in no region keep what the buffer held.  labels may be NULL; else
+ *                labels[p] = the index of out[p] within its region's returned palette (= dq_colortable_indexes of the
+ *                region's output, asGreyscale = 0).
+ * The device partitions the pixels by tag (a stable radix sort, one pass per byte: up to 256, 65 536, 2^24 regions), then
+ * the regions with pixels go through the quant_recurse batch, and the results are scattered back.  num_regions > 2^24 and
+ * ks[r] == 0 for any r are fatal (message + abort) before any device work; num_regions = 0 does nothing.  d_out and
+ * d_labels must not overlap d_in, d_tags or each other.  The _ctx form copies pixels, tags, out (and labels when asked)
+ * up and out (and labels) down.  Synchronous on return, no timing lines.  Afterwards dq_call_stats is zeroed apart from
+ * kernel_launches; dq_context_last_batch_stats gives items = num_regions, batched_items and single_call_items of the
+ * regions with pixels, empty_clusters, kernel_launches (all the call launched, sort and scatter included) and
+ * host_palette_ms. */
+void dq_quant_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t *d_in, const uint32_t *d_tags,
+                             uint32_t num_regions, uint32_t *d_out, uint32_t *ks, uint32_t *colortables, uint32_t *d_labels);
+void dq_quant_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixels, const uint32_t *tags,
+                          uint32_t num_regions, uint32_t *outPixels, uint32_t *ks, uint32_t *colortables, uint32_t *labels);
+
 /* ------------------------------------------------------------------------------------------------
  * 3. Test hooks (used by tests/ to compare intermediate results with the oracle).
  * ---------------------------------------------------------------------------------------------- */

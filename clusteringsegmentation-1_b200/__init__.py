@@ -101,6 +101,8 @@ def load_library(path=LIB_PATH):
         "dq_map_colors_batch_ctx": (None, [vp, C.c_uint32, _u32p, C.c_uint32, _u32p, _u32p, C.POINTER(C.c_int), _u32p, _u32p]),
         "dq_quant_regions_device": (None, [vp, C.c_uint32, vp, vp, C.c_uint32, vp, _u32p, _u32p, vp]),
         "dq_quant_regions_ctx": (None, [vp, C.c_uint32, _u32p, _u32p, C.c_uint32, _u32p, _u32p, _u32p, _u32p]),
+        "dq_map_regions_device": (None, [vp, C.c_uint32, vp, vp, C.c_uint32, C.POINTER(C.c_int), _u32p, vp, vp]),
+        "dq_map_regions_ctx": (None, [vp, C.c_uint32, _u32p, _u32p, C.c_uint32, C.POINTER(C.c_int), _u32p, _u32p, _u32p]),
         "dq_context_set_split_ctas": (None, [vp, C.c_int]),
         "dq_context_set_exact_small": (None, [vp, C.c_int]),
         "dq_context_set_exact_max_points": (None, [vp, C.c_uint32]),
@@ -159,6 +161,7 @@ EXPORTED_C_SYMBOLS = [
     "dq_pipeline_resolved_frames", "dq_pipeline_rerun_frames",
     "dq_quant_recurse_batch_device", "dq_quant_recurse_batch_ctx", "dq_context_last_batch_stats",
     "dq_map_colors_batch_device", "dq_map_colors_batch_ctx", "dq_quant_regions_device", "dq_quant_regions_ctx",
+    "dq_map_regions_device", "dq_map_regions_ctx",
     "dq_debug_split_points", "dq_debug_histogram", "dq_debug_split_timeline", "dq_host_dedup_palette", "dq_host_build_search_tables", "dq_host_select_cut_overrides",
     "dq_host_build_label_table",
 ]
@@ -329,6 +332,58 @@ class DivQuant:
             self.lib.dq_quant_regions_device(ctx or self.lib.dq_default_context(), pixels.numel(), pixels.data_ptr(), tags.data_ptr(),
                                              nk.size, out.data_ptr(), _p(nk), _p(ct), lab.data_ptr() if labels else None)
         return (out, ct, nk, lab) if labels else (out, ct, nk)
+
+    @staticmethod
+    def _region_palettes(palettes, num_pixels, num_tags, labels):
+        """(sizes, packed palettes) for dq_map_regions_*, after the checks the library would abort on."""
+        if num_tags != num_pixels:
+            raise ValueError("one tag per pixel")
+        if len(palettes) > 1 << 24:
+            raise ValueError(f"{len(palettes)} palettes; at most 2^24 regions")
+        if any(np.ndim(p) != 1 for p in palettes):
+            raise ValueError("one palette (a 1-D array, empty = not mapped) per region")
+        pals = [_u32(p) for p in palettes]
+        sizes = np.asarray([p.size for p in pals], np.int32)
+        if labels and sizes.size and sizes.max() > 24000:
+            raise ValueError("label images support palettes of at most 24000 entries")
+        ct = np.concatenate(pals) if sizes.sum() else np.zeros(1, np.uint32)
+        return sizes, ct
+
+    def map_regions(self, pixels, tags, palettes, labels=False, ctx=None):
+        """map_colors_mps of every region of a tag image, each to its own palette, in one call (dq_map_regions_ctx).
+        Region r is pixels[tags == r] in raster order, mapped to palettes[r] (a uint32 array; an empty one leaves the
+        region unmapped); pixels whose tag is >= len(palettes) are in no region.  Returns out, or (out, labels) with
+        labels=True: out[tags == r] and its labels equal map_colors_batch's result for that region, and pixels in no
+        region or in an unmapped region come back as 0."""
+        px = _u32(pixels)
+        tg = _u32(tags)
+        sizes, ct = self._region_palettes(palettes, px.size, tg.size, labels)
+        out = np.zeros_like(px)
+        lab = np.zeros_like(px) if labels else None
+        if sizes.size:
+            self.lib.dq_map_regions_ctx(ctx or self.lib.dq_default_context(), px.size, _p(px), _p(tg), sizes.size,
+                                        sizes.ctypes.data_as(C.POINTER(C.c_int)), _p(ct), _p(out), _p(lab) if labels else None)
+        return (out, lab) if labels else out
+
+    def map_regions_device(self, pixels, tags, palettes, labels=False, ctx=None, out=None, labels_out=None):
+        """Device form (dq_map_regions_device): `pixels` and `tags` are contiguous CUDA tensors of 32-bit words, one tag
+        per pixel.  Writes out (and labels) at the pixels of mapped regions only: tensors passed as `out` / `labels_out`
+        keep their other pixels (a `labels_out` tensor implies labels=True).  Returns out, or (out, labels), as
+        map_regions."""
+        import torch
+        for t in (pixels, tags):
+            if t.dtype not in (torch.int32, torch.uint32) or not t.is_cuda or not t.is_contiguous():
+                raise ValueError("pixels and tags must be contiguous CUDA tensors of 32-bit words")
+        labels = labels or labels_out is not None
+        sizes, ct = self._region_palettes(palettes, pixels.numel(), tags.numel(), labels)
+        out = torch.zeros_like(pixels) if out is None else out
+        lab = (torch.zeros_like(pixels) if labels_out is None else labels_out) if labels else None
+        if sizes.size:
+            torch.cuda.current_stream(pixels.device).synchronize()  # the library works on its context's stream
+            self.lib.dq_map_regions_device(ctx or self.lib.dq_default_context(), pixels.numel(), pixels.data_ptr(), tags.data_ptr(),
+                                           sizes.size, sizes.ctypes.data_as(C.POINTER(C.c_int)), _p(ct), out.data_ptr(),
+                                           lab.data_ptr() if labels else None)
+        return (out, lab) if labels else out
 
     def last_batch_stats(self, ctx=None):
         st = BatchStats()

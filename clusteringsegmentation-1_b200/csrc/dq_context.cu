@@ -1164,12 +1164,18 @@ void map_colors_batch_impl(dq_context *ctx, uint32_t num_items, const uint32_t *
   bs.host_palette_ms = (float)host_ms;
 }
 
-// Fatal before any device work: more than 2^24 regions (the sort's three digit passes) and a region asking for K = 0.
-void check_regions_args(uint32_t num_regions, const uint32_t *ks) {
+// ---- every region of a tag image in one call (kernels: dq_regions.cu) ------------------------------------------------
+// Fatal before any device work: more than 2^24 regions (the sort's three digit passes).
+void check_region_count(uint32_t num_regions, const char *call) {
   if (num_regions > (1u << 24)) {
-    fprintf(stderr, "divquant_b200: %u regions; dq_quant_regions takes at most 2^24\n", num_regions);
+    fprintf(stderr, "divquant_b200: %u regions; %s takes at most 2^24\n", num_regions, call);
     abort();
   }
+}
+
+// ... and for quant_recurse, a region asking for K = 0.
+void check_regions_args(uint32_t num_regions, const uint32_t *ks) {
+  check_region_count(num_regions, "dq_quant_regions");
   for (uint32_t r = 0; r < num_regions; ++r) {
     if (ks[r] == 0) {
       fprintf(stderr, "divquant_b200: region %u requests K = 0\n", r);
@@ -1178,30 +1184,82 @@ void check_regions_args(uint32_t num_regions, const uint32_t *ks) {
   }
 }
 
-// quant_recurse_batch_impl over the regions of a tag image: the pixels partitioned by tag on the device (dq_regions.cu),
-// the regions with pixels quantized as the batch's items in region order, the results scattered back to image layout.
-void quant_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
-                        uint32_t *d_out, uint32_t *ks, uint32_t *colortables, uint32_t *d_labels) {
-  uint32_t launches = 0, m = 0;
-  const uint2 *sorted = nullptr;
-  uint32_t *g_in = nullptr, *g_out = nullptr, *g_labels = nullptr;
+// ... and for map_colors_mps, a palette of negative size and, with labels, one above dq_colortable_indexes' limit.
+void check_map_regions_args(uint32_t num_regions, const int *sizes, bool labels) {
+  check_region_count(num_regions, "dq_map_regions");
+  for (uint32_t r = 0; r < num_regions; ++r) {
+    if (sizes[r] < 0) {
+      fprintf(stderr, "divquant_b200: region %u has a colortable of %d entries\n", r, sizes[r]);
+      abort();
+    }
+    if (labels && sizes[r] > 24000) {
+      fprintf(stderr, "divquant_b200: region %u has a colortable of %d entries; label images support 1..24000\n", r, sizes[r]);
+      abort();
+    }
+  }
+}
+
+// The pixels of a tag image partitioned by region on the device (dq_regions.cu), which both regions calls work on.
+struct RegionPartition {
+  const uint32_t *off = nullptr;  // HOST, num_regions + 1: region r = sorted positions [off[r], off[r + 1]), off[num_regions] = m
+  uint32_t m = 0, launches = 0;
+  const uint2 *sorted = nullptr;  // the m (tag, index) pairs in region order
+  uint32_t *g_in = nullptr, *g_out = nullptr, *g_labels = nullptr;  // in, out and labels in that order (g_labels: with labels)
+};
+
+// h_dropped: nullptr, or a host bitmap of (num_regions + 31) / 32 words; the pixels of the regions set in it are left out
+// like pixels in no region, so those regions come back with no pixels.
+RegionPartition partition_regions(dq_context *ctx, uint32_t n, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                                  const uint32_t *h_dropped, bool labels) {
+  RegionPartition rp;
   ctx->r_offsets.ensure((size_t)num_regions + 1);
   uint32_t *const off = ctx->r_offsets.ptr;
+  rp.off = off;
   if (n == 0) {
     memset(off, 0, ((size_t)num_regions + 1) * sizeof(uint32_t));
-  } else {
-    ctx->r_pairs.ensure(2 * (size_t)n);
-    ctx->r_px.ensure((d_labels != nullptr ? 3 : 2) * (size_t)n);
-    ctx->r_scratch.ensure(region_scratch_words(n, num_regions));
-    g_in = ctx->r_px.ptr;
-    g_out = g_in + n;
-    g_labels = d_labels != nullptr ? g_out + n : nullptr;
-    launches += region_partition(d_in, d_tags, n, num_regions, ctx->r_pairs.ptr, g_in, ctx->r_scratch.ptr, &sorted, ctx->stream);
-    DQ_CUDA_CHECK(cudaMemcpyAsync(off, region_offsets(ctx->r_scratch.ptr, n), ((size_t)num_regions + 1) * sizeof(uint32_t),
-                                  cudaMemcpyDeviceToHost, ctx->stream));
-    ctx->wait();
-    m = off[num_regions];
+    return rp;
   }
+  const size_t scratch = region_scratch_words(n, num_regions), dropped_words = h_dropped != nullptr ? ((size_t)num_regions + 31) / 32 : 0;
+  ctx->r_pairs.ensure(2 * (size_t)n);
+  ctx->r_px.ensure((labels ? 3 : 2) * (size_t)n);
+  ctx->r_scratch.ensure(scratch + dropped_words);
+  uint32_t *const d_dropped = h_dropped != nullptr ? ctx->r_scratch.ptr + scratch : nullptr;
+  if (d_dropped != nullptr)
+    DQ_CUDA_CHECK(cudaMemcpyAsync(d_dropped, h_dropped, dropped_words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  rp.g_in = ctx->r_px.ptr;
+  rp.g_out = rp.g_in + n;
+  rp.g_labels = labels ? rp.g_out + n : nullptr;
+  rp.launches = region_partition(d_in, d_tags, n, num_regions, d_dropped, ctx->r_pairs.ptr, rp.g_in, ctx->r_scratch.ptr, &rp.sorted,
+                                 ctx->stream);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(off, region_offsets(ctx->r_scratch.ptr, n), ((size_t)num_regions + 1) * sizeof(uint32_t),
+                                cudaMemcpyDeviceToHost, ctx->stream));
+  ctx->wait();
+  rp.m = off[num_regions];
+  return rp;
+}
+
+// The gathered out (and labels) back to image layout at the partitioned pixels, and the call's statistics.
+void finish_regions(dq_context *ctx, const RegionPartition &rp, uint32_t num_regions, uint32_t launches, uint32_t *d_out,
+                    uint32_t *d_labels) {
+  if (rp.m > 0) {
+    region_scatter_back(rp.sorted, rp.m, rp.g_out, rp.g_labels, d_out, d_labels, ctx->stream);
+    launches++;
+    ctx->wait();
+  }
+  dq_batch_stats &bs = ctx->batch_stats;
+  bs.items = num_regions;
+  bs.kernel_launches = launches;
+  memset(&ctx->stats, 0, sizeof(ctx->stats));  // (as after a batch: only the launches are kept)
+  ctx->stats.kernel_launches = launches;
+}
+
+// quant_recurse_batch_impl over the regions of a tag image: the pixels partitioned by tag, the regions with pixels
+// quantized as the batch's items in region order, the results scattered back to image layout.
+void quant_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                        uint32_t *d_out, uint32_t *ks, uint32_t *colortables, uint32_t *d_labels) {
+  const RegionPartition rp = partition_regions(ctx, n, d_in, d_tags, num_regions, nullptr, d_labels != nullptr);
+  const uint32_t *const off = rp.off;
+  uint32_t launches = rp.launches;
   // the regions with pixels, in region order, are the batch's items; their palettes are packed by requested K
   std::vector<uint32_t> item_off, item_k, item_region;
   size_t item_pal = 0;
@@ -1212,11 +1270,11 @@ void quant_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const
     item_region.push_back(r);
     item_pal += ks[r];
   }
-  item_off.push_back(m);
+  item_off.push_back(rp.m);
   const uint32_t num_items = (uint32_t)item_region.size();
   std::vector<uint32_t> pal(std::max<size_t>(item_pal, 1));
   if (num_items > 0) {
-    quant_recurse_batch_impl(ctx, num_items, item_off.data(), g_in, g_out, item_k.data(), pal.data(), 0, g_labels);
+    quant_recurse_batch_impl(ctx, num_items, item_off.data(), rp.g_in, rp.g_out, item_k.data(), pal.data(), 0, rp.g_labels);
     launches += ctx->batch_stats.kernel_launches;
   } else {
     ctx->batch_stats = dq_batch_stats();
@@ -1234,16 +1292,46 @@ void quant_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const
     }
     at += requested;
   }
-  if (m > 0) {
-    region_scatter_back(sorted, m, g_out, g_labels, d_out, d_labels, ctx->stream);
-    launches++;
-    ctx->wait();
+  finish_regions(ctx, rp, num_regions, launches, d_out, d_labels);
+}
+
+// map_colors_batch_impl over the regions of a tag image: the pixels partitioned by tag, the mapped regions with pixels
+// remapped as the batch's items in region order, the results scattered back to image layout.  A region with an empty
+// palette is not mapped: the partition drops its pixels as it drops those in no region, so they are never sorted,
+// gathered or scattered.
+void map_regions_impl(dq_context *ctx, uint32_t n, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                      const int *sizes, const uint32_t *colortables, uint32_t *d_out, uint32_t *d_labels) {
+  std::vector<uint32_t> dropped;  // only when some region is unmapped
+  for (uint32_t r = 0; r < num_regions; ++r) {
+    if (sizes[r] != 0) continue;
+    if (dropped.empty()) dropped.assign(((size_t)num_regions + 31) / 32, 0u);
+    dropped[r >> 5] |= 1u << (r & 31u);
   }
-  dq_batch_stats &bs = ctx->batch_stats;
-  bs.items = num_regions;
-  bs.kernel_launches = launches;
-  memset(&ctx->stats, 0, sizeof(ctx->stats));  // (as after a quant_recurse batch: only the launches are kept)
-  ctx->stats.kernel_launches = launches;
+  const RegionPartition rp = partition_regions(ctx, n, d_in, d_tags, num_regions, dropped.empty() ? nullptr : dropped.data(),
+                                               d_labels != nullptr);
+  const uint32_t *const off = rp.off;
+  uint32_t launches = rp.launches;
+  // the regions with pixels, in region order, are the batch's items, with their palettes packed end to end
+  std::vector<uint32_t> item_off, packed;
+  std::vector<int> item_size;
+  size_t at = 0;
+  for (uint32_t r = 0; r < num_regions; ++r) {
+    const uint32_t *const ct = colortables + at;
+    at += (size_t)sizes[r];
+    if (off[r + 1] == off[r]) continue;
+    item_off.push_back(off[r]);
+    item_size.push_back(sizes[r]);
+    packed.insert(packed.end(), ct, ct + sizes[r]);
+  }
+  item_off.push_back(rp.m);
+  const uint32_t num_items = (uint32_t)item_size.size();
+  if (num_items > 0) {
+    map_colors_batch_impl(ctx, num_items, item_off.data(), rp.g_in, rp.g_out, item_size.data(), packed.data(), rp.g_labels);
+    launches += ctx->batch_stats.kernel_launches;
+  } else {
+    ctx->batch_stats = dq_batch_stats();
+  }
+  finish_regions(ctx, rp, num_regions, launches, d_out, d_labels);
 }
 
 std::mutex g_default_mutex;
@@ -1525,6 +1613,14 @@ void dq_quant_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t
   quant_regions_impl(ctx, numPixels, d_in, d_tags, num_regions, d_out, ks, colortables, d_labels);
 }
 
+void dq_map_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t *d_in, const uint32_t *d_tags, uint32_t num_regions,
+                           const int *colormapSizes, const uint32_t *colortables, uint32_t *d_out, uint32_t *d_labels) {
+  if (num_regions == 0 || numPixels == 0) return;
+  require_device(ctx);
+  check_map_regions_args(num_regions, colormapSizes, d_labels != nullptr);
+  map_regions_impl(ctx, numPixels, d_in, d_tags, num_regions, colormapSizes, colortables, d_out, d_labels);
+}
+
 void dq_context_last_batch_stats(const dq_context *ctx, dq_batch_stats *out) { *out = ctx->batch_stats; }
 
 // ---- host-pointer entry points ----
@@ -1583,6 +1679,26 @@ void dq_quant_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *i
   DQ_CUDA_CHECK(cudaMemcpyAsync(d_out, outPixels, bytes, cudaMemcpyHostToDevice, ctx->stream));
   if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(d_labels, labels, bytes, cudaMemcpyHostToDevice, ctx->stream));
   quant_regions_impl(ctx, numPixels, ctx->d_in.ptr, ctx->d_in.ptr + n, num_regions, d_out, ks, colortables, d_labels);
+  DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels, d_out, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(labels, d_labels, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+}
+
+void dq_map_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixels, const uint32_t *tags, uint32_t num_regions,
+                        const int *colormapSizes, const uint32_t *colortables, uint32_t *outPixels, uint32_t *labels) {
+  if (num_regions == 0 || numPixels == 0) return;
+  require_device(ctx);
+  check_map_regions_args(num_regions, colormapSizes, labels != nullptr);
+  // as dq_quant_regions_ctx: d_in = [pixels | tags], d_out = [out | labels], out and labels up and down
+  const size_t n = numPixels, bytes = n * sizeof(uint32_t);
+  ctx->d_in.ensure(2 * n);
+  ctx->d_out.ensure(2 * n);
+  uint32_t *const d_out = ctx->d_out.ptr, *const d_labels = labels != nullptr ? d_out + n : nullptr;
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr, inPixels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->d_in.ptr + n, tags, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  DQ_CUDA_CHECK(cudaMemcpyAsync(d_out, outPixels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(d_labels, labels, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  map_regions_impl(ctx, numPixels, ctx->d_in.ptr, ctx->d_in.ptr + n, num_regions, colormapSizes, colortables, d_out, d_labels);
   DQ_CUDA_CHECK(cudaMemcpyAsync(outPixels, d_out, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   if (labels != nullptr) DQ_CUDA_CHECK(cudaMemcpyAsync(labels, d_labels, bytes, cudaMemcpyDeviceToHost, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));

@@ -97,15 +97,16 @@ size_t srm_scratch_words(uint32_t width, uint32_t height);
 int srm_sorted_edges(const uint8_t *d_in, uint32_t width, uint32_t height, uint32_t channels, uint32_t width_step,
                      uint32_t *d_pairs, uint32_t *d_scratch, cudaStream_t st);
 
-// ---- dq_regions.cu: stable partition of a tag image by region (dq_quant_regions_*) ----
+// ---- dq_regions.cu: stable partition of a tag image by region (dq_quant_regions_*, dq_map_regions_*) ----
 uint32_t region_passes(uint32_t num_regions);  // digit passes of the sort: 1 up to 256 regions, 2 up to 65 536, 3 above
 // d_scratch words for n pixels (n >= 1): per-tile digit counts, digit totals, the num_regions + 1 region offsets
 size_t region_scratch_words(uint32_t n, uint32_t num_regions);
 // Sorts the pixels with tags[p] < num_regions by tag, stable, in d_pairs (2 n pairs, ping-pong); *d_sorted = the m sorted
 // (tag, index) pairs, d_gathered[j] = d_in[index of pair j], region_offsets(d_scratch, n) = num_regions + 1 offsets of the
-// regions in that order (the last is m).  Returns the number of kernels launched.
-int region_partition(const uint32_t *d_in, const uint32_t *d_tags, uint32_t n, uint32_t num_regions, uint2 *d_pairs,
-                     uint32_t *d_gathered, uint32_t *d_scratch, const uint2 **d_sorted, cudaStream_t st);
+// regions in that order (the last is m).  d_dropped: nullptr, or a bitmap of (num_regions + 31) / 32 words whose set bits
+// mark regions whose pixels are dropped like those in no region.  Returns the number of kernels launched.
+int region_partition(const uint32_t *d_in, const uint32_t *d_tags, uint32_t n, uint32_t num_regions, const uint32_t *d_dropped,
+                     uint2 *d_pairs, uint32_t *d_gathered, uint32_t *d_scratch, const uint2 **d_sorted, cudaStream_t st);
 const uint32_t *region_offsets(const uint32_t *d_scratch, uint32_t n);
 // d_out[index of pair j] = d_g_out[j] and, with d_labels, d_labels[index] = d_g_labels[j] for j < m (one launch)
 void region_scatter_back(const uint2 *d_sorted, uint32_t m, const uint32_t *d_g_out, const uint32_t *d_g_labels, uint32_t *d_out,

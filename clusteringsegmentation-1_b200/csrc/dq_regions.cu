@@ -1,5 +1,6 @@
-// dq_regions.cu -- stable partition of a tag image by region for dq_quant_regions_*: the pixel indexes sorted by tag, the
-// pixels gathered in that order and the region offsets; afterwards the scatter of the quantized pixels and labels back.
+// dq_regions.cu -- stable partition of a tag image by region for dq_quant_regions_* and dq_map_regions_*: the pixel
+// indexes sorted by tag, the pixels gathered in that order and the region offsets; afterwards the scatter of the
+// quantized or mapped pixels and labels back.
 //
 // LSD radix sort of (tag, index) pairs, one pass per byte of the largest tag: 1 pass up to 256 regions, 2 up to 65 536,
 // 3 up to 2^24.  A pass is the stable counting sort of dq_srm.cu over tiles of 2048 consecutive pairs:
@@ -9,9 +10,10 @@
 //            tile (warp match -> per-segment counts -> per-digit running prefix over the tile's 64 segments)
 // Every pass is stable, so region r's pixels come out in raster order: the order the single call and the batch see them
 // in, on which the ordered split's first-seen ties depend.  The first pass reads the tags straight from the image and
-// drops pixels whose tag is >= num_regions, so the later passes sort only the m pixels that lie in a region; they take m
-// from the first pass's digit totals (the host does not know it until the offsets come back).  The last pass also
-// gathers in[index] into sorted order.
+// drops pixels whose tag is >= num_regions or whose region is set in the optional bitmap of dropped regions (the regions
+// dq_map_regions does not map), so the later passes sort only the m pixels that lie in a kept region; they take m from
+// the first pass's digit totals (the host does not know it until the offsets come back).  A dropped region comes out
+// with no pixels.  The last pass also gathers in[index] into sorted order.
 #include "dq_kernels.cuh"
 
 namespace dq {
@@ -26,6 +28,7 @@ struct RegionPass {
   const uint32_t *tags;     // first pass: the tag image
   const uint2 *src;         // later passes: the previous pass's (tag, index) pairs
   const uint32_t *m_total;  // later passes: the first pass's 256 digit totals, whose sum is the number of pairs
+  const uint32_t *dropped;  // first pass: nullptr, or bit r of word r / 32 set = region r's pixels are dropped
   uint32_t n, num_regions, shift;
 };
 
@@ -49,7 +52,7 @@ __device__ __forceinline__ bool load_pair(const RegionPass &p, uint32_t e, uint3
     if (e >= p.n) return false;
     tag = p.tags[e];
     idx = e;
-    return tag < p.num_regions;
+    return tag < p.num_regions && (p.dropped == nullptr || ((p.dropped[tag >> 5] >> (tag & 31u)) & 1u) == 0u);
   }
   if (e >= m) return false;
   const uint2 v = p.src[e];
@@ -173,12 +176,12 @@ size_t region_scratch_words(uint32_t n, uint32_t num_regions) {
   return (size_t)256 * region_tiles(n) + 512 + (size_t)num_regions + 1;
 }
 
-int region_partition(const uint32_t *d_in, const uint32_t *d_tags, uint32_t n, uint32_t num_regions, uint2 *d_pairs,
-                     uint32_t *d_gathered, uint32_t *d_scratch, const uint2 **d_sorted, cudaStream_t st) {
+int region_partition(const uint32_t *d_in, const uint32_t *d_tags, uint32_t n, uint32_t num_regions, const uint32_t *d_dropped,
+                     uint2 *d_pairs, uint32_t *d_gathered, uint32_t *d_scratch, const uint2 **d_sorted, cudaStream_t st) {
   const uint32_t tiles = region_tiles(n), passes = region_passes(num_regions);
   uint32_t *const counts = d_scratch, *const total0 = counts + (size_t)256 * tiles, *const total1 = total0 + 256;
   uint32_t *const offsets = total1 + 256;
-  RegionPass p = {d_tags, nullptr, total0, n, num_regions, 0u};
+  RegionPass p = {d_tags, nullptr, total0, d_dropped, n, num_regions, 0u};
   uint2 *dst = d_pairs;
   for (uint32_t pass = 0; pass < passes; ++pass) {
     const bool first = pass == 0, last = pass + 1 == passes;

@@ -383,6 +383,38 @@ void dq_quant_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t
 void dq_quant_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixels, const uint32_t *tags,
                           uint32_t num_regions, uint32_t *outPixels, uint32_t *ks, uint32_t *colortables, uint32_t *labels);
 
+/* map_colors_mps of every region of a tag image, each region to its own palette (the per-region remaps of
+ * ClusteringSegmentation.cpp:2434, :3816), optionally with the label image of the result (OpenCVUtil.cpp:787-849): the
+ * step after dq_quant_regions once the caller has edited the palettes.
+ * Region r = the pixels p with tags[p] == r, in index (raster) order; tags[p] >= num_regions = in no region.  Region r's
+ * palette is colortables[P_r, P_r + colormapSizes[r]), P_r = the sum of colormapSizes of the regions before r (the map
+ * batch's packing).  Palettes may hold duplicates, alpha bits, equal r+g+b sums and colours absent from the region.
+ *   colormapSizes, colortables: HOST arrays (num_regions and sum of colormapSizes words).  colormapSizes[r] == 0 = region
+ *                r is not mapped: its pixels are treated like pixels in no region (so dq_quant_regions' returned K, 0 for
+ *                a region without pixels, can be passed unchanged).
+ *   out:         at every pixel of region r, bit for bit what dq_map_colors_batch_device on this context returns for the
+ *                item "pixels of region r" (= map_colors_mps of them against that palette): alpha ignored on input, zero
+ *                on output.
+ *   labels:      NULL = none; else labels[p] = what the map batch writes for p: the 0-based index within region r's
+ *                palette of the LAST entry whose 24-bit colour equals out[p].
+ *   Pixels in no region and pixels of unmapped regions keep what out / labels held.
+ * The device partitions the pixels of the mapped regions by tag (the sort of dq_quant_regions; the first pass drops the
+ * unmapped regions' pixels), the regions with pixels go through the map batch as its items in region order, and the
+ * results are scattered back.  A call whose mapped regions all have at most 512 entries launches 3 x passes + 3 kernels
+ * (passes = 1 up to 256 regions, 2 up to 65 536, 3 above), whatever the number of regions, with or without labels.
+ * num_regions > 2^24, colormapSizes[r] < 0 and, with labels, colormapSizes[r] > 24000 are fatal (message + abort) before
+ * any device work; num_regions = 0 or numPixels = 0 does nothing.  d_out and d_labels must not overlap d_in, d_tags or
+ * each other.  The _ctx form copies pixels, tags, out (and labels when asked) up and out (and labels) down.  Synchronous
+ * on return, no timing lines.  Afterwards dq_call_stats is zeroed apart from kernel_launches; dq_context_last_batch_stats
+ * gives items = num_regions, batched_items (palettes <= 512 entries) and single_call_items of the mapped regions with
+ * pixels, empty_clusters = 0, kernel_launches (all the call launched, sort and scatter included) and host_palette_ms. */
+void dq_map_regions_device(dq_context *ctx, uint32_t numPixels, const uint32_t *d_in, const uint32_t *d_tags,
+                           uint32_t num_regions, const int *colormapSizes, const uint32_t *colortables,
+                           uint32_t *d_out, uint32_t *d_labels);
+void dq_map_regions_ctx(dq_context *ctx, uint32_t numPixels, const uint32_t *inPixels, const uint32_t *tags,
+                        uint32_t num_regions, const int *colormapSizes, const uint32_t *colortables,
+                        uint32_t *outPixels, uint32_t *labels);
+
 /* ------------------------------------------------------------------------------------------------
  * 3. Test hooks (used by tests/ to compare intermediate results with the oracle).
  * ---------------------------------------------------------------------------------------------- */

@@ -405,7 +405,7 @@ void run_split(dq_context *ctx, SplitRun run) {
       if (a.mailbox_seq == 0) a.mailbox_seq = ++ctx->mailbox_seq;  // 0 is the idle value
     }
     // the ordered path always runs inside this kernel: its plan makes room for it in the dynamic shared memory
-    const SplitLaunch plan = split2_plan(ctx->split_ctas, ctx->sm_count, K, exact_path);
+    const SplitLaunch plan = split2_plan(ctx->split_ctas, ctx->sm_count, K);
     if (exact_path) {
       x.exact_fused = (ctx->exact_parallel && plan.grid > 1) ? 2 : 1;
       x.exact_src = sampling;
@@ -2146,7 +2146,10 @@ dq_pipeline *dq_pipeline_create_lanes(int device, uint32_t max_pixels, int lanes
     // histogram / remap kernels, which cannot share an SM with a split CTA (it owns the register file).  Measured at
     // 4K, 12 lanes, with the chunked histogram (tools/lanes_check.py, B200): 8 CTAs each 0.158 ms/frame, 9: 0.153,
     // 10: 0.154, 11: 0.156; 1080p K = 64: 8: 0.100, 9: 0.095, 10: 0.094, 11: 0.093.  Before the chunked histogram the
-    // best was 8 CTAs (11/16): more split SMs left it too few free SMs to keep enough L2 atomics in flight.
+    // best was 8 CTAs (11/16): more split SMs left it too few free SMs to keep enough L2 atomics in flight.  With the
+    // wide-job points kept in shared memory (B200, 1000 W; 4K, 960 frames, two runs): 12 lanes x 8 CTAs 0.129 ms/frame,
+    // x 9: 0.128-0.129, x 10: 0.135-0.136; 16 x 6: 0.122-0.123, 16 x 7: 0.129.  The shorter split did not move the best
+    // partition.
     if (split_ctas <= 0) split_ctas = std::max(split2_max_ctas(lane.ctx->sm_count, 256) * 3 / 4 / lanes, lanes > 1 ? 4 : 1);
     if (lanes == 1) split_ctas = 0;  // a single lane is a single call: all SMs
     dq_context_set_split_ctas(lane.ctx, split_ctas);

@@ -238,9 +238,12 @@ struct Split2Extra {
   unsigned char *exact_scratch;  // split_exact_scratch_bytes()
   double *exact_f64;   // 8*K doubles
   int32_t *exact_i32;  // K ints
+  // points of a CTA's wide-job shares that the round's cut pass keeps in the dynamic shared memory behind the integer path's
+  // arrays, so that its later passes and the partition do not read them from L2 again (set by split2_launch from the plan)
+  uint32_t wide_cache_points;
 };
 size_t split2_slot_capacity(uint32_t point_capacity, uint32_t num_colors, int sm_count);
-SplitLaunch split2_plan(int requested_ctas, int sm_count, uint32_t num_colors, bool exact_fused = false);
+SplitLaunch split2_plan(int requested_ctas, int sm_count, uint32_t num_colors);
 int split2_max_ctas(int sm_count, uint32_t num_colors);
 void split2_launch(const SplitArgs &args, const Split2Extra &extra, const SplitLaunch &plan, cudaStream_t stream);
 

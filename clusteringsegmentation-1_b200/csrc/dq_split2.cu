@@ -36,7 +36,6 @@ namespace {
 constexpr int kWarps = 16;
 constexpr int T = 32 * kWarps;  // 16 warps, up to 128 registers per thread: points stay in registers without spills
 constexpr uint32_t kWideTile = 1024;  // points per wide tile
-constexpr int kWidePPT = 2;           // points per thread when a CTA classifies its share of a wide job
 constexpr int kNarrowPPT = 8;         // points per thread of a narrow job (kept in registers for all passes)
 constexpr uint32_t kNarrowMax = kNarrowPPT * T;
 constexpr int kGroupWarps = 8;                 // warps of a narrow-job group
@@ -137,6 +136,9 @@ struct Arrays {
   // so these two live in their memory.
   uint64_t (*wprev)[4];  // [K]  {cnt, R, G, B} of the last pass gathered (in rank[], cap * 4 >= K * 32 bytes)
   int32_t *wfin;         // [K]  1 + the pass that ran as the job's final one, 0 while it runs (in cand[])
+  // [Split2Extra::wide_cache_points] this CTA's shares of the round's wide jobs, back to back in mywide order, as far as they
+  // fit: written by the cut pass, read by the later passes and the partition of the same round
+  uint2 *wcache;
 };
 
 __device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long *p) {
@@ -984,45 +986,43 @@ __device__ __forceinline__ unsigned narrow_pass(St &S, const uint2 (&p)[kNarrowP
   return newmask;
 }
 
-// This CTA's share of a wide job in one pass: partial sums into v[].
-template <bool SPLIT, bool FINAL, typename OffsetFn>
-__device__ __forceinline__ void wide_classify(const PassParams &pp, const tie::PassExt *ext, const uint2 (&pre)[kWidePPT], uint32_t n_my, uint32_t nthr,
-                                              const uint2 *seg, OffsetFn offset_of, uint64_t (&v)[kAccWords]) {
+// This CTA's share of a wide job in one pass, seg[0 .. n_my): partial sums into v[].  Thread tid takes points
+// tid + k * nthr, the same ones in every pass.  The first n_cached points live in cache[] for the rest of the round: the
+// cut pass (SPLIT) loads every point from L2 and stores those, later passes read them back -- each thread only what it
+// stored itself, so no barrier is needed -- and only the remainder comes from L2 again, four loads in flight per trip.
+template <bool SPLIT, bool FINAL>
+__device__ __forceinline__ void wide_classify(const PassParams &pp, const tie::PassExt *ext, uint32_t n_my, uint32_t nthr,
+                                              const uint2 *seg, uint2 *cache, uint32_t n_cached, uint64_t (&v)[kAccWords]) {
   AccD acc = acc_zero();
   bool near = false;
   const uint32_t tid = threadIdx.x;
   if (tid < nthr) {
-#pragma unroll
-    for (int k = 0; k < kWidePPT; ++k) {
-      const uint32_t q = tid + (uint32_t)k * nthr;
-      if (q < n_my) {
-        if (goes_new_audit<SPLIT>(pp, ext, to_point(pre[k]), near)) acc_add(acc, pre[k], FINAL);
+    uint32_t q = tid;
+    if (!SPLIT) {
+#pragma unroll 4
+      for (; q < n_cached; q += nthr) {
+        const uint2 p = cache[q];
+        if (goes_new_audit<SPLIT>(pp, ext, to_point(p), near)) acc_add(acc, p, FINAL);
       }
     }
-    // beyond the register-resident points (few CTAs per frame): four loads in flight per trip
-    for (uint32_t q = tid + kWidePPT * nthr; q < n_my; q += 4u * nthr) {
+    for (; q < n_my; q += 4u * nthr) {
       uint2 raw[4];
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         const uint32_t qq = q + (uint32_t)u * nthr;
-        raw[u] = (qq < n_my) ? ld_cg_u2(seg + offset_of(qq)) : make_uint2(0u, 0u);
+        raw[u] = (qq < n_my) ? ld_cg_u2(seg + qq) : make_uint2(0u, 0u);
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
-        if (q + (uint32_t)u * nthr < n_my && goes_new_audit<SPLIT>(pp, ext, to_point(raw[u]), near)) acc_add(acc, raw[u], FINAL);
+        const uint32_t qq = q + (uint32_t)u * nthr;
+        if (SPLIT && qq < n_cached) cache[qq] = raw[u];
+        if (qq < n_my && goes_new_audit<SPLIT>(pp, ext, to_point(raw[u]), near)) acc_add(acc, raw[u], FINAL);
       }
     }
   }
-  if (near) {  // some point passed the audit's integer filter: settle it with the real test (cold)
+  if (near) {  // some point passed the audit's integer filter: settle it with the real test (cold; L2 holds the same bytes)
     near = false;
-    for (uint32_t q = tid; q < n_my; q += nthr) {
-      const uint2 raw = (q < kWidePPT * nthr) ? pre[0] : ld_cg_u2(seg + offset_of(q));
-      uint2 pt = raw;
-#pragma unroll
-      for (int k = 0; k < kWidePPT; ++k)
-        if (q == tid + (uint32_t)k * nthr) pt = pre[k];
-      near = near || recheck_near<SPLIT>(pp, ext, to_point(pt));
-    }
+    for (uint32_t q = tid; q < n_my; q += nthr) near = near || recheck_near<SPLIT>(pp, ext, to_point(ld_cg_u2(seg + q)));
   }
   acc_words(acc, v);
   v[kAccPts] += (uint64_t)near << 32;  // tie audit (split_near_warp0)
@@ -1102,6 +1102,18 @@ __device__ __forceinline__ void narrow_job(const SplitArgs &A, const Shared2 &S,
   sync();
 }
 
+// Dynamic shared memory of the integer path (Shared2 + the arrays of Arrays), 16-B aligned.  The wide-point cache
+// (Split2Extra::wide_cache_points) starts at this offset and takes whatever the launch reserves beyond it.
+__host__ __device__ size_t split2_smem_bytes(uint32_t K, uint32_t cap) {
+  size_t s = (sizeof(Shared2) + 15) & ~size_t(15);
+  s += (size_t)cap * (8 + 4 + 4 + 4 + 4);
+  s += (size_t)K * (8 + 4 + 4 + 4);
+  s += (size_t)(K + 1) * 4 * 3;
+  s += (size_t)K * 2 * 2;
+  s += (size_t)K + 16 + (size_t)cap * (8 + 4);  // tie audit: jobtie, terr, byrank
+  return (s + 64 + 15) & ~size_t(15);
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // The kernel
 // ---------------------------------------------------------------------------------------------------------
@@ -1151,6 +1163,7 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
     R.terr = reinterpret_cast<double *>(cur);
     cur += (size_t)cap * 8;
     R.byrank = reinterpret_cast<int32_t *>(cur);
+    R.wcache = reinterpret_cast<uint2 *>(smem_raw + split2_smem_bytes((uint32_t)K, cap));
   }
   const bool audit = A.tie_audit != 0u;
 
@@ -1450,9 +1463,8 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
     DQ_PROGRESS(round * 10000 + 1000 + n_mywide * 10 + n_mynarrow);
 
     // ================= wide jobs: all passes, partial sums exchanged through tagged slots =================
-    // A CTA's share of a wide job = a contiguous run of its kWideTile-point tiles.  It is classified by as few
-    // warps as possible (kWidePPT points per thread): the warp reductions, not the arithmetic, are what a
-    // pass costs, so fewer, busier warps are faster.
+    // A CTA's share of a wide job = a contiguous run of its kWideTile-point tiles, classified by the warps it has
+    // points for (wide_classify).
     const unsigned seq0 = 1u + (unsigned)round * (unsigned)(P + 1);
     auto wide_const = [&](int mw) -> JobConst {
       if (mw < kWideCache) return S.wide[mw];
@@ -1473,23 +1485,10 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       sh.n_my = min(hi * kWideTile, size) - sh.first_point;
       return sh;
     };
-    // The points of a CTA's share do not change during a round: with a single wide job (the common case) they
-    // are loaded once and stay in registers for all passes.
-    uint2 pre0[kWidePPT];
-    const bool single_wide = (n_mywide == 1);
-    if (single_wide) {
-      const int j = R.mywide[0];
-      const JobConst jc = wide_const(0);
-      const Share sh = share_of(j, jc.size);
-      const uint32_t n_my = sh.n_my;
-      const uint32_t nthr = min((uint32_t)T, (n_my + 31u) & ~31u);
-#pragma unroll
-      for (int k = 0; k < kWidePPT; ++k) {
-        const uint32_t q = (uint32_t)tid + (uint32_t)k * nthr;
-        pre0[k] = make_uint2(0, 0);
-        if ((uint32_t)tid < nthr && q < n_my) pre0[k] = ld_cg_u2(A.pts[jc.buf] + jc.begin + sh.first_point + q);
-      }
-    }
+    // The points of a CTA's shares do not change during a round: the cut pass puts them into R.wcache, back to back
+    // in mywide order (job mw from `base` on), and the later passes and the partition read the first n_cached of each share
+    // from there.  Only what does not fit (few CTAs per frame, large K) is read from L2 in every pass.
+    auto n_cached_of = [&](uint32_t base, uint32_t n_my) { return X.wide_cache_points > base ? min(n_my, X.wide_cache_points - base) : 0u; };
     // Fixed-point exit: every participant gathers the same totals, so each of them finds on its own
     // that {cnt, R, G, B} repeat the previous pass's -- the next parameters, and so every later classification, repeat
     // that pass exactly -- and runs this pass as the final one, as a narrow job does.  The participants therefore all
@@ -1499,26 +1498,19 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
     for (int pass = 0; pass <= P && n_running > 0; ++pass) {
       unsigned long long *slots_w = X.slots + (size_t)(pass & 1) * X.slot_cap * kAccWords;
       const unsigned long long *slots_r = X.slots + (size_t)((pass & 1) ^ 1) * X.slot_cap * kAccWords;
+      uint32_t base = 0;
       for (int mw = 0; mw < n_mywide; ++mw) {
-        if (R.wfin[mw] != 0) continue;
         const int j = R.mywide[mw];
+        const Share sh = share_of(j, R.size[R.jobnode[j]]);
+        const uint32_t n_cached = n_cached_of(base, sh.n_my);
+        uint2 *const cache = R.wcache + base;
+        base += sh.n_my;
+        if (R.wfin[mw] != 0) continue;
         const JobConst jc = wide_const(mw);
-        const Share sh = share_of(j, jc.size);
         const int m = (int)sh.m;
         const uint32_t me = sh.me;
         const uint32_t n_my = sh.n_my;
         const uint32_t nthr = min((uint32_t)T, (n_my + 31u) & ~31u);  // spread over as many warps as there are points for
-        // prefetch the first points of this CTA's share while the previous pass's totals arrive
-        uint2 pre[kWidePPT];
-#pragma unroll
-        for (int k = 0; k < kWidePPT; ++k) {
-          const uint32_t q = (uint32_t)tid + (uint32_t)k * nthr;
-          pre[k] = pre0[k];
-          if (!single_wide) {
-            pre[k] = make_uint2(0, 0);
-            if ((uint32_t)tid < nthr && q < n_my) pre[k] = ld_cg_u2(A.pts[jc.buf] + jc.begin + sh.first_point + q);
-          }
-        }
 #ifdef DQ_PROFILE_NARROW
         const long long w0 = clock64();
         long long w1 = w0;
@@ -1552,11 +1544,10 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
         const PassParams pp = S.pp;
         uint64_t v[kAccWords];
         {
-          const uint2 *seg = A.pts[jc.buf] + jc.begin;
-          auto off = [&](uint32_t q) { return sh.first_point + q; };
-          if (pass == 0) wide_classify<true, false>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
-          else if (fin) wide_classify<false, true>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
-          else wide_classify<false, false>(pp, &S.ext, pre, n_my, nthr, seg, off, v);
+          const uint2 *seg = A.pts[jc.buf] + jc.begin + sh.first_point;
+          if (pass == 0) wide_classify<true, false>(pp, &S.ext, n_my, nthr, seg, cache, n_cached, v);
+          else if (fin) wide_classify<false, true>(pp, &S.ext, n_my, nthr, seg, cache, n_cached, v);
+          else wide_classify<false, false>(pp, &S.ext, n_my, nthr, seg, cache, n_cached, v);
         }
 #ifdef DQ_PROFILE_NARROW
         const long long w3 = clock64();
@@ -1611,10 +1602,14 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       DQ_PROGRESS(round * 10000 + 2000 + pass);
     }
     // partition of the wide jobs + children
+    uint32_t base = 0;
     for (int mw = 0; mw < n_mywide; ++mw) {
       const int j = R.mywide[mw];
       const JobConst jc = wide_const(mw);
       const Share sh = share_of(j, jc.size);
+      const uint32_t n_cached = n_cached_of(base, sh.n_my);
+      const uint2 *const cache = R.wcache + base;
+      base += sh.n_my;
       const int m = (int)sh.m;
       const uint32_t me = sh.me;
       const int pf = R.wfin[mw] - 1;  // the job's final pass
@@ -1653,13 +1648,16 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
       }
       uint32_t run_new = S.base_new, run_old = S.base_old;
       int flip = 0;
+      // (the cache was written by other threads in the cut pass: the barriers since then order it)
+      const uint2 *seg = A.pts[jc.buf] + jc.begin + sh.first_point;
+      auto point = [&](uint32_t q) { return q < n_cached ? cache[q] : ld_cg_u2(seg + q); };
       uint2 p_next = make_uint2(0, 0);
-      if ((uint32_t)tid < sh.n_my) p_next = ld_cg_u2(A.pts[jc.buf] + jc.begin + sh.first_point + tid);
+      if ((uint32_t)tid < sh.n_my) p_next = point(tid);
       for (uint32_t piece = 0; piece < sh.n_my; piece += T) {
         // T-point pieces of this CTA's (contiguous) share, in order; the next piece's points are already on their way
         const bool valid = piece + tid < sh.n_my;
         const uint2 p = p_next;
-        if (piece + T + tid < sh.n_my) p_next = ld_cg_u2(A.pts[jc.buf] + jc.begin + sh.first_point + piece + T + tid);
+        if (piece + T + tid < sh.n_my) p_next = point(piece + T + tid);
         const bool to_new = valid && goes_new(pp, false, p.x);
         const unsigned m_new = __ballot_sync(0xffffffffu, to_new);
         const unsigned m_old = __ballot_sync(0xffffffffu, valid && !to_new);
@@ -1732,16 +1730,6 @@ __global__ void __launch_bounds__(T, 65536 / (128 * T)) split2_kernel(const Spli
   }
 }
 
-size_t split2_smem_bytes(uint32_t K, uint32_t cap) {
-  size_t s = (sizeof(Shared2) + 15) & ~size_t(15);
-  s += (size_t)cap * (8 + 4 + 4 + 4 + 4);
-  s += (size_t)K * (8 + 4 + 4 + 4);
-  s += (size_t)(K + 1) * 4 * 3;
-  s += (size_t)K * 2 * 2;
-  s += (size_t)K + 16 + (size_t)cap * (8 + 4);  // tie audit: jobtie, terr, byrank
-  return s + 64;
-}
-
 }  // namespace
 
 size_t split2_slot_capacity(uint32_t point_capacity, uint32_t num_colors, int sm_count) {
@@ -1769,13 +1757,15 @@ int split2_max_ctas(int sm_count, uint32_t num_colors) {
   return it->second * sm_count;
 }
 
-SplitLaunch split2_plan(int requested_ctas, int sm_count, uint32_t num_colors, bool exact_fused) {
+SplitLaunch split2_plan(int requested_ctas, int sm_count, uint32_t num_colors) {
   SplitLaunch plan;
   const int cap = split2_max_ctas(sm_count, num_colors);
   plan.grid = (requested_ctas >= 1 && requested_ctas <= cap) ? requested_ctas : cap;
-  plan.smem_bytes = split2_smem_bytes(num_colors, 8 * num_colors + 16);
-  // the small-input body lives in the same dynamic shared memory (one CTA per SM either way: 128 registers x 512)
-  if (exact_fused) plan.smem_bytes = std::max(plan.smem_bytes, split_exact_smem_bytes());
+  // The small-input body lives in the same dynamic shared memory, and the integer path keeps its wide-job points in what
+  // that body needs beyond the integer path's own arrays (one CTA per SM either way: 128 registers x 512).  Every launch
+  // reserves it, fused small-input body or not.  (Not more: crossing the 196 KB carve-out step costs the frame pipeline
+  // 10-40 %, DESIGN 5.5.)
+  plan.smem_bytes = std::max(split2_smem_bytes(num_colors, 8 * num_colors + 16), split_exact_smem_bytes());
   return plan;
 }
 
@@ -1784,6 +1774,8 @@ void split2_launch(const SplitArgs &args_in, const Split2Extra &extra, const Spl
   args.node_cap = 8 * args.num_colors + 16;
   (void)split2_max_ctas(1, args.num_colors);  // raises the kernel's dynamic shared memory limit once
   Split2Extra x = extra;
+  const size_t arrays = split2_smem_bytes(args.num_colors, args.node_cap);
+  x.wide_cache_points = plan.smem_bytes > arrays ? (uint32_t)((plan.smem_bytes - arrays) / sizeof(uint2)) : 0u;
   void *kargs[] = {(void *)&args, (void *)&x};
   DQ_CUDA_CHECK(cudaLaunchCooperativeKernel((const void *)split2_kernel, dim3(plan.grid), dim3(T), kargs, plan.smem_bytes, stream));
 }

@@ -120,18 +120,11 @@ struct dq_context {
   DevBuf<int4> d_pal_scratch;
   DevBuf<unsigned long long> d_timeline;
   DevBuf<unsigned long long> d_slots;
-  DevBuf<uint32_t> d_cursors;
   DevBuf<uint32_t> d_progress;
   int exact_small = 1;    // small weighted inputs take the sequential-order kernel (DIVQUANT_B200_EXACT_SMALL=0 turns it off)
-  int exact_parallel = 1;  // the ordered path runs on all CTAs of the split kernel (DIVQUANT_B200_EXACT_PARALLEL=0: CTA 0 only)
   uint32_t exact_max_points = kExactDefaultPoints;  // ... up to this many unique colours (DIVQUANT_B200_EXACT_MAX)
   DevBuf<uint64_t> d_exact;
   DevBuf<uint32_t> d_tie;  // flagged clusters / nodes, resolver status words, a counter (layout: dq_split.cuh, kTieListWords)
-  // a split that has been launched but whose palette has not been collected yet (run_split / run_split_finish)
-  struct PendingSplit {
-    SplitArgs a;
-    bool use_v2 = false, unaudited = false;
-  } pend;
   // A quantize call between its two halves (quantize_begin / quantize_finish): the one description of its split, from
   // which every run of the split kernel takes its inputs and outputs (run_split).
   struct QuantState {
@@ -145,7 +138,16 @@ struct dq_context {
     dq_split_record *records = nullptr;
     double *mean_out = nullptr;
     uint32_t *size_out = nullptr;
-    int phase = 0;  // quantize_step
+    // the paths of the call, fixed before its first run (plan_paths)
+    bool v2 = false;        // the latency-optimised split kernel (K <= kSplit2MaxColors); else the generic one
+    bool audited = false;   // the split audits its decisions against the reference's rounding noise (dq_tie.cuh)
+    bool report_unaudited = false;  // weighted and not audited: a run beyond its ordered-path limit reports kTieUnaudited
+    uint32_t exact_limit = 0;  // points up to which a run takes the ordered path (0: never); the ordered re-run: kExactMaxPoints
+    bool mailbox = false;   // the palette comes back through the mapped mailbox (else stream wait + copies)
+    bool resolve_ok = false;  // a flagged frame may go to the tie resolver (quantize_step checks its flags and lists)
+    bool rerun_ok = false;    // ... or be computed again on the ordered path (if it has at most kExactMaxPoints points)
+    SplitArgs split;          // the split launched last, whose palette run_split_finish collects
+    enum class Step { kSplit, kResolve, kResolveLarge, kOrdered } step = Step::kSplit;  // what quantize_step waits for next
     uint32_t flags = 0, flags_all = 0, tie_count = 0, cut_count = 0, k_first = 0, resplits = 0;
     CutOverride h_ovr[kCutOverrideCap];  // forced cuts of the next run (SplitRun::kForcedCuts)
     uint32_t n_ovr = 0;
@@ -162,7 +164,6 @@ struct dq_context {
   int tie_policy = 2;
   int resolve_mode = 3;  // bit 0: the resolver's shared-memory form, bit 1: its large form (DIVQUANT_B200_RESOLVE; testing)
   long long spin_cycles = 0;  // DIVQUANT_B200_SPIN_MS: bound of the split kernel's waits on other CTAs (0 = built-in 0.2 s)
-  int split_version = 2;  // 1 = generic kernel, 2 = latency-optimised kernel (falls back to 1 when it cannot run)
   int trace_split = 0;
   int profile_narrow = 0;  // DQ_PROFILE_NARROW set: the cycle counters of a -DDQ_PROFILE_NARROW build to stderr after every split
   int *d_lut = nullptr;
@@ -196,7 +197,6 @@ struct dq_context {
   DevBuf<uint2> r_pairs;
   DevBuf<uint32_t> r_px, r_scratch;
   PinnedBuf r_offsets;
-  int use_mailbox = 1;  // DIVQUANT_B200_MAILBOX=0: always wait for the stream and copy
   void wait() {
     if (!blocking_wait) {
       DQ_CUDA_CHECK(cudaStreamSynchronize(stream));
@@ -294,16 +294,36 @@ void reset_control(dq_context *ctx) {
 // can hold goes there), or the re-run with the resolver's forced cuts (QuantState::h_ovr).
 enum class SplitRun { kFirst, kOrdered, kForcedCuts };
 
+// Decides, once before the first run of the call that ctx->qs describes, the paths that stay fixed for the whole call:
+// the split kernel, its tie audit, the ordered path's limit, how the palette comes back, and which recovery steps a
+// flagged frame may take (quantize_step).
+void plan_paths(dq_context *ctx) {
+  dq_context::QuantState &q = ctx->qs;
+  // a histogram is weighted; one of the pixels in q.d_in also gives the ordered path its input (a merged one has no
+  // pixels here)
+  const bool hist = q.table_dirty, pixels = hist && q.merged.colours == nullptr;
+  const bool settle = ctx->tie_policy == 2 && hist && ctx->exact_small;
+  q.v2 = q.K <= kSplit2MaxColors;
+  q.audited = hist && q.v2 && ctx->tie_policy != 0;
+  q.report_unaudited = hist && !q.audited && ctx->tie_policy != 0;
+  q.exact_limit = 0;
+  if (pixels && q.K <= kExactMaxColors && ctx->exact_small && ctx->exact_max_points > 0)
+    // the generic kernel carries no tie audit: everything the ordered path can hold goes there
+    q.exact_limit = (!q.v2 && ctx->tie_policy != 0) ? kExactMaxPoints : ctx->exact_max_points;
+  q.mailbox = q.v2 && !ctx->blocking_wait && !ctx->trace_split && q.records == nullptr && q.mean_out == nullptr &&
+              q.size_out == nullptr;
+  q.resolve_ok = settle && q.records == nullptr && q.mean_out == nullptr;
+  q.rerun_ok = settle && q.v2 && pixels;
+}
+
 // Queues the divisive phase that ctx->qs describes, on its points: the histogram in the direct table and d_uniq
 // (q.table_dirty), or ctx->d_pts0[0..U).  U is read on the device from d_cb->ucount.  Nothing is waited for: the caller
 // polls split_ready() and collects the palette with run_split_finish().
 void run_split(dq_context *ctx, SplitRun run) {
-  const dq_context::QuantState &q = ctx->qs;
+  dq_context::QuantState &q = ctx->qs;
   const uint32_t K = q.K, point_capacity = q.point_cap;
   const int max_iters = q.max_iters;
-  // a histogram is collected by the split kernel and weighted; one of the pixels in q.d_in also gives the ordered path
-  // its input (a merged one has no pixels here)
-  const bool hist = q.table_dirty, pixels = hist && q.merged.colours == nullptr;
+  const bool hist = q.table_dirty;  // (collected by the split kernel)
   if (max_iters < 1 || max_iters > kSplitMaxIters) {
     fprintf(stderr, "divquant_b200: max_iters ( %d ) must be in [1,%d] (the reference hard-wires local k-means on)\n",
             max_iters, kSplitMaxIters);
@@ -352,10 +372,8 @@ void run_split(dq_context *ctx, SplitRun run) {
     a.timeline_cap = 8192;
   }
 
-  const bool use_v2 = ctx->split_version == 2 && K <= kSplit2MaxColors;
-  // weighted points on exact-integer sums: audit the decisions against the reference's rounding noise (dq_tie.cuh)
   a.spin_cycles = ctx->spin_cycles;
-  a.tie_audit = (hist && use_v2 && ctx->tie_policy != 0) ? 1u : 0u;
+  a.tie_audit = q.audited ? 1u : 0u;
   if (a.tie_audit) {
     ctx->d_tie.ensure(kTieListWords);
     a.tie_list = ctx->d_tie.ptr;
@@ -365,39 +383,33 @@ void run_split(dq_context *ctx, SplitRun run) {
     }
   }
   ctx->mark(2);
-  const uint32_t max_points = run == SplitRun::kOrdered ? kExactMaxPoints : ctx->exact_max_points;
-  const bool exact_path = pixels && K <= kExactMaxColors && ctx->exact_small && max_points > 0;
+  // (the ordered re-run is only queued when q.rerun_ok, which implies every condition of q.exact_limit)
+  const bool exact_path = run == SplitRun::kOrdered || q.exact_limit > 0;
   ExactSampling sampling;
   memset(&sampling, 0, sizeof(sampling));
   if (exact_path) {
     // small inputs: the reference's own summation order (dq_split_exact.cuh); large ones take one branch
     ctx->d_ctl_f64.ensure((size_t)8 * K + node_cap + 16);
     a.g_cluster_tse = ctx->d_ctl_f64.ptr;
-    a.exact_small_max = std::min<uint32_t>(max_points, kExactMaxPoints);
-    // the generic kernel (K > kSplit2MaxColors) carries no tie audit: everything the ordered path can hold goes there
-    if (!use_v2 && ctx->tie_policy != 0) a.exact_small_max = kExactMaxPoints;
+    a.exact_small_max = run == SplitRun::kOrdered ? kExactMaxPoints : q.exact_limit;
     ctx->d_exact.ensure((split_exact_scratch_bytes() + ((size_t)8 * K + 16 + 64) * sizeof(uint32_t)) / 8 + 2);
     sampling = exact_sampling(q.d_in, q.rows, q.cols, (uint32_t)q.dec, q.num_bits);
   }
-  if (use_v2) {
+  if (q.v2) {
     Split2Extra x;
     memset(&x, 0, sizeof(x));
     const size_t slot_cap = split2_slot_capacity(point_capacity, K, ctx->sm_count);
     ctx->d_slots.ensure(2 * slot_cap * kAccWords);
-    ctx->d_cursors.ensure((size_t)4 * K);
     ctx->d_nodes.ensure((size_t)8 * K + 16);
     a.nodes = ctx->d_nodes.ptr;
     x.slots = ctx->d_slots.ptr;
     x.slot_cap = (uint32_t)slot_cap;
-    x.cursors = ctx->d_cursors.ptr;
     ctx->d_progress.ensure(1024);
     x.progress = ctx->d_progress.ptr;
     x.collect_uniq = hist ? ctx->d_uniq.ptr : nullptr;
     x.collect_table = hist ? ctx->d_table : nullptr;
     if (ctx->profile_narrow) DQ_CUDA_CHECK(cudaMemsetAsync(ctx->d_progress.ptr, 0, 1024 * sizeof(uint32_t), ctx->stream));
-    const bool mail = ctx->use_mailbox && !ctx->blocking_wait && !ctx->trace_split && q.records == nullptr &&
-                      q.mean_out == nullptr && q.size_out == nullptr;
-    if (mail) {
+    if (q.mailbox) {
       void *dev = nullptr;
       DQ_CUDA_CHECK(cudaHostGetDevicePointer(&dev, const_cast<uint32_t *>(ctx->mailbox), 0));
       a.mailbox = static_cast<uint32_t *>(dev);
@@ -407,7 +419,7 @@ void run_split(dq_context *ctx, SplitRun run) {
     // the ordered path always runs inside this kernel: its plan makes room for it in the dynamic shared memory
     const SplitLaunch plan = split2_plan(ctx->split_ctas, ctx->sm_count, K);
     if (exact_path) {
-      x.exact_fused = (ctx->exact_parallel && plan.grid > 1) ? 2 : 1;
+      x.exact_fused = plan.grid > 1 ? 2 : 1;
       x.exact_src = sampling;
       x.exact_first_seen = ctx->d_map;
       x.exact_scratch = reinterpret_cast<unsigned char *>(ctx->d_exact.ptr);
@@ -428,14 +440,12 @@ void run_split(dq_context *ctx, SplitRun run) {
   }
   ctx->mark(3);
   ctx->stats.kernel_launches++;
-  ctx->pend.a = a;
-  ctx->pend.use_v2 = use_v2;
-  ctx->pend.unaudited = hist && !a.tie_audit && ctx->tie_policy != 0;
+  q.split = a;
 }
 
 // Has the split launched last on this context delivered its palette?  (non-blocking; true when there is nothing to poll)
 bool split_ready(dq_context *ctx) {
-  const SplitArgs &a = ctx->pend.a;
+  const SplitArgs &a = ctx->qs.split;
   if (a.mailbox == nullptr) return true;
   if (ctx->mailbox[0] == a.mailbox_seq) return true;
   return cudaStreamQuery(ctx->stream) != cudaErrorNotReady;  // an error exit leaves the stream idle without the number
@@ -445,8 +455,7 @@ bool split_ready(dq_context *ctx) {
 // Returns the number of palette entries.
 uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out) {
   const dq_context::QuantState &q = ctx->qs;
-  const SplitArgs &a = ctx->pend.a;
-  const bool use_v2 = ctx->pend.use_v2;
+  const SplitArgs &a = q.split;
   const uint32_t K = q.K;
   ctx->ensure_small((size_t)K + 16);
   bool mailed = false;
@@ -480,9 +489,9 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out) {
   }
   if (ctx->h_cb->ctl[kCtlError] != 0) {
     fprintf(stderr, "divquant_b200: split controller failed (code %u, kernel v%d, detail %u/%u/%u, barrier counter %u; internal error)\n",
-            ctx->h_cb->ctl[kCtlError], use_v2 ? 2 : 1, ctx->h_cb->ctl[kCtlWords - 1], ctx->h_cb->ctl[kCtlJobs],
+            ctx->h_cb->ctl[kCtlError], q.v2 ? 2 : 1, ctx->h_cb->ctl[kCtlWords - 1], ctx->h_cb->ctl[kCtlJobs],
             ctx->h_cb->ctl[kCtlTiles], ctx->h_cb->ctl[kCtlNodes]);
-    if (use_v2) {
+    if (q.v2) {
       std::vector<uint32_t> prog(split2_max_ctas(ctx->sm_count, K));
       cudaMemcpy(prog.data(), ctx->d_progress.ptr, prog.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost);
       fprintf(stderr, "  last stage per CTA:");
@@ -491,7 +500,7 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out) {
     }
     abort();
   }
-  if (use_v2 && ctx->profile_narrow) {
+  if (q.v2 && ctx->profile_narrow) {
     uint32_t prof[8];
     cudaMemcpy(prof, ctx->d_progress.ptr + 756, sizeof(prof), cudaMemcpyDeviceToHost);
     uint32_t wp[9];
@@ -515,7 +524,7 @@ uint32_t run_split_finish(dq_context *ctx, uint32_t *colortable_out) {
   ctx->stats.splits_computed = ctx->h_cb->ctl[kCtlSplits];
   ctx->stats.tie_flags = a.tie_audit ? ctx->h_cb->ctl[kCtlTie] : 0u;
   // exact-integer sums without an audit (the generic kernel beyond the ordered path's reach): say so
-  if (ctx->pend.unaudited && ctx->h_cb->ucount > a.exact_small_max) ctx->stats.tie_flags |= (uint32_t)kTieUnaudited;
+  if (q.report_unaudited && ctx->h_cb->ucount > a.exact_small_max) ctx->stats.tie_flags |= (uint32_t)kTieUnaudited;
   if (q.records && K > 1)
     DQ_CUDA_CHECK(cudaMemcpy(q.records, ctx->d_records.ptr, (size_t)(K - 1) * sizeof(SplitRecord), cudaMemcpyDeviceToHost));
   if (q.mean_out) DQ_CUDA_CHECK(cudaMemcpy(q.mean_out, ctx->d_cluster_mean.ptr, (size_t)3 * K * sizeof(double), cudaMemcpyDeviceToHost));
@@ -621,6 +630,7 @@ void rebuild_histogram(dq_context *ctx) {
 // source, or one per pixel of q.d_in), then the split.  Nothing is waited for.
 void quantize_launch(dq_context *ctx) {
   const dq_context::QuantState &q = ctx->qs;
+  plan_paths(ctx);
   ctx->mark(0);
   ctx->d_pts0.ensure(q.point_cap);
   if (q.table_dirty) {
@@ -663,13 +673,18 @@ void quantize_begin(dq_context *ctx, uint32_t n, const uint32_t *d_in, uint32_t 
   quantize_launch(ctx);
 }
 
-// Second half, as a small state machine so that a host thread that drives several contexts never has to wait inside it:
-//   phase 0  the split's palette is collected; a clean frame is done.  A flagged frame (tie audit, dq_tie.cuh) either gets
-//            the resolver queued (only palette roundings in doubt: dq_resolve.cu) -> phase 1, or is queued once more on
-//            the ordered path -> phase 2
-//   phase 1  the resolver's verdict: palette words patched, done -- or not resolvable there -> phase 2
-//   phase 2  the ordered re-run's palette is collected, done
-// quantize_step() advances one phase and says what to poll next; quantize_pending_ready() is the non-blocking poll.
+// Second half, as a small state machine so that a host thread that drives several contexts never has to wait inside it
+// (QuantState::step is what comes next):
+//   kSplit         the split's palette is collected; a clean frame is done.  A flagged frame (tie audit, dq_tie.cuh) gets
+//                  the resolver queued (only palette roundings and cuts in doubt: dq_resolve.cu) -> kResolve or
+//                  kResolveLarge, or goes to the fallback
+//   kResolve       the resolver's verdict: palette words patched, done -- or a cut the reference makes elsewhere: the split
+//   kResolveLarge  once more with that cut forced -> kSplit -- or, after the shared-memory form, a chain through a large
+//                  node: the large form -> kResolveLarge -- or the fallback
+//   kOrdered       the ordered re-run's palette is collected, done
+// The fallback queues the ordered re-run -> kOrdered where the call allows it and the ordered path holds the frame; else
+// the frame is done and stays flagged in the stats.
+// quantize_step() advances one step and says what to poll next; quantize_pending_ready() is the non-blocking poll.
 enum QuantStepResult { kQuantDone = 0, kQuantPending = 1 };
 
 // Which of the resolver's cut entries become forced cuts of the next run of the split (host logic of the re-split, pure):
@@ -693,20 +708,26 @@ uint32_t select_cut_overrides(const CutOverride *rec, const uint32_t *status, ui
 }
 
 bool quantize_pending_ready(dq_context *ctx) {
-  if (ctx->qs.phase == 1 || ctx->qs.phase == 3) return cudaEventQuery(ctx->tie_ev) != cudaErrorNotReady;
+  using Step = dq_context::QuantState::Step;
+  if (ctx->qs.step == Step::kResolve || ctx->qs.step == Step::kResolveLarge)
+    return cudaEventQuery(ctx->tie_ev) != cudaErrorNotReady;
   return split_ready(ctx);
 }
 
 QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colortable) {
+  using Step = dq_context::QuantState::Step;
   dq_context::QuantState &q = ctx->qs;
   const uint32_t K = q.K;
-  auto queue_rerun = [&]() {
+  auto rerun_or_done = [&]() {
     // Some decision of the exact-integer split sits inside the rounding noise of the reference's sequential sums:
     // the reference's own summation order decides.  The count table is all-zero again (the split kernel zeroed what
     // it collected), so the frame simply goes through the histogram and the split once more, on the ordered path.
+    // Where the call or the frame's size rules that out, the frame is done and stays flagged in the stats.
+    if (!q.rerun_ok || ctx->stats.num_points > kExactMaxPoints) return kQuantDone;
     rebuild_histogram(ctx);
     run_split(ctx, SplitRun::kOrdered);
-    q.phase = 2;
+    q.step = Step::kOrdered;
+    return kQuantPending;
   };
   auto queue_resplit = [&]() {
     // The reference cuts some node on the other side of an integer than the exact mean does (the resolver found out, and
@@ -717,25 +738,34 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     rebuild_histogram(ctx);
     run_split(ctx, SplitRun::kForcedCuts);
     q.resplits++;
-    q.phase = 0;
+    q.step = Step::kSplit;
   };
-  auto queue_big_resolve = [&]() {
-    // the resolver's large form (dq_resolve.cu): chains through nodes of any size, a global sort instead of one in shared memory
+  auto queue_resolve = [&](bool large) {
+    // the resolver (dq_resolve.cu) in its shared-memory form, or its large form: chains through nodes of any size, a global
+    // sort instead of one in shared memory; its verdict comes back in h_small: [palette | status words | reference cuts]
     const uint32_t U = ctx->stats.num_points;
     uint32_t n_pow2 = 2;
     while (n_pow2 < U) n_pow2 <<= 1;
-    ctx->d_keys.ensure(n_pow2);
-    ctx->d_sortvals.ensure(n_pow2);
-    ctx->d_flat.ensure(U);
+    if (large) {
+      ctx->d_keys.ensure(n_pow2);
+      ctx->d_sortvals.ensure(n_pow2);
+      ctx->d_flat.ensure(U);
+    }
     uint32_t *d_status = ctx->d_tie.ptr + kTieStatus;
     DQ_CUDA_CHECK(cudaMemsetAsync(d_status, 0, 2 * kTieListCap * sizeof(uint32_t), ctx->stream));
     uint2 *pts[2] = {ctx->d_pts0.ptr, ctx->d_pts1.ptr};
-    tie_resolve_big_launch(ctx->d_nodes.ptr, ctx->h_cb->ctl[kCtlNodes], pts, ctx->d_map, U, q.norm, 8 - q.num_bits, ctx->d_tie.ptr,
-                           q.tie_count, q.cut_count, ctx->d_keys.ptr, ctx->d_sortvals.ptr, ctx->d_flat.ptr,
-                           ctx->d_tie.ptr + kTieCounter, ctx->d_palette.ptr, d_status, ctx->sm_count, ctx->stream);
-    uint32_t steps = 0;
-    for (uint32_t k = 2; k <= n_pow2; k <<= 1) steps += (uint32_t)__builtin_ctz(k);
-    ctx->stats.kernel_launches += 3 + steps;
+    if (large) {
+      tie_resolve_big_launch(ctx->d_nodes.ptr, ctx->h_cb->ctl[kCtlNodes], pts, ctx->d_map, U, q.norm, 8 - q.num_bits, ctx->d_tie.ptr,
+                             q.tie_count, q.cut_count, ctx->d_keys.ptr, ctx->d_sortvals.ptr, ctx->d_flat.ptr,
+                             ctx->d_tie.ptr + kTieCounter, ctx->d_palette.ptr, d_status, ctx->sm_count, ctx->stream);
+      uint32_t steps = 0;
+      for (uint32_t k = 2; k <= n_pow2; k <<= 1) steps += (uint32_t)__builtin_ctz(k);
+      ctx->stats.kernel_launches += 3 + steps;
+    } else {
+      tie_resolve_launch(ctx->d_nodes.ptr, ctx->h_cb->ctl[kCtlNodes], pts, ctx->d_map, q.norm, 8 - q.num_bits, ctx->d_tie.ptr,
+                         q.tie_count, q.cut_count, ctx->d_palette.ptr, d_status, ctx->stream);
+      ctx->stats.kernel_launches++;
+    }
     DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->h_small + K, d_status, (q.tie_count + q.cut_count) * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                                   ctx->stream));
     if (q.cut_count)
@@ -744,21 +774,16 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
     DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->h_small, ctx->d_palette.ptr, (size_t)q.k_first * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                                   ctx->stream));
     DQ_CUDA_CHECK(cudaEventRecord(ctx->tie_ev, ctx->stream));
-    q.phase = 3;
+    q.step = large ? Step::kResolveLarge : Step::kResolve;
   };
-  const bool can_rerun = ctx->tie_policy == 2 && q.table_dirty && ctx->exact_small && K <= kExactMaxColors && K <= kSplit2MaxColors &&
-                         ctx->split_version == 2 && q.merged.colours == nullptr;
-  if (q.phase == 0) {
+  if (q.step == Step::kSplit) {
     *k_inout = run_split_finish(ctx, colortable);
     q.flags = ctx->stats.tie_flags;
     q.flags_all |= q.flags;
     ctx->stats.tie_flags = q.flags_all;  // (a frame that needed forced cuts stays marked as flagged)
     ctx->stats.cut_overrides = q.n_ovr;
     if (q.flags == 0u) return kQuantDone;
-    if ((q.flags & ~(uint32_t)(kTieRound | kTieCut)) == 0u && ctx->tie_policy == 2 && q.table_dirty && ctx->exact_small &&
-        q.records == nullptr && q.mean_out == nullptr) {
-      // Only palette roundings are in doubt (a cluster mean exactly on x.5: the commonest tie by far): the reference's own
-      // ordered sums are redone for just the flagged clusters (dq_resolve.cu), on top of a first-seen pass over the pixels.
+    if (q.resolve_ok && (q.flags & ~(uint32_t)(kTieRound | kTieCut)) == 0u) {
       // Palette roundings and cuts are in doubt, nothing else (by far the commonest flags): both hang on the mean of ONE node,
       // which the resolver recomputes in the reference's arithmetic (dq_resolve.cu) on top of a first-seen pass over the pixels.
       // A rounding is rewritten; a cut either separates the same points as the reference's (nothing to do) or it does not
@@ -773,75 +798,47 @@ QuantStepResult quantize_step(dq_context *ctx, uint32_t *k_inout, uint32_t *colo
         ctx->ensure_small((size_t)K + 16 + 8 * kTieListCap + 2);
         q.k_first = *k_inout;
         if (!ctx->tie_ev) DQ_CUDA_CHECK(cudaEventCreateWithFlags(&ctx->tie_ev, cudaEventDisableTiming));
-        if ((ctx->resolve_mode & 1) == 0) {
-          queue_big_resolve();
-          return kQuantPending;
-        }
-        uint32_t *d_status = ctx->d_tie.ptr + kTieStatus;
-        DQ_CUDA_CHECK(cudaMemsetAsync(d_status, 0, 2 * kTieListCap * sizeof(uint32_t), ctx->stream));
-        uint2 *pts[2] = {ctx->d_pts0.ptr, ctx->d_pts1.ptr};
-        tie_resolve_launch(ctx->d_nodes.ptr, ctx->h_cb->ctl[kCtlNodes], pts, ctx->d_map, q.norm, 8 - q.num_bits, ctx->d_tie.ptr,
-                           q.tie_count, q.cut_count, ctx->d_palette.ptr, d_status, ctx->stream);
-        ctx->stats.kernel_launches++;
-        DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->h_small + K, d_status, (q.tie_count + q.cut_count) * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                                      ctx->stream));
-        if (q.cut_count)
-          DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->h_small + K + 2 * kTieListCap, ctx->d_tie.ptr + kTieRefCut,
-                                        q.cut_count * sizeof(CutOverride), cudaMemcpyDeviceToHost, ctx->stream));
-        DQ_CUDA_CHECK(cudaMemcpyAsync(ctx->h_small, ctx->d_palette.ptr, (size_t)q.k_first * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                                      ctx->stream));
-        DQ_CUDA_CHECK(cudaEventRecord(ctx->tie_ev, ctx->stream));
-        q.phase = 1;
+        queue_resolve((ctx->resolve_mode & 1) == 0);
         return kQuantPending;
       }
     }
-    if (can_rerun && ctx->stats.num_points <= kExactMaxPoints) {
-      queue_rerun();
-      return kQuantPending;
-    }
-    return kQuantDone;  // flagged and not resolvable here (more colours than the ordered path takes): reported in the stats
+    return rerun_or_done();
   }
-  if (q.phase == 1 || q.phase == 3) {
-    DQ_CUDA_CHECK(cudaEventSynchronize(ctx->tie_ev));  // (already complete when the caller polled)
-    bool resolved = true, differs = false;
-    for (uint32_t i = 0; i < q.tie_count + q.cut_count; ++i) {
-      resolved = resolved && ctx->h_small[K + i] == 1u;
-      differs = differs || ctx->h_small[K + i] == 3u;  // a cut the reference makes elsewhere: only a re-run helps
-    }
-    if (resolved) {
-      memcpy(colortable, ctx->h_small, (size_t)q.k_first * sizeof(uint32_t));
-      *k_inout = q.k_first;
-      ctx->stats.tie_resolved = q.tie_count + q.cut_count;
-      return kQuantDone;
-    }
-    if (differs && q.resplits < 8) {
-      // status-3 cut entries whose range is not inside another one's (a cut below a cut that changes is decided next time)
-      CutOverride rec[kTieListCap];  // (copied out: K odd leaves the doubles inside h_small unaligned)
-      memcpy(rec, ctx->h_small + K + 2 * kTieListCap, q.cut_count * sizeof(CutOverride));
-      const uint32_t *st = ctx->h_small + K + q.tie_count;
-      const uint32_t added = select_cut_overrides(rec, st, q.cut_count, q.h_ovr, &q.n_ovr, kCutOverrideCap);
-      if (added) {
-        queue_resplit();
-        return kQuantPending;
-      }
-    }
-    if (q.phase == 1 && !differs && (ctx->resolve_mode & 2)) {  // a chain through a large node: the resolver's large form
-      queue_big_resolve();
-      return kQuantPending;
-    }
-    if (can_rerun && ctx->stats.num_points <= kExactMaxPoints) {
-      queue_rerun();
-      return kQuantPending;
-    }
+  if (q.step == Step::kOrdered) {
+    *k_inout = run_split_finish(ctx, colortable);
+    ctx->stats.tie_flags = q.flags;
+    ctx->stats.ordered_rerun = 1;
     return kQuantDone;
   }
-  // phase 2
-  const uint32_t launches = ctx->stats.kernel_launches;
-  *k_inout = run_split_finish(ctx, colortable);
-  ctx->stats.kernel_launches = launches;
-  ctx->stats.tie_flags = q.flags;
-  ctx->stats.ordered_rerun = 1;
-  return kQuantDone;
+  // the resolver's verdict (kResolve, kResolveLarge)
+  DQ_CUDA_CHECK(cudaEventSynchronize(ctx->tie_ev));  // (already complete when the caller polled)
+  bool resolved = true, differs = false;
+  for (uint32_t i = 0; i < q.tie_count + q.cut_count; ++i) {
+    resolved = resolved && ctx->h_small[K + i] == 1u;
+    differs = differs || ctx->h_small[K + i] == 3u;  // a cut the reference makes elsewhere: only a re-run helps
+  }
+  if (resolved) {
+    memcpy(colortable, ctx->h_small, (size_t)q.k_first * sizeof(uint32_t));
+    *k_inout = q.k_first;
+    ctx->stats.tie_resolved = q.tie_count + q.cut_count;
+    return kQuantDone;
+  }
+  if (differs && q.resplits < 8) {
+    // status-3 cut entries whose range is not inside another one's (a cut below a cut that changes is decided next time)
+    CutOverride rec[kTieListCap];  // (copied out: K odd leaves the doubles inside h_small unaligned)
+    memcpy(rec, ctx->h_small + K + 2 * kTieListCap, q.cut_count * sizeof(CutOverride));
+    const uint32_t *st = ctx->h_small + K + q.tie_count;
+    const uint32_t added = select_cut_overrides(rec, st, q.cut_count, q.h_ovr, &q.n_ovr, kCutOverrideCap);
+    if (added) {
+      queue_resplit();
+      return kQuantPending;
+    }
+  }
+  if (q.step == Step::kResolve && !differs && (ctx->resolve_mode & 2)) {  // a chain through a large node: the large form
+    queue_resolve(true);
+    return kQuantPending;
+  }
+  return rerun_or_done();
 }
 
 // Blocking form.  Returns true if a unique list exists (d_uniq / d_cb->ucount) for a following table remap.
@@ -1421,16 +1418,13 @@ dq_context *dq_context_create(int device) {
     memset(mb, 0, kMailboxWords * sizeof(uint32_t));
     ctx->mailbox = static_cast<volatile uint32_t *>(mb);
   }
-  if (const char *e = getenv("DIVQUANT_B200_MAILBOX")) ctx->use_mailbox = (e[0] != '0');
   memset(&ctx->stats, 0, sizeof(ctx->stats));
   for (int i = 0; i < 8; ++i) DQ_CUDA_CHECK(cudaEventCreate(&ctx->ev[i]));
   ctx->display_timings = display_timings_default();
-  if (const char *e = getenv("DIVQUANT_B200_SPLIT")) ctx->split_version = (e[0] == '1') ? 1 : 2;
   if (const char *e = getenv("DIVQUANT_B200_TIE")) ctx->tie_policy = std::min(std::max(atoi(e), 0), 2);
   if (const char *e = getenv("DIVQUANT_B200_RESOLVE")) ctx->resolve_mode = atoi(e) & 3;
   if (const char *e = getenv("DIVQUANT_B200_SPIN_MS")) ctx->spin_cycles = (long long)std::max(atol(e), 0l) * 2000000ll;  // ~2 GHz
   if (const char *e = getenv("DIVQUANT_B200_EXACT_SMALL")) ctx->exact_small = (e[0] != '0');
-  if (const char *e = getenv("DIVQUANT_B200_EXACT_PARALLEL")) ctx->exact_parallel = (e[0] != '0');
   if (const char *e = getenv("DIVQUANT_B200_EXACT_MAX")) ctx->exact_max_points = (uint32_t)std::min<long>(std::max<long>(atol(e), 0), kExactMaxPoints);
   ctx->profile_narrow = getenv("DQ_PROFILE_NARROW") != nullptr;
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
@@ -1471,7 +1465,6 @@ void dq_context_destroy(dq_context *ctx) {
   ctx->d_pal_scratch.release();
   ctx->d_timeline.release();
   ctx->d_slots.release();
-  ctx->d_cursors.release();
   ctx->d_progress.release();
   ctx->d_exact.release();
   ctx->d_tie.release();
@@ -2276,6 +2269,7 @@ uint32_t dq_debug_split_points(dq_context *ctx, const uint32_t *colours, const u
   ctx->h_cb->ucount = num_points;
   DQ_CUDA_CHECK(cudaMemcpyAsync(&ctx->d_cb->ucount, &ctx->h_cb->ucount, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   DQ_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+  plan_paths(ctx);
   run_split(ctx, SplitRun::kFirst);
   return run_split_finish(ctx, colortable);
 }
